@@ -1,17 +1,26 @@
 #!/usr/bin/env python
 """bench.py — env-steps/s of the fused trading-env step kernel (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c4] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of envs: one fe_step launch over this GPU's envs.
 Default workload = BASELINE config 2 (single asset, 1 Mi envs per GPU, W=60, synthetic GBM daily bars).
 N>1 is launched by torchrun, one rank per GPU; envs are sharded (weak scaling: 1 Mi envs per GPU), the
 series is replicated, the step needs no collective.  Rank 0 prints ONE JSON line.
 
-Timing: W warm-up steps, then the K-step block is timed `blocks` times back to back (CUDA events on the
-launch stream, barrier + synchronize around every block, max over ranks per block); `value` / `ms_per_step`
-come from the MEDIAN block, `timing` also gives min and max — a 20-step block is 5 ms, one block alone is
-at the mercy of a clock ramp.
+Timing: W warm-up steps, then exactly K timed steps right behind them, split into `blocks` blocks that run back to
+back (a CUDA event on the launch stream at every block boundary, barrier + synchronize before the warm-up and after
+the K steps, max over ranks per block); `value` / `ms_per_step` come from the MEDIAN block's time per step, `timing`
+also gives min and max — a 20-step block is 5 ms, one block alone is at the mercy of a clock ramp.
+The default K = 200 (ten 20-step blocks) gave 4.712, 4.718 and 4.714 G env-steps/s in three c2 runs on one B200 at
+1000 W.  Longer windows are not steadier: the per-step time rises from 0.222 ms over steps 10-210 to about 0.25 ms
+towards step 600 (median SM clock 1957 MHz against 1965 at K = 200), so K = 600 gave 4.31 - 4.36 across three runs.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what the timed call (step_into) returned in the last
+step as float32 .npy files: rewards.npy (N,), dones.npy (N,) as 0/1, obs.npy (N, W, 5A).  An array larger than
+its share of 48 MB in all is replaced by the rows of a fixed, seeded sample of envs (sorted env indices drawn
+with DUMP_SEED).  Series, actions and env seeds are fixed, so the same arguments give the same inputs on every
+run and two builds can be compared output for output.
 
 value    = device-resident throughput through TimeSeriesEnv.step_into (caller-owned outputs, actions in HBM).
 public_step = the same loop through the drop-in call TimeSeriesEnv.step(actions) (allocates obs/rewards/dones).
@@ -26,7 +35,8 @@ roofline = DRAM bytes per launch / average launch duration (live, CUDA events), 
            L2-resident: those never reach DRAM, and counting them gave round 1 a "fraction" of 1.34) and `algorithmic_*`
            (all 2264 B).
 also     = the other BASELINE workloads measured in the same process (N=1: c4, c3, c5 and c1; N>1: c4 and c5), same protocol;
-           c1 = the reference's native size (1024 envs), the configuration cpu_baseline times the reference on;
+           c1 = the reference's native size (1024 envs), the configuration cpu_baseline times the reference on (at least
+           300 timed steps: a step there takes microseconds);
            c5 = the ES population rollout (policy forward + env step + return bookkeeping per step, EvoAgent.train() per
            generation; perturbations are stored as fp16 where the reference draws f32).
 collectives (N>1) = device time of the NCCL collectives the path uses outside the step (episode statistics
@@ -46,6 +56,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True   # the benchmark leaves the source tree as it found it
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -55,6 +66,8 @@ METRIC = "env_steps_per_sec"
 UNIT = "env-steps/s"
 SERIES_SEED = 20260101
 ACTION_SEED = 1234
+DUMP_SEED = 4321
+DUMP_BYTES = {"obs": 32 << 20, "rewards": 8 << 20, "dones": 8 << 20}   # --dump-outputs: 48 MB in all
 L2_RESIDENT_BYTES = 48 << 20   # the library's own threshold for the "cached" flavour (fe_step.cu: pick_pipe_stages)
 
 
@@ -377,7 +390,7 @@ def cpu_baseline_block(rb: dict) -> dict:
     best = rb["best"]
     if best is None:   # no reference tree on this box: the port is all there is
         p = rb["cpu_port"]
-        return {**p, "note": "baseline/_ref absent: oracle port only"}
+        return {**p, "cpu_port": p, "note": "baseline/_ref absent: oracle port only"}
     return {"value": best["value"], "unit": UNIT, "cores": best["threads"], "kind": "reference", "tree": "baseline/_ref",
             "sample": (f"unmodified reference TimeSeriesEnv.step, c2 series as CSV, W=60, {best['envs']} envs per step "
                        f"({'C1 native' if best['envs'] <= 4096 else 'widened, SURVEY App. C.4'}), {best['steps']} steps, "
@@ -410,7 +423,8 @@ def run_reference_arm(args, rank: int):
 
 # ------------------------------------------------------------------------------ GPU arm ------
 class Timer:
-    """K-step blocks timed with CUDA events, barrier + synchronize around every block, max over ranks per block."""
+    """Exactly `steps` timed steps in back-to-back blocks right behind the warm-up, a CUDA event at every block boundary,
+    barrier + synchronize before the warm-up and after the last block, max over ranks per block."""
 
     def __init__(self, torch, dist, dev, world):
         self.torch, self.dist, self.dev, self.world = torch, dist, dev, world
@@ -421,38 +435,60 @@ class Timer:
             self.dist.barrier()
 
     def blocks(self, fn, steps: int, warmup: int, nblocks: int, wall: bool = False):
+        """Returns [(ms, steps)] per block; the block sizes differ by at most one and add up to `steps`."""
         torch = self.torch
         stream = torch.cuda.current_stream()
+        nblocks = max(1, min(nblocks, steps))
+        sizes = [steps // nblocks + (b < steps % nblocks) for b in range(nblocks)]
+        events = [torch.cuda.Event(enable_timing=True) for _ in range(nblocks + 1)]
+        self.sync_all()
         k = 0
-        for _ in range(warmup):
+        for _ in range(warmup):   # still queued when the first event is recorded: the device never idles in between
             fn(k)
             k += 1
-        ms = []
-        for _ in range(nblocks):
-            self.sync_all()
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            t0 = time.perf_counter()
-            e0.record(stream)
-            for _ in range(steps):
+        walls = [time.perf_counter()]
+        events[0].record(stream)
+        for b, n in enumerate(sizes):
+            for _ in range(n):
                 fn(k)
                 k += 1
-            e1.record(stream)
-            self.sync_all()
-            t = e0.elapsed_time(e1)
-            if wall:   # a host-synchronous call: the wall clock is the larger of the two
-                t = max(t, (time.perf_counter() - t0) * 1e3)
-            ms.append(t)
+            events[b + 1].record(stream)
+            walls.append(time.perf_counter())
+        self.sync_all()
+        ms = [events[b].elapsed_time(events[b + 1]) for b in range(nblocks)]
+        if wall:   # a host-synchronous call: the wall clock is the larger of the two
+            ms = [max(t, (walls[b + 1] - walls[b]) * 1e3) for b, t in enumerate(ms)]
         v = torch.tensor(ms, dtype=torch.float64, device=self.dev)
         if self.world > 1:
             self.dist.all_reduce(v, op=self.dist.ReduceOp.MAX)
-        return [float(x) for x in v.tolist()]
+        return [(float(x), n) for x, n in zip(v.tolist(), sizes)]
 
 
-def summarize(ms_blocks, steps: int, total_envs: int):
-    med, lo, hi = float(np.median(ms_blocks)), float(min(ms_blocks)), float(max(ms_blocks))
-    return {"value": total_envs * steps / (med * 1e-3), "ms_per_step": med / steps,
-            "timing": {"blocks": len(ms_blocks), "steps_per_block": steps, "ms_per_step_median": med / steps,
-                       "ms_per_step_min": lo / steps, "ms_per_step_max": hi / steps}}
+def summarize(blocks, total_envs: int):
+    per_step = [ms / n for ms, n in blocks]
+    med, lo, hi = float(np.median(per_step)), float(min(per_step)), float(max(per_step))
+    return {"value": total_envs / (med * 1e-3), "ms_per_step": med,
+            "timing": {"blocks": len(blocks), "timed_steps": sum(n for _, n in blocks),
+                       "steps_per_block": [n for _, n in blocks], "ms_per_step_median": med,
+                       "ms_per_step_min": lo, "ms_per_step_max": hi}}
+
+
+def dump_sample(n: int, row_bytes: int, budget: int):
+    """Sorted indices of a fixed, seeded sample of n rows that fits `budget` bytes; None when all n rows fit."""
+    k = max(1, budget // row_bytes)
+    if k >= n:
+        return None
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n, k, replace=False))
+
+
+def dump_outputs(out_dir: str, torch, outputs: dict):
+    """--dump-outputs: the timed call's outputs of its last step as float32 .npy files (module docstring)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        idx = dump_sample(t.shape[0], t[0].numel() * 4, DUMP_BYTES[name])
+        if idx is not None:
+            t = t.index_select(0, torch.from_numpy(idx).to(t.device))
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.float().cpu().numpy())
 
 
 def load_peak():
@@ -496,8 +532,9 @@ def roofline_block(workload: str, W: int, N: int, A: int, kernel_s: float, table
 
 
 def measure_workload(torch, par, loader, timer, workload, N, W, rank, world, local_rank, steps, warmup, nblocks, variant,
-                     full: bool):
-    """One workload on this rank's GPU.  full=True adds the public step() and the host-buffer (e2e) legs."""
+                     full: bool, dump_dir: str | None = None):
+    """One workload on this rank's GPU.  full=True adds the public step() and the host-buffer (e2e) legs;
+    dump_dir: rank 0 writes the device-resident leg's last outputs there (--dump-outputs)."""
     dev = f"cuda:{local_rank}"
     A = WORKLOAD_ASSETS[workload]
     total = N * world
@@ -515,13 +552,15 @@ def measure_workload(torch, par, loader, timer, workload, N, W, rank, world, loc
 
     out = {}
     dev_blocks = timer.blocks(lambda i: env.step_into(ring[i % 8], obs, rewards, dones), steps, warmup, nblocks)
-    res = summarize(dev_blocks, steps, total)
+    if dump_dir is not None and rank == 0:
+        dump_outputs(dump_dir, torch, {"obs": obs, "rewards": rewards, "dones": dones})
+    res = summarize(dev_blocks, total)
     kernel_s = res["ms_per_step"] * 1e-3   # only fe_step launches sit between the events
     table_bytes = int(series.logret.numel() * series.logret.element_size())
     res["roofline"] = roofline_block(workload, W, N, A, kernel_s, table_bytes, env.kernel_name())
     res["episodes_finished_last_step"] = int(dones.sum().item())
     launches_per_step = 2 if " + " in env.kernel_name() else 1
-    launches = launches_per_step * steps * nblocks
+    launches = launches_per_step * steps
     out.update(res)
     if full:
         del obs
@@ -531,11 +570,11 @@ def measure_workload(torch, par, loader, timer, workload, N, W, rank, world, loc
             held.clear()
             held.append(env.step(ring[i % 8]))   # fresh obs / rewards / dones every call, like the reference
 
-        pub = summarize(timer.blocks(public_step, steps, warmup, nblocks), steps, total)
+        pub = summarize(timer.blocks(public_step, steps, warmup, nblocks), total)
         held.clear()
         out["public_step"] = {"value": pub["value"], "unit": UNIT, "ms_per_step": pub["ms_per_step"], "timing": pub["timing"],
                               "api": "TimeSeriesEnv.step(actions) -> (obs, rewards, dones, info): allocates its outputs"}
-        launches += launches_per_step * steps * nblocks
+        launches += launches_per_step * steps
         ring_host = [a.cpu().pin_memory() for a in ring[:4]]
         check = [0.0]
 
@@ -547,13 +586,13 @@ def measure_workload(torch, par, loader, timer, workload, N, W, rank, world, loc
             env.step_host(ring_host[i % 4], packed_dones=True)
             check[0] += float(r_np[0]) + int(d_np[0])   # the host reads the step's result
 
-        e2e = summarize(timer.blocks(host_step, steps, warmup, nblocks, wall=True), steps, total)
+        e2e = summarize(timer.blocks(host_step, steps, warmup, nblocks, wall=True), total)
         h2d, d2h = env.host_bytes_per_step(packed_dones=True)
         out["e2e"] = {"value": e2e["value"], "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
                       "ms_per_step": e2e["ms_per_step"], "timing": e2e["timing"],
                       "api": "TimeSeriesEnv.step_host(packed_dones=True) -> fe_step_host_packed (pinned host buffers; rewards f32, "
                              "dones 1 bit per env)"}
-        launches += launches_per_step * steps * nblocks   # the persistent kernels pack the dones themselves
+        launches += launches_per_step * steps   # the persistent kernels pack the dones themselves
 
         _, r_h, d_h, _ = env.step_host(ring_host[0])
         r_np32, d_np32 = r_h.numpy(), d_h.numpy()
@@ -562,11 +601,11 @@ def measure_workload(torch, par, loader, timer, workload, N, W, rank, world, loc
             env.step_host(ring_host[i % 4])
             check[0] += float(r_np32[0]) + int(d_np32[0])
 
-        e2e32 = summarize(timer.blocks(host_step_i32, steps, warmup, nblocks, wall=True), steps, total)
+        e2e32 = summarize(timer.blocks(host_step_i32, steps, warmup, nblocks, wall=True), total)
         h2d32, d2h32 = env.host_bytes_per_step()
         out["e2e"]["int32_dones"] = {"value": e2e32["value"], "ms_per_step": e2e32["ms_per_step"], "h2d_bytes_per_step": h2d32,
                                      "d2h_bytes_per_step": d2h32, "api": "TimeSeriesEnv.step_host -> fe_step_host"}
-        launches += launches_per_step * steps * nblocks
+        launches += launches_per_step * steps
     out["gpu_launches"] = launches
     out["meta"] = meta
     del env, series, ring
@@ -629,25 +668,33 @@ def measure_collectives(torch, dist, par, dev, world, N):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200, help="timed steps per measured leg (module docstring: Timing)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c2", choices=["c2", "c3", "c4"])
     ap.add_argument("--envs", type=int, default=None, help="envs per GPU (default: 1 Mi; c3: 65536)")
     ap.add_argument("--window", type=int, default=None, help="default 60; c3: 128")
     ap.add_argument("--variant", default="auto")
-    ap.add_argument("--blocks", type=int, default=None, help="how many times the K-step block is timed (default: ~200 steps in total, 3..10)")
+    ap.add_argument("--blocks", type=int, default=None,
+                    help="how many blocks the K timed steps are split into (default: K // 20, at least 3 and at most 10)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--ref-widened-envs", type=int, default=65536,
                     help="second size the unmodified reference is timed at (SURVEY App. C.4 widening); 0 = native N=1024 only")
     ap.add_argument("--no-also", action="store_true", help="skip the other workloads / collectives")
     ap.add_argument("--no-c5", action="store_true", help="skip the ES population rollout (also.c5)")
     ap.add_argument("--no-numa-bind", action="store_true", help="do not pin the rank to its GPU's NUMA-local CPUs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the timed call's outputs of its last step to DIR/<name>.npy (float32, a seeded sample of "
+                         "envs where an array exceeds its share of 48 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the GPU arm's outputs (--impl ours)")
     args.warmup = max(args.warmup, 3)
     args.envs = args.envs or WORKLOAD_DEFAULTS[args.workload][0]
     args.window = args.window or WORKLOAD_DEFAULTS[args.workload][1]
-    nblocks = args.blocks or max(3, min(10, -(-200 // args.steps)))
+    nblocks = args.blocks or max(3, min(10, args.steps // 20))
 
     rank = int(os.environ.get("RANK", "0"))
     if args.impl == "reference":
@@ -671,7 +718,7 @@ def main():
     sampler = ClockSampler(local_rank)
     with sampler:
         main_res = measure_workload(torch, par, loader, timer, args.workload, args.envs, args.window, rank, world, local_rank,
-                                    args.steps, args.warmup, nblocks, args.variant, full=True)
+                                    args.steps, args.warmup, nblocks, args.variant, full=True, dump_dir=args.dump_outputs)
     also, collectives = {}, None
     if not args.no_also:
         others = [w for w in (("c4", "c3") if world == 1 else ("c4",)) if w != args.workload]
@@ -690,7 +737,7 @@ def main():
             # BASELINE config 1, the size the reference itself runs at (cpu_baseline times the reference on exactly this):
             # launch-bound, so what counts is the public step() and the host-buffer call, not a roofline
             n, win = WORKLOAD_DEFAULTS["c1"]
-            r = measure_workload(torch, par, loader, timer, "c1", n, win, rank, world, local_rank, max(args.steps, 100), args.warmup,
+            r = measure_workload(torch, par, loader, timer, "c1", n, win, rank, world, local_rank, max(args.steps, 300), args.warmup,
                                  3, "auto", full=True)
             also["c1"] = {"workload": WORKLOAD_NAMES["c1"], "envs_per_gpu": n, "window": win, "assets": 1, "value": r["value"],
                           "unit": UNIT, "ms_per_step": r["ms_per_step"], "kernel": r["roofline"]["kernel"],

@@ -43,9 +43,10 @@ def csv_arrays(path: str) -> dict:
 
 
 def trace(csv: str, window: int, steps: int, seed: int, *, evaluate=False, widen=None, action_fn=None,
-          scripted=None, store_all_obs=False, max_obs_steps=10, params=None) -> dict:
+          scripted=None, store_all_obs=False, max_obs_steps=10, params=None, obs_at=None) -> dict:
     """`params`: (max_shares, starting_balance, per_share_commission, initial_margin_requirement,
-    maintenance_margin_requirement) when they differ from the reference's defaults (time_series_env.py:20-26)."""
+    maintenance_margin_requirement) when they differ from the reference's defaults (time_series_env.py:20-26).
+    `obs_at`: the steps whose full observation is stored (default: the first two, the first steps with dones, the last)."""
     ref_kw = {}
     if params is not None:
         ref_kw = dict(max_shares=int(params[0]), starting_balance=float(params[1]), per_share_commission=float(params[2]),
@@ -84,7 +85,10 @@ def trace(csv: str, window: int, steps: int, seed: int, *, evaluate=False, widen
         states.append(np.stack([s["seg"].astype(np.float64), s["ptr"].astype(np.float64), s["cash"].astype(np.float64),
                                 s["long_sh"].astype(np.float64), s["short_sh"].astype(np.float64), s["margin"]]))
         obs_sums.append(o.reshape(N, -1).sum(axis=1))
-        keep = store_all_obs or t < 2 or (d.any() and len(obs_steps) < max_obs_steps) or t == steps - 1
+        if obs_at is not None:
+            keep = t in obs_at
+        else:
+            keep = store_all_obs or t < 2 or (d.any() and len(obs_steps) < max_obs_steps) or t == steps - 1
         if keep:
             obs_kept.append(o); obs_steps.append(t)
         if info:
@@ -133,8 +137,8 @@ def main():
         t = trace(csvs[name], W, steps, seed, evaluate=ev, max_obs_steps=4 if W == 390 else 10)
         np.savez_compressed(f"trace_{name.lower()}_w{W}{'_eval' if ev else ''}.npz", **t)
 
-    # ---- widened N on a real CSV (env i -> segment i mod D)
-    t = trace(csvs["OIH"], 60, 300, 12, widen=256)
+    # ---- widened N on a real CSV (env i -> segment i mod D); 100 steps and three full observations keep it under 1 MB
+    t = trace(csvs["OIH"], 60, 100, 12, widen=256, obs_at=(0, 19, 24))
     np.savez_compressed("trace_oih_w60_n256.npz", **t)
 
     # ---- adversarial GBM: big intrabar spikes + short-biased actions => margin calls at High and

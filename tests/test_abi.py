@@ -83,13 +83,12 @@ def test_tile_sizes(built):
 def test_env_has_no_cpu_fallback(built):
     import torch
 
-    if torch.cuda.is_available():
-        pytest.skip("CUDA present")
     from finenvs_b200.environments import TimeSeriesEnv
 
-    with pytest.raises(RuntimeError, match="no CPU fallback"):
-        TimeSeriesEnv("IBM", "dummy")
-    with pytest.raises(RuntimeError, match="no CPU fallback"):
+    if not torch.cuda.is_available():   # the default device is cuda:0: only refused where there is none
+        with pytest.raises(RuntimeError, match="no CPU fallback"):
+            TimeSeriesEnv("IBM", "dummy")
+    with pytest.raises(RuntimeError, match="no CPU fallback"):   # an explicit CPU device is refused everywhere
         TimeSeriesEnv("IBM", "dummy", device_id=-1)
 
 

@@ -1,10 +1,13 @@
 """bench.py's JSON contract, checked on the arm that needs no GPU: `--impl reference` (the unmodified reference env from
-baseline/_ref on the host cores, the C oracle port beside it).  The keys and their meaning are the driver's contract
-(see bench.py's docstring)."""
+baseline/_ref on the host cores, the C oracle port beside it).  The keys and their meaning are documented in bench.py's
+docstring.  On a GPU: the GPU arm times exactly --steps steps and --dump-outputs writes repeatable outputs."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -56,3 +59,36 @@ def test_reference_arm_forces_the_thread_count_under_torchrun():
     ncpu = len(os.sched_getaffinity(0))
     assert d["cpu_baseline"]["cores"] == ncpu and d["cpu_baseline"]["cpu_port"]["cores"] == ncpu
     assert d["config"]["total_envs"] == 2 << 20
+
+
+def _run_gpu_arm(dump_dir, envs):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "7", "--warmup", "3", "--envs", str(envs),
+                          "--no-also", "--no-cpu-baseline", "--dump-outputs", str(dump_dir)],
+                         capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    lines = [l for l in out.stdout.splitlines() if l.startswith("{")]
+    assert len(lines) == 1
+    return json.loads(lines[0])
+
+
+@pytest.mark.gpu
+def test_gpu_arm_times_exactly_the_requested_steps_and_dumps_repeatable_outputs(tmp_path):
+    envs = 65536                      # the full observation (79 MB) exceeds its share: obs.npy is the seeded sample
+    a, b = _run_gpu_arm(tmp_path / "a", envs), _run_gpu_arm(tmp_path / "b", envs)
+    for d in (a, b):
+        assert d["steps"] == 7 and d["timing"]["timed_steps"] == 7 and sum(d["timing"]["steps_per_block"]) == 7
+        assert d["public_step"]["timing"]["timed_steps"] == 7 and d["e2e"]["timing"]["timed_steps"] == 7
+        per_step = 2 if " + " in d["roofline"]["kernel"] else 1
+        assert d["gpu_launches"] == 4 * 7 * per_step   # device-resident, step(), two host-buffer legs
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == ["dones.npy", "obs.npy", "rewards.npy"] and sorted(os.listdir(tmp_path / "b")) == names
+    assert sum(os.path.getsize(tmp_path / "a" / n) for n in names) <= 64 << 20
+    arrays = {n: np.load(tmp_path / "a" / n) for n in names}
+    assert all(x.dtype == np.float32 for x in arrays.values())
+    assert arrays["rewards.npy"].shape == arrays["dones.npy"].shape == (envs,)
+    assert set(np.unique(arrays["dones.npy"])) <= {0.0, 1.0}
+    assert arrays["dones.npy"].sum() == a["episodes_finished_last_step"] > 0   # the dump holds the last timed step
+    obs = arrays["obs.npy"]
+    assert 0 < obs.shape[0] < envs and obs.shape[1:] == (60, 5) and np.isfinite(obs).all()
+    for n in names:                   # same arguments, same inputs: the outputs repeat bit for bit
+        assert np.array_equal(arrays[n], np.load(tmp_path / "b" / n)), n

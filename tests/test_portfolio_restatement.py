@@ -19,7 +19,7 @@ from oracle import ref_harness as rh
 from parity_utils import assert_bits_equal, day_labels, gbm_ohlc
 from portfolio_restatement import PortfolioRestatement, butterfly_sum
 
-pytestmark = pytest.mark.skipif(not rh.available(), reason="reference checkout not present")
+needs_reference = pytest.mark.skipif(not rh.available(), reason="reference checkout not present")
 
 
 def _asset_csvs(tmp_path, A, bars, sigmas, seed, s0=lambda a: 20.0 + 13.0 * a):
@@ -79,6 +79,7 @@ def test_butterfly_sum_is_the_warp_order():
     assert torch.equal(butterfly_sum(one), one)
 
 
+@needs_reference
 @pytest.mark.parametrize("sigma,frac,seed", [(0.12, 0.7, 31), (0.03, 0.9, 32), (0.15, 0.55, 33)])
 def test_restatement_equals_the_real_reference_at_one_asset(tmp_path, sigma, frac, seed):
     """The pin: same torch ops in the same order as time_series_env.py:277-521 when A = 1."""
@@ -118,6 +119,7 @@ def test_restatement_equals_the_real_reference_at_one_asset(tmp_path, sigma, fra
             r.close()
 
 
+@needs_reference
 @pytest.mark.parametrize("A,sigmas,frac,seed,params", [
     (2, [0.12, 0.05], 0.7, 41, {}),
     (5, [0.15, 0.02, 0.08, 0.12, 0.05], 0.6, 42, {}),
