@@ -103,6 +103,9 @@ _PROTOTYPES = {
     "fe_step_lazy": (C.c_int, [C.POINTER(FeParams), C.POINTER(FeSeries), C.POINTER(FeState), C.c_void_p, C.c_void_p,
                                C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
     "fe_materialize": (C.c_int, [C.POINTER(FeParams), C.POINTER(FeSeries), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "fe_gather_obs": (C.c_int, [C.POINTER(FeParams), C.POINTER(FeSeries), C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
+                                C.c_void_p, C.c_void_p]),
+    "fe_gather_obs_kernel_name": (C.c_char_p, [C.POINTER(FeParams), C.POINTER(FeSeries)]),
     "fe_es_params_padded": (C.c_int64, [C.POINTER(FeEsNet)]),
     "fe_es_packed_index": (C.c_int64, [C.POINTER(FeEsNet), C.c_int32, C.c_int32, C.c_int32]),
     "fe_es_perturb": (C.c_int, [C.POINTER(FeEsNet), C.c_uint64, C.c_uint64, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p]),

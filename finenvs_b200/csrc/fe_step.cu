@@ -1166,21 +1166,138 @@ fe_lazy_kernel(const FeParams p, const FeSeries s, const FeState st, const Const
     if (!kObserve) accumulate_stats(stats, r, active);
 }
 
-// handle -> tensor: warp per env, same element order as the direct variant
+// handles -> tensor (fe_gather_obs, LSU path): warp per sample, same element order as the direct variant; sample b is
+// handle index[b] (index == NULL: handle b)
 template <typename OutT>
 __global__ void __launch_bounds__(kThreads)
 fe_materialize_kernel(const int64_t N, const int W, const OutT *__restrict__ logret, const int64_t *__restrict__ row0,
-                      const OutT *__restrict__ pf, OutT *__restrict__ obs) {
+                      const OutT *__restrict__ pf, const int64_t *__restrict__ index, OutT *__restrict__ obs) {
     const int lane = threadIdx.x & 31;
     const int64_t e = ((int64_t)blockIdx.x * kThreads + threadIdx.x) >> 5;
     if (e >= N) return;
-    const OutT *src = logret + row0[e] * 4;
+    const int64_t h = index ? index[e] : e;
+    const OutT *src = logret + row0[h] * 4;
     OutT *dst = obs + (size_t)e * W * 5;
-    const OutT pfe = pf[e];
+    const OutT pfe = pf[h];
     for (int f = lane; f < W * 5; f += 32) {
         const int j = f / 5, c = f - j * 5;
         dst[f] = c == 4 ? pfe : __ldg(src + j * 4 + c);
     }
+}
+
+// handles -> tensor (fe_gather_obs, TMA path): the gather variant's movers without its bookkeepers.  Every warp is
+// autonomous: it owns the 32-sample tiles gw, gw + NW, ... (gw = global warp id, NW = warps in the grid) and a private
+// ring of S slots.  Lane l of the warp holds the handle of sample l of the tile being stored (as {tensor row index,
+// position feature}) and, loaded one tile ahead, of the next one.  A unit = one gather4 = 4 samples (2 for windows
+// fetched in two parts); per unit: wait for the slot's mbarrier -> the position-feature column -> proxy fence -> one
+// bulk store of the unit's contiguous output bytes -> (once the store has read the slot) the gather of unit i + S.
+// In the ragged last tile the missing samples repeat the last valid handle, so a gather4 always has 4 valid rows, and
+// the store covers only the valid samples.
+constexpr int kGoMaxWarps = 16;
+constexpr int kGoBarBytes = kGoMaxWarps * kGaMaxStages * 8; // one mbarrier per slot
+
+template <typename OutT, int kParts>
+__global__ void __launch_bounds__(kGoMaxWarps * 32)
+fe_gather_obs_kernel(const __grid_constant__ CUtensorMap tmap, const int64_t count, const int W, const int64_t *__restrict__ row0,
+                     const OutT *__restrict__ pf, const int64_t *__restrict__ index, OutT *__restrict__ obs, const int S,
+                     const int rows_per_phase) {
+    constexpr bool kF64 = sizeof(OutT) == 8;
+    constexpr int kUnitEnvs = 4 / kParts;      // samples per unit
+    constexpr int kTileUnits = 32 / kUnitEnvs; // units per 32-sample tile: 8 or 16 (> S: a refill is at most one tile ahead)
+    constexpr int kRounds = (kParts == 1 && kF64) ? 2 : 4; // ceil(W / 32) for the largest W ga_parts() admits
+    static_assert(kParts == 1 || kParts == 2, "a window is fetched in one or two parts");
+    extern __shared__ __align__(128) unsigned char smem[];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
+    const uint32_t pitch = ga_slot_pitch(W, kF64);
+    const uint32_t bars = smem_u32(smem) + 8u * (uint32_t)(warp * S);
+    unsigned char *slots = smem + kGoBarBytes + (size_t)warp * S * pitch;
+    const uint32_t row_b = (uint32_t)ga_row_bytes(kF64) * W, unit_b = kUnitEnvs * row_b; // row_b: one window
+    const int part_rows = (int)(row_b / 2) / kGaPitch; // two parts: tensor rows from a window's first half to its second
+    const int shift = ga_phase_shift(kF64);
+    const int64_t gw = (int64_t)blockIdx.x * nwarps + warp, NW = (int64_t)gridDim.x * nwarps;
+    const int64_t ntiles = (count + 31) / 32;
+    if (gw >= ntiles) return;
+    const int64_t my_tiles = (ntiles - gw + NW - 1) / NW;
+    const int64_t last_tile = gw + (my_tiles - 1) * NW;
+    const int last_units = (int)(((count - last_tile * 32 < 32 ? count - last_tile * 32 : 32) + kUnitEnvs - 1) / kUnitEnvs);
+    const int64_t n_units = (my_tiles - 1) * kTileUnits + last_units;
+
+    if (lane == 0) {
+        for (int si = 0; si < S; ++si) mbar_init(bars + 8u * si, 1);
+        mbar_fence_init();
+    }
+    __syncwarp();
+
+    auto load = [&](int64_t k, int &row, OutT &v) { // handle of sample `lane` of this warp's k-th tile
+        int64_t b = (gw + k * NW) * 32 + lane;
+        if (b >= count) b = count - 1;
+        const int64_t h = index ? __ldg(index + b) : b;
+        const int64_t r0 = __ldg(row0 + h);
+        v = __ldg(pf + h);
+        row = (int)((r0 & ((1 << shift) - 1)) * rows_per_phase + (r0 >> shift)); // copy (row0 mod P), row (row0 div P)
+    };
+    int cur_row = 0, nxt_row = 0;
+    OutT cur_pf = 0, nxt_pf = 0;
+    int64_t kc = 0; // tile (of this warp's) whose units are being stored
+    load(0, cur_row, cur_pf);
+    if (my_tiles > 1) load(1, nxt_row, nxt_pf);
+    const uint64_t keep = l2_policy_evict_last(), stream_out = l2_policy_evict_first();
+
+    auto issue = [&](int64_t j) { // whole warp (shuffles); lane 0 issues the gather of unit j into slot j % S
+        const int src = (j / kTileUnits == kc) ? cur_row : nxt_row;
+        const int g = (int)(j % kTileUnits);
+        int4 rows4;
+        if constexpr (kParts == 1) {
+            rows4 = make_int4(__shfl_sync(0xFFFFFFFFu, src, 4 * g), __shfl_sync(0xFFFFFFFFu, src, 4 * g + 1),
+                              __shfl_sync(0xFFFFFFFFu, src, 4 * g + 2), __shfl_sync(0xFFFFFFFFu, src, 4 * g + 3));
+        } else { // (first half, second half) of sample 2g, then of sample 2g + 1
+            const int a = __shfl_sync(0xFFFFFFFFu, src, 2 * g), b = __shfl_sync(0xFFFFFFFFu, src, 2 * g + 1);
+            rows4 = make_int4(a, a + part_rows, b, b + part_rows);
+        }
+        if (lane == 0) {
+            const int si = (int)(j % S);
+            mbar_arrive_expect_tx(bars + 8u * si, unit_b);
+            tma_gather4(smem_u32(slots + (size_t)si * pitch), &tmap, rows4.x, rows4.y, rows4.z, rows4.w, bars + 8u * si, keep);
+        }
+    };
+    for (int64_t j = 0; j < S && j < n_units; ++j) issue(j);
+
+    // position-feature column: sample e of a unit owns rows [eW, (e+1)W) of the slot; this lane writes rows eW + lane + 32k
+    uint32_t round_mask = 0; // bit k: lane + 32k < W
+#pragma unroll
+    for (int kk = 0; kk < kRounds; ++kk) round_mask |= (uint32_t)(lane + 32 * kk < W) << kk;
+    const uint32_t env_stride = (uint32_t)W * 5; // values per sample
+    for (int64_t j = 0; j < n_units; ++j) {
+        if (j / kTileUnits != kc) { // next tile: its handles arrived a tile ago; fetch the one after it
+            kc = j / kTileUnits;
+            cur_row = nxt_row; cur_pf = nxt_pf;
+            if (kc + 1 < my_tiles) load(kc + 1, nxt_row, nxt_pf);
+        }
+        const int si = (int)(j % S), g = (int)(j % kTileUnits);
+        if (lane == 0) mbar_wait(bars + 8u * si, (uint32_t)((j / S) & 1)); // the unit's windows have landed
+        __syncwarp();
+        unsigned char *slot = slots + (size_t)si * pitch;
+        OutT *col = reinterpret_cast<OutT *>(slot) + 5 * lane + 4; // position-feature slot of row `lane` of sample 0
+#pragma unroll
+        for (int e = 0; e < kUnitEnvs; ++e) {
+            const OutT v = __shfl_sync(0xFFFFFFFFu, cur_pf, kUnitEnvs * g + e);
+#pragma unroll
+            for (int kk = 0; kk < kRounds; ++kk)
+                if (round_mask & (1u << kk)) col[e * env_stride + 160 * kk] = v;
+        }
+        fence_proxy_async_smem(); // generic-proxy writes -> visible to the bulk store
+        __syncwarp();
+        if (lane == 0) {
+            const int64_t b0 = (gw + kc * NW) * 32 + (int64_t)kUnitEnvs * g;
+            const int nv = count - b0 >= kUnitEnvs ? kUnitEnvs : (int)(count - b0); // fewer only in the ragged last tile
+            bulk_store_hint(obs + (size_t)b0 * W * 5, smem_u32(slot), (uint32_t)nv * row_b, stream_out);
+            bulk_commit();
+            if (j + S < n_units) bulk_wait_read_all(); // the store has read the slot: it can be refilled
+        }
+        __syncwarp();
+        if (j + S < n_units) issue(j + S);
+    }
+    if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); // stores complete before the warp exits
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1961,6 +2078,59 @@ int launch(const FeParams &p, const FeSeries &s, const FeState &st, const float 
     return (int)cudaGetLastError();
 }
 
+// handles -> tensor (fe_gather_obs / fe_materialize).  TMA path while the gather variant could serve this window from an
+// L2-resident observation-layout table; the warp-per-sample copy otherwise (and for an output or table that is not 16-byte
+// aligned, which only fe_materialize accepts).
+enum ObsPath { OBS_NONE, OBS_TMA, OBS_LSU };
+ObsPath choose_obs_path(const FeParams &p, const FeSeries &s) {
+    if (p.num_assets != 1) return OBS_NONE;
+    const bool f64 = p.out_f64 != 0;
+    return s.obs_table && ga_parts(p.window, f64) > 0 && gather_table_resident(p, f64) ? OBS_TMA : OBS_LSU;
+}
+
+template <typename OutT>
+int gather_obs(const FeParams &p, const FeSeries &s, const int64_t *row0, const void *pf, const int64_t *index, int64_t count,
+               void *obs, cudaStream_t stream) {
+    constexpr bool f64 = sizeof(OutT) == 8;
+    if (choose_obs_path(p, s) != OBS_TMA || (((uintptr_t)obs | (uintptr_t)s.obs_table) & 15)) {
+        const int64_t blocks = (count * 32 + kThreads - 1) / kThreads;
+        fe_materialize_kernel<OutT><<<(unsigned)blocks, kThreads, 0, stream>>>(count, p.window, (const OutT *)s.logret, row0,
+                                                                               (const OutT *)pf, index, (OutT *)obs);
+        return (int)cudaGetLastError();
+    }
+    int sms = 0;
+    int rc = device_sm_count(p.device, &sms);
+    if (rc) return rc;
+    const int64_t rpp = ga_rows_per_phase(p.num_rows, p.window, f64);
+    const int parts = ga_parts(p.window, f64);
+    CUtensorMap tmap;
+    if ((rc = gather_tensor_map(s.obs_table, rpp << ga_phase_shift(f64), ga_row_bytes(f64) * p.window / parts, p.device, &tmap)))
+        return rc;
+    // 3 slots per warp when at least 8 warps of them fit in shared memory, else 2; up to 16 warps per block and, for short
+    // windows whose rings are small, up to 4 blocks per SM
+    const size_t pitch = ga_slot_pitch(p.window, f64), room = (size_t)kSmemMax - kGoBarBytes;
+    int S = 3;
+    if (room / (S * pitch) < 8) S = 2;
+    const int warps = (int)(room / (S * pitch) < (size_t)kGoMaxWarps ? room / (S * pitch) : kGoMaxWarps);
+    const size_t smem = kGoBarBytes + (size_t)warps * S * pitch;
+    int per_sm = (int)((size_t)(228 * 1024) / (smem + 1024));
+    per_sm = per_sm < 1 ? 1 : per_sm > 4 ? 4 : per_sm;
+    const int64_t need = ((count + 31) / 32 + warps - 1) / warps;
+    const unsigned blocks = (unsigned)(need < (int64_t)sms * per_sm ? need : (int64_t)sms * per_sm);
+    if (parts == 1) {
+        auto kern = fe_gather_obs_kernel<OutT, 1>;
+        static std::atomic<uint32_t> configured{0};
+        if ((rc = opt_in_smem(kern, configured, p.device))) return rc;
+        kern<<<blocks, warps * 32, smem, stream>>>(tmap, count, p.window, row0, (const OutT *)pf, index, (OutT *)obs, S, (int)rpp);
+    } else {
+        auto kern = fe_gather_obs_kernel<OutT, 2>;
+        static std::atomic<uint32_t> configured{0};
+        if ((rc = opt_in_smem(kern, configured, p.device))) return rc;
+        kern<<<blocks, warps * 32, smem, stream>>>(tmap, count, p.window, row0, (const OutT *)pf, index, (OutT *)obs, S, (int)rpp);
+    }
+    return (int)cudaGetLastError();
+}
+
 // step ordinal kept on the device (fe_step_captured): one thread bumps it ahead of the step kernel
 __global__ void fe_bump_kernel(uint64_t *counter) { *counter += 1; }
 
@@ -2173,14 +2343,30 @@ int fe_materialize(const FeParams *p, const FeSeries *s, const int64_t *obs_row0
     if (p->num_envs <= 0 || p->window <= 0 || p->num_assets != 1) return FE_EINVAL;
     DeviceGuard guard(p->device);
     if (guard.rc) return guard.rc;
-    const unsigned blocks = (unsigned)((p->num_envs * 32 + kThreads - 1) / kThreads);
-    if (p->out_f64)
-        fe_materialize_kernel<double><<<blocks, kThreads, 0, (cudaStream_t)stream>>>(
-            p->num_envs, p->window, (const double *)s->logret, obs_row0_dev, (const double *)obs_posfeat_dev, (double *)obs_dev);
-    else
-        fe_materialize_kernel<float><<<blocks, kThreads, 0, (cudaStream_t)stream>>>(
-            p->num_envs, p->window, (const float *)s->logret, obs_row0_dev, (const float *)obs_posfeat_dev, (float *)obs_dev);
-    return (int)cudaGetLastError();
+    return p->out_f64 ? gather_obs<double>(*p, *s, obs_row0_dev, obs_posfeat_dev, nullptr, p->num_envs, obs_dev, (cudaStream_t)stream)
+                      : gather_obs<float>(*p, *s, obs_row0_dev, obs_posfeat_dev, nullptr, p->num_envs, obs_dev, (cudaStream_t)stream);
+}
+
+int fe_gather_obs(const FeParams *p, const FeSeries *s, const int64_t *row0_dev, const void *posfeat_dev,
+                  const int64_t *index_dev, int64_t count, void *obs_dev, void *stream) {
+    if (!p || !s || !s->logret || !row0_dev || !posfeat_dev || !obs_dev || count < 0) return FE_EINVAL;
+    if (p->window <= 0 || p->num_assets != 1) return FE_EINVAL;
+    if (((uintptr_t)obs_dev | (uintptr_t)s->obs_table) & 15) return FE_EALIGN;
+    if (count == 0) return 0;
+    DeviceGuard guard(p->device);
+    if (guard.rc) return guard.rc;
+    return p->out_f64 ? gather_obs<double>(*p, *s, row0_dev, posfeat_dev, index_dev, count, obs_dev, (cudaStream_t)stream)
+                      : gather_obs<float>(*p, *s, row0_dev, posfeat_dev, index_dev, count, obs_dev, (cudaStream_t)stream);
+}
+
+const char *fe_gather_obs_kernel_name(const FeParams *p, const FeSeries *s) {
+    if (!p || !s) return "";
+    const bool f64 = p->out_f64 != 0;
+    switch (choose_obs_path(*p, *s)) {
+    case OBS_TMA: return f64 ? "fe_gather_obs_kernel<double>" : "fe_gather_obs_kernel<float>";
+    case OBS_LSU: return f64 ? "fe_materialize_kernel<double>" : "fe_materialize_kernel<float>";
+    default: return "none (handles exist for single-asset series only)";
+    }
 }
 
 // Host-buffer step, pipelined: the envs are cut into chunks (multiples of 1024 envs, so every chunk's slice of

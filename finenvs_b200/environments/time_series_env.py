@@ -139,6 +139,9 @@ class CapturedRollout:
 
 
 class TimeSeriesEnv(BaseObject):
+    _obs_ring = None      # Buffer bound with bind_env(env): observations are written into its states slots
+    _handle_ring = None   # Buffer bound with bind_env(env, lazy=True): it keeps the observations' handles
+
     def __init__(
         self,
         instrument_name: str,
@@ -377,6 +380,8 @@ class TimeSeriesEnv(BaseObject):
 
     def reset(self) -> torch.Tensor:
         """:423-435 — materialises the current observation; touches no state (reference semantics)."""
+        if self._handle_ring is not None:
+            return self._observe_via_handle(None, for_reset=True)
         obs = self._new_obs(for_reset=True)
         _lib.check(self._L.fe_observe(self._pp, self._ps, self._pst, obs.data_ptr(), self._stream()), "fe_observe")
         return obs
@@ -394,10 +399,13 @@ class TimeSeriesEnv(BaseObject):
     def step(self, actions: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, dict]:
         """:277-296 — one kernel launch, no host synchronisation in training mode."""
         actions = self._prepare_actions(actions)
-        obs = self._new_obs()
         rewards = torch.empty(self.num_envs, dtype=self.obs_dtype, device=self._dev)
         dones = torch.empty(self.num_envs, dtype=torch.int32, device=self._dev)
-        self.step_into(actions, obs, rewards, dones)
+        if self._handle_ring is not None:
+            obs = self._observe_via_handle((actions, rewards, dones), for_reset=False)
+        else:
+            obs = self._new_obs()
+            self.step_into(actions, obs, rewards, dones)
         info_dict = self.record_evaluation_metrics() if self.evaluate else {}
         return (obs, rewards, dones, info_dict)
 
@@ -440,6 +448,52 @@ class TimeSeriesEnv(BaseObject):
         )
         info_dict = self.record_evaluation_metrics() if self.evaluate else {}
         return (lo, rewards, dones, info_dict)
+
+    # ------------------------------------------------------------------ rollout buffer that keeps handles ----
+    def _bind_handle_ring(self, ring) -> None:
+        """Buffer.bind_env(env, lazy=True): reset() / step() write each observation's handle into the buffer's next handle
+        slot (fe_observe_lazy / fe_step_lazy) and return the dense tensor fe_gather_obs builds from it.  fe_gather_obs
+        calls get their own FeSeries carrying the series' observation-layout table (built here once per series when it
+        stays L2-resident) so that they take the TMA path; the step kernel's FeSeries, and with it `auto`, is unchanged."""
+        if self.num_assets != 1:
+            raise NotImplementedError("lazy observations are implemented for single-asset envs")
+        s = self.series
+        table = s.obs_table()
+        self._gather_cseries = _lib.FeSeries(s.prices.data_ptr(), s.logret.data_ptr(), s.seg_start.data_ptr(),
+                                             s.seg_len.data_ptr(), table.data_ptr() if table is not None else None)
+        self._pgs = C.byref(self._gather_cseries)
+        self._obs_ring, self._handle_ring = None, ring
+
+    def gather_obs_kernel_name(self) -> str:
+        """Which kernel fe_gather_obs launches for this env once bound to a buffer with bind_env(env, lazy=True)."""
+        return self._L.fe_gather_obs_kernel_name(self._pp, self._pgs).decode()
+
+    def gather_obs(self, row0: torch.Tensor, posfeat: torch.Tensor, index: Optional[torch.Tensor], out: torch.Tensor) -> None:
+        """out[b] = the observation of handle index[b] (index None: handle b), b < out.shape[0] (fe_gather_obs).  The index
+        values must lie in [0, row0.numel())."""
+        _lib.check(self._L.fe_gather_obs(self._pp, self._pgs, row0.data_ptr(), posfeat.data_ptr(),
+                                         index.data_ptr() if index is not None else None, out.shape[0], out.data_ptr(),
+                                         self._stream()), "fe_gather_obs")
+
+    def _observe_via_handle(self, step_args, for_reset: bool) -> torch.Tensor:
+        row0, posfeat = self._handle_ring.next_handle_slot(self.num_envs, self.obs_dtype, for_reset)
+        if step_args is None:
+            _lib.check(self._L.fe_observe_lazy(self._pp, self._ps, self._pst, row0.data_ptr(), posfeat.data_ptr(),
+                                               self._stream()), "fe_observe_lazy")
+        else:
+            actions, rewards, dones = step_args
+            self.step_count += 1
+            _lib.check(
+                self._L.fe_step_lazy(self._pp, self._ps, self._pst, actions.data_ptr(), row0.data_ptr(), posfeat.data_ptr(),
+                                     rewards.data_ptr(), dones.data_ptr(), self._stats_ptr, self.step_count, self._stream()),
+                "fe_step_lazy",
+            )
+        shape = ((self.num_envs, self.num_intervals * self.num_obs) if self.flat_obs
+                 else (self.num_envs, self.num_intervals, self.num_obs))
+        obs = torch.empty(shape, dtype=self.obs_dtype, device=self._dev)
+        self.gather_obs(row0, posfeat, None, obs)
+        self._handle_ring.hand_out(obs)
+        return obs
 
     def step_host(self, actions_host: torch.Tensor, packed_dones: bool = False) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, dict]:
         """step() for a host-resident policy, through fe_step_host: `actions_host` is a CPU tensor

@@ -172,6 +172,17 @@ int fe_step_lazy(const FeParams *p, const FeSeries *s, const FeState *st, const 
                  void *stream);
 int fe_materialize(const FeParams *p, const FeSeries *s, const int64_t *obs_row0_dev, const void *obs_posfeat_dev,
                    void *obs_dev, void *stream);
+/* obs[b] = the observation described by handle index[b] (index_dev == NULL: handle b), b < count; (count, W, 5) written
+ * contiguously to obs_dev (16-byte aligned).  Bit-identical to what fe_step / fe_materialize write for the same handle.
+ * Single-asset series only.  Index values are the caller's responsibility (like fe_materialize's handles).  A rollout
+ * buffer keeps the 12-byte handles and builds shuffled minibatches with this call.  Two paths: while s->obs_table is
+ * staged for this window and L2-resident (as for the gather variant), windows arrive by TMA gather4 (four samples, or
+ * two for windows fetched in two parts, per instruction) and leave by bulk stores; otherwise a warp per sample copies
+ * from s->logret.  fe_materialize is this call with index_dev == NULL and count = p->num_envs.  count == 0: nothing is
+ * launched. */
+int fe_gather_obs(const FeParams *p, const FeSeries *s, const int64_t *row0_dev, const void *posfeat_dev,
+                  const int64_t *index_dev, int64_t count, void *obs_dev, void *stream);
+const char *fe_gather_obs_kernel_name(const FeParams *p, const FeSeries *s); /* which path; host-only, for tests */
 
 /* Same step driven from HOST buffers (the call a non-torch embedder makes).  When actions_host, rewards_host and
  * dones_host are all pinned (cudaHostAlloc / cudaHostRegister), the step kernel itself reads the actions from and
