@@ -112,6 +112,7 @@ _PROTOTYPES = {
     "fe_es_forward": (C.c_int, [C.POINTER(FeEsNet), C.c_void_p, C.c_void_p, C.c_float, C.c_int64, C.c_int64, C.c_void_p,
                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_float, C.c_uint64, C.c_uint64,
                                 C.c_int64, C.c_void_p, C.c_int32, C.c_void_p]),
+    "fe_es_forward_kernel_name": (C.c_char_p, [C.POINTER(FeEsNet), C.c_int32, C.c_int32]),
     "fe_es_gradient_scratch": (C.c_int64, [C.POINTER(FeEsNet), C.c_int64]),
     "fe_es_gradient": (C.c_int, [C.POINTER(FeEsNet), C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
     "fe_es_store": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_uint64, C.c_void_p,

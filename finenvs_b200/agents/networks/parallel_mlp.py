@@ -199,6 +199,11 @@ class ParallelMLP(BaseObject):
         )
         return actions
 
+    def forward_kernel_name(self, lazy: bool = True, obs_aligned: bool = True) -> str:
+        """Which fe_es_forward kernel `forward` launches for this network (and its launch shape); host-only.
+        `obs_aligned`: a dense input starts on a 16-byte boundary (freshly allocated tensors do)."""
+        return self._L.fe_es_forward_kernel_name(self._pnet, int(lazy), int(obs_aligned)).decode()
+
     # ------------------------------------------------------------------ perturbations (:112-174)
     def perturb_parameters(self) -> None:
         """:112-155 — new mirrored perturbations for every pair (a new `generation` of the keyed stream)."""

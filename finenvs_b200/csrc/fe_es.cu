@@ -26,6 +26,7 @@
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <stdio.h>
 #include <stdlib.h>
 
 #include <atomic>
@@ -833,6 +834,79 @@ fe_es_store_kernel(const RewT *__restrict__ rewards, const int32_t *__restrict__
     }
 }
 
+// ------------------------------------------------------------------------------------------
+// forward routing: which of the three kernels runs a network, and its launch shape.  A host function of the layout
+// alone (no device attribute), shared by fe_es_forward and fe_es_forward_kernel_name so the two cannot disagree.
+// ------------------------------------------------------------------------------------------
+enum EsKern { ES_FAST, ES_STREAM, ES_GENERIC, ES_ERR_SMEM };
+struct EsRoute {
+    EsKern kern;
+    size_t smem;     // dynamic shared memory of the launch
+    FastShape fast;  // ES_FAST
+    StreamShape stream; // ES_STREAM
+    bool theta_smem; // ES_GENERIC: theta staged in shared memory (else read from global memory)
+};
+
+// obs_aligned: dense observations start on a 16-byte boundary (always true for lazy handles)
+EsRoute route_forward(const EsLayout &lay, const bool lazy, const bool obs_aligned) {
+    EsRoute rt{};
+    const int64_t P = lay.off[lay.L];
+    // ---- fast path: 5R -> <= 8 first layer (R <= 63), inputs 16-byte granular, ring fits in shared memory
+    const bool no_fast = env_override("FE_ES_NO_FAST") != 0; // A/B runs (experiment builds only)
+    if (!no_fast && lay.out[0] <= 8 && lay.in[0] % 5 == 0 && lay.in[0] / 5 <= 63 &&
+        (lazy || (lay.in[0] % 4 == 0 && obs_aligned))) {
+        FastShape &f = rt.fast;
+        f.rows = lay.in[0] / 5;
+        f.x_bytes = lazy ? f.rows * 16 : f.rows * 20;
+        f.eps_bytes = (int)(P * 2);
+        f.stage_bytes = (f.eps_bytes + 2 * f.x_bytes + 16 + 127) & ~127;
+        int md = 1;
+        for (int l = 1; l <= lay.L; ++l) md = lay.out[l - 1] > md ? lay.out[l - 1] : md;
+        f.act_stride = (md + 1 + 3) & ~3;
+        f.tail_in_regs = lay.L == 2 && lay.out[1] <= 8;
+        f.theta_bytes = (int)((P * 4 + 127) & ~(int64_t)127);
+        rt.smem = fast_smem_bytes(f);
+        if (rt.smem <= 226 * 1024) {
+            rt.kern = ES_FAST;
+            return rt;
+        }
+    }
+    // ---- streaming path: every layer has <= 319 inputs, eps chunks 16-byte granular (always), ring + activations fit
+    const bool no_stream = env_override("FE_ES_NO_STREAM") != 0;
+    bool stream_ok = !no_stream;
+    for (int l = 0; l < lay.L; ++l) stream_ok = stream_ok && lay.in[l] + 1 <= 32 * kStRows;
+    if (stream_ok) {
+        StreamShape &f = rt.stream;
+        int max_in1 = 0, a = 0, b = 0;
+        f.chunks[0] = 0;
+        for (int l = 0; l < lay.L; ++l) {
+            if (lay.in[l] + 1 > max_in1) max_in1 = lay.in[l] + 1;
+            f.chunks[l + 1] = f.chunks[l] + (lay.out[l] + 7) / 8;
+            // buffer A holds the inputs of even layers (and the outputs of odd ones), buffer B the others
+            const int need_in = lay.in[l] + 1, need_out = lay.out[l] + 1;
+            if (l % 2 == 0) { a = need_in > a ? need_in : a; b = need_out > b ? need_out : b; }
+            else { b = need_in > b ? need_in : b; a = need_out > a ? need_out : a; }
+        }
+        f.stage_bytes = (max_in1 * 16 + 127) & ~127;
+        f.strideA = (a + 1) & ~1;
+        f.strideB = (b + 1) & ~1;
+        f.U = kStMaxU;
+        while (f.U > 1 && stream_smem_bytes(f) > 226 * 1024) --f.U;
+        rt.smem = stream_smem_bytes(f);
+        if (rt.smem <= 226 * 1024) {
+            rt.kern = ES_STREAM;
+            return rt;
+        }
+    }
+    // ---- generic kernel: theta in shared memory while the block stays small enough for >= 2 blocks per SM
+    const int stride = (lay.max_dim + 1 + 3) & ~3;
+    const size_t act_bytes = (size_t)kEsWarps * 4 * stride * sizeof(float);
+    rt.theta_smem = act_bytes + (size_t)P * sizeof(float) <= 100 * 1024;
+    rt.smem = act_bytes + (rt.theta_smem ? (size_t)P * sizeof(float) : 0);
+    rt.kern = rt.smem <= 226 * 1024 ? ES_GENERIC : ES_ERR_SMEM;
+    return rt;
+}
+
 } // namespace
 
 extern "C" {
@@ -877,6 +951,8 @@ int fe_es_forward(const FeEsNet *net, const float *theta_packed_dev, const void 
         if ((uintptr_t)logret_dev & 15) return FE_EALIGN;
     }
     if (((uintptr_t)eps_dev | (uintptr_t)theta_packed_dev) & 15) return FE_EALIGN;
+    const EsRoute rt = route_forward(lay, lazy, lazy || ((uintptr_t)obs_dev & 15) == 0);
+    if (rt.kern == ES_ERR_SMEM) return FE_ESMEM;
     cudaError_t e;
     DeviceGuard guard(device);
     if (guard.rc) return guard.rc;
@@ -888,88 +964,65 @@ int fe_es_forward(const FeEsNet *net, const float *theta_packed_dev, const void 
         if ((e = cudaDeviceGetAttribute(&num_sms[dev], cudaDevAttrMultiProcessorCount, device)) != cudaSuccess) return (int)e;
         num_sms_cache[dev].store(num_sms[dev], std::memory_order_relaxed);
     }
-    const int64_t P = lay.off[lay.L];
-    // ---- fast path: 5R -> <= 8 first layer (R <= 64), inputs 16-byte granular, ring fits in shared memory
-    const bool no_fast = env_override("FE_ES_NO_FAST") != 0; // A/B runs (experiment builds only)
-    if (!no_fast && lay.out[0] <= 8 && lay.in[0] % 5 == 0 && lay.in[0] / 5 <= 63 &&
-        (lazy || (lay.in[0] % 4 == 0 && ((uintptr_t)obs_dev & 15) == 0))) {
-        FastShape f;
-        f.rows = lay.in[0] / 5;
-        f.x_bytes = lazy ? f.rows * 16 : f.rows * 20;
-        f.eps_bytes = (int)(P * 2);
-        f.stage_bytes = (f.eps_bytes + 2 * f.x_bytes + 16 + 127) & ~127;
-        int md = 1;
-        for (int l = 1; l <= lay.L; ++l) md = lay.out[l - 1] > md ? lay.out[l - 1] : md;
-        f.act_stride = (md + 1 + 3) & ~3;
-        f.tail_in_regs = lay.L == 2 && lay.out[1] <= 8;
-        f.theta_bytes = (int)((P * 4 + 127) & ~(int64_t)127);
-        const size_t smem = fast_smem_bytes(f);
-        if (smem <= 226 * 1024) {
-            auto kern = lazy ? fe_es_forward_fast_kernel<true> : fe_es_forward_fast_kernel<false>;
-            if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return (int)e;
-            const int64_t units = train / 2 + num_eval_envs;
-            int64_t blocks = (units + kFastWarps - 1) / kFastWarps;
-            if (blocks > num_sms[dev]) blocks = num_sms[dev];
-            kern<<<(unsigned)blocks, kFastThreads, smem, (cudaStream_t)stream>>>(
-                lay, f, theta_packed_dev, (const __half *)eps_dev, sigma, train / 2, num_eval_envs, obs_dev,
-                (const float *)logret_dev, obs_row0_dev, obs_posfeat_dev, action_noise_std, seed, step_counter, env_id_base,
-                actions_dev);
-            return (int)cudaGetLastError();
-        }
-    }
-    // ---- streaming path: every layer has <= 319 inputs, eps chunks 16-byte granular (always), ring + activations fit
-    const bool no_stream = env_override("FE_ES_NO_STREAM") != 0;
-    bool stream_ok = !no_stream;
-    for (int l = 0; l < lay.L; ++l) stream_ok = stream_ok && lay.in[l] + 1 <= 32 * kStRows;
-    if (stream_ok) {
-        StreamShape f;
-        int max_in1 = 0, a = 0, b = 0;
-        f.chunks[0] = 0;
-        for (int l = 0; l < lay.L; ++l) {
-            if (lay.in[l] + 1 > max_in1) max_in1 = lay.in[l] + 1;
-            f.chunks[l + 1] = f.chunks[l] + (lay.out[l] + 7) / 8;
-            // buffer A holds the inputs of even layers (and the outputs of odd ones), buffer B the others
-            const int need_in = lay.in[l] + 1, need_out = lay.out[l] + 1;
-            if (l % 2 == 0) { a = need_in > a ? need_in : a; b = need_out > b ? need_out : b; }
-            else { b = need_in > b ? need_in : b; a = need_out > a ? need_out : a; }
-        }
-        f.stage_bytes = (max_in1 * 16 + 127) & ~127;
-        f.strideA = (a + 1) & ~1;
-        f.strideB = (b + 1) & ~1;
-        f.U = kStMaxU;
-        while (f.U > 1 && stream_smem_bytes(f) > 226 * 1024) --f.U;
-        if (stream_smem_bytes(f) <= 226 * 1024) {
-            const size_t smem = stream_smem_bytes(f);
-            auto kern = lazy ? fe_es_forward_stream_kernel<true> : fe_es_forward_stream_kernel<false>;
-            if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return (int)e;
-            const int64_t units = train / 2 + num_eval_envs;
-            int64_t blocks = (units + (int64_t)kStWarps * f.U - 1) / ((int64_t)kStWarps * f.U);
-            if (blocks > num_sms[dev]) blocks = num_sms[dev];
-            kern<<<(unsigned)blocks, kStThreads, smem, (cudaStream_t)stream>>>(
-                lay, f, theta_packed_dev, (const __half *)eps_dev, sigma, train / 2, num_eval_envs, obs_dev,
-                (const float *)logret_dev, obs_row0_dev, obs_posfeat_dev, window, action_noise_std, seed, step_counter,
-                env_id_base, actions_dev);
-            return (int)cudaGetLastError();
-        }
-    }
-    const int stride = (lay.max_dim + 1 + 3) & ~3;
-    const size_t act_bytes = (size_t)kEsWarps * 4 * stride * sizeof(float);
-    const bool theta_smem = act_bytes + (size_t)P * sizeof(float) <= 100 * 1024; // keep >= 2 blocks per SM
-    const size_t smem = act_bytes + (theta_smem ? (size_t)P * sizeof(float) : 0);
-    if (smem > 226 * 1024) return FE_ESMEM;
-    auto kern = lazy ? (theta_smem ? fe_es_forward_kernel<true, true> : fe_es_forward_kernel<true, false>)
-                     : (theta_smem ? fe_es_forward_kernel<false, true> : fe_es_forward_kernel<false, false>);
-    if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return (int)e;
     const int64_t units = train / 2 + num_eval_envs;
-    int per_sm = (int)((226 * 1024) / (smem + 1024));
+    if (rt.kern == ES_FAST) {
+        auto kern = lazy ? fe_es_forward_fast_kernel<true> : fe_es_forward_fast_kernel<false>;
+        if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rt.smem)) != cudaSuccess) return (int)e;
+        int64_t blocks = (units + kFastWarps - 1) / kFastWarps;
+        if (blocks > num_sms[dev]) blocks = num_sms[dev];
+        kern<<<(unsigned)blocks, kFastThreads, rt.smem, (cudaStream_t)stream>>>(
+            lay, rt.fast, theta_packed_dev, (const __half *)eps_dev, sigma, train / 2, num_eval_envs, obs_dev,
+            (const float *)logret_dev, obs_row0_dev, obs_posfeat_dev, action_noise_std, seed, step_counter, env_id_base,
+            actions_dev);
+        return (int)cudaGetLastError();
+    }
+    if (rt.kern == ES_STREAM) {
+        auto kern = lazy ? fe_es_forward_stream_kernel<true> : fe_es_forward_stream_kernel<false>;
+        if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rt.smem)) != cudaSuccess) return (int)e;
+        int64_t blocks = (units + (int64_t)kStWarps * rt.stream.U - 1) / ((int64_t)kStWarps * rt.stream.U);
+        if (blocks > num_sms[dev]) blocks = num_sms[dev];
+        kern<<<(unsigned)blocks, kStThreads, rt.smem, (cudaStream_t)stream>>>(
+            lay, rt.stream, theta_packed_dev, (const __half *)eps_dev, sigma, train / 2, num_eval_envs, obs_dev,
+            (const float *)logret_dev, obs_row0_dev, obs_posfeat_dev, window, action_noise_std, seed, step_counter,
+            env_id_base, actions_dev);
+        return (int)cudaGetLastError();
+    }
+    auto kern = lazy ? (rt.theta_smem ? fe_es_forward_kernel<true, true> : fe_es_forward_kernel<true, false>)
+                     : (rt.theta_smem ? fe_es_forward_kernel<false, true> : fe_es_forward_kernel<false, false>);
+    if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rt.smem)) != cudaSuccess) return (int)e;
+    int per_sm = (int)((226 * 1024) / (rt.smem + 1024));
     if (per_sm > 8) per_sm = 8;
     if (per_sm < 1) per_sm = 1;
     int64_t blocks = (units + kEsWarps - 1) / kEsWarps;
     if (blocks > (int64_t)num_sms[dev] * per_sm) blocks = (int64_t)num_sms[dev] * per_sm;
-    kern<<<(unsigned)blocks, kEsThreads, smem, (cudaStream_t)stream>>>(
+    kern<<<(unsigned)blocks, kEsThreads, rt.smem, (cudaStream_t)stream>>>(
         lay, theta_packed_dev, (const __half *)eps_dev, sigma, train / 2, num_eval_envs, obs_dev, (const float *)logret_dev,
         obs_row0_dev, obs_posfeat_dev, window, action_noise_std, seed, step_counter, env_id_base, actions_dev);
     return (int)cudaGetLastError();
+}
+
+const char *fe_es_forward_kernel_name(const FeEsNet *net, int32_t lazy, int32_t obs_aligned) {
+    EsLayout lay;
+    if (!make_layout(net, lay)) return "";
+    const bool lz = lazy != 0;
+    const EsRoute rt = route_forward(lay, lz, lz || obs_aligned != 0);
+    // one name per (input form, U) for whatever kStMaxU the build uses (FE_ES_ST_MAXU); filled once, thread-safely
+    static const struct StreamNames {
+        char s[2][kStMaxU][48];
+        StreamNames() {
+            for (int l = 0; l < 2; ++l)
+                for (int u = 0; u < kStMaxU; ++u)
+                    snprintf(s[l][u], sizeof s[l][u], "fe_es_forward_stream_kernel<%s> U=%d", l ? "lazy" : "dense", u + 1);
+        }
+    } stream_names;
+    switch (rt.kern) {
+    case ES_FAST: return lz ? "fe_es_forward_fast_kernel<lazy>" : "fe_es_forward_fast_kernel<dense>";
+    case ES_STREAM: return stream_names.s[lz][rt.stream.U - 1];
+    case ES_GENERIC:
+        return rt.theta_smem ? (lz ? "fe_es_forward_kernel<lazy,theta_smem>" : "fe_es_forward_kernel<dense,theta_smem>")
+                             : (lz ? "fe_es_forward_kernel<lazy,theta_global>" : "fe_es_forward_kernel<dense,theta_global>");
+    default: return "none (FE_ESMEM: the network's activations do not fit in shared memory)";
+    }
 }
 
 int64_t fe_es_gradient_scratch(const FeEsNet *net, int64_t num_pairs) {

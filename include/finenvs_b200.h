@@ -262,6 +262,11 @@ int fe_es_forward(const FeEsNet *net, const float *theta_packed_dev, const void 
                   int64_t num_eval_envs, const float *obs_dev, const void *logret_dev, const int64_t *obs_row0_dev,
                   const float *obs_posfeat_dev, int32_t window, float action_noise_std, uint64_t seed,
                   uint64_t step_counter, int64_t env_id_base, float *actions_dev, int32_t device, void *stream);
+/* Which forward kernel fe_es_forward launches for this network (host-only, for tests): "fe_es_forward_fast_kernel<lazy>",
+ * "fe_es_forward_stream_kernel<dense> U=2" (U: pairs per warp), "fe_es_forward_kernel<lazy,theta_smem>" /
+ * "...,theta_global>", or "none (FE_ESMEM: ...)".  lazy: observations come as handles; obs_aligned: the dense
+ * observation pointer is 16-byte aligned (ignored when lazy).  "" for an invalid network. */
+const char *fe_es_forward_kernel_name(const FeEsNet *net, int32_t lazy, int32_t obs_aligned);
 
 /* update_parameters' reduction (:176-218): grad_packed[q] = sum_p pair_weights[p] * eps[p, q] (pair_weights =
  * fitness(+) - fitness(-)); deterministic.  scratch_dev: fe_es_gradient_scratch(net, num_pairs) floats. */
