@@ -72,6 +72,17 @@ class FeEsNet(C.Structure):
 # FeStats as a flat tensor: 4 x u64 then 2 x f64 = 48 bytes
 STATS_BYTES = 48
 
+# FeMetricsSummary as a flat tensor: 2 x u64 then 6 x f64 = 64 bytes
+METRICS_SUMMARY_KEYS = ("episodes", "sum_len", "sum_return", "sum_sharpe", "sum_sharpe_sq", "sum_mdd", "max_mdd",
+                        "sum_hit_rate")
+METRICS_SUMMARY_BYTES = 64
+
+
+class FeMetricsState(C.Structure):
+    _fields_ = [(name, C.c_void_p) for name in (
+        "len", "pos", "sum", "mean", "m2", "peak", "mdd", "mdd_rel", "emitted",
+        "fin_key", "fin_env", "fin_len", "fin_return", "fin_sharpe", "fin_mdd", "fin_mdd_rel", "fin_hit_rate", "summary")]
+
 _PROTOTYPES = {
     "fe_version": (C.c_int, []),
     "fe_error_string": (C.c_char_p, [C.c_int]),
@@ -106,6 +117,8 @@ _PROTOTYPES = {
     "fe_gather_obs": (C.c_int, [C.POINTER(FeParams), C.POINTER(FeSeries), C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
                                 C.c_void_p, C.c_void_p]),
     "fe_gather_obs_kernel_name": (C.c_char_p, [C.POINTER(FeParams), C.POINTER(FeSeries)]),
+    "fe_episode_metrics": (C.c_int, [C.POINTER(FeParams), C.POINTER(FeMetricsState), C.c_void_p, C.c_void_p, C.c_uint64,
+                                     C.c_void_p, C.c_int64, C.c_void_p]),
     "fe_es_params_padded": (C.c_int64, [C.POINTER(FeEsNet)]),
     "fe_es_packed_index": (C.c_int64, [C.POINTER(FeEsNet), C.c_int32, C.c_int32, C.c_int32]),
     "fe_es_perturb": (C.c_int, [C.POINTER(FeEsNet), C.c_uint64, C.c_uint64, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p]),

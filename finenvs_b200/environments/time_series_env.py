@@ -120,6 +120,7 @@ class CapturedRollout:
                                         self._counter.data_ptr(), env._stream()),
                 "fe_step_captured",
             )
+            env._launch_metrics(self.rewards[t].data_ptr(), self.dones[t].data_ptr(), self._counter.data_ptr())
 
     def replay(self, refresh_obs: Optional[bool] = None):
         """Run the captured num_steps steps.  `refresh_obs=True` first rebuilds `obs` from the env's current state
@@ -167,6 +168,8 @@ class TimeSeriesEnv(BaseObject):
         variant: str = "auto",
         flat_obs: bool = False,
         num_eval_envs: Optional[int] = None,
+        track_metrics: bool = False,
+        metrics_capacity: Optional[int] = None,
     ):
         """Reference arguments: :15-29.  Extensions:
 
@@ -191,6 +194,11 @@ class TimeSeriesEnv(BaseObject):
                       (parallel_mlp.py:98-103); same memory, only the shape differs.
         num_eval_envs reported in get_env_args() for the ES agent (evo_agent.py:53); the last
                       num_eval_envs envs are the evaluation envs by the reference's convention.
+        track_metrics record per-episode trading metrics on the device after every step (fe_episode_metrics: length,
+                      return, per-step Sharpe ratio, max drawdown absolute and relative to peak equity, hit rate; see
+                      episode_metrics(), metrics_summary()).  Off: no extra launch.
+        metrics_capacity  entries of the finished-episode list (default: num_envs in evaluate mode, where an env records
+                      only its first episode between metric resets; else max(8 * num_envs, 65536)).
         """
         if obs_dtype not in (torch.float32, torch.float64):
             raise ValueError("obs_dtype must be torch.float32 or torch.float64")
@@ -235,6 +243,8 @@ class TimeSeriesEnv(BaseObject):
         self.track_stats = bool(track_stats)
         self.flat_obs = bool(flat_obs)
         self.num_eval_envs = num_eval_envs
+        self.track_metrics = bool(track_metrics)
+        self._metrics_capacity = metrics_capacity
         self.set_environment_params(num_envs, env_id_base, total_envs, _VARIANTS[variant])
 
     # ------------------------------------------------------------------ metadata (:218-243) ----
@@ -313,6 +323,7 @@ class TimeSeriesEnv(BaseObject):
             self._sched.data_ptr() if table is not None else None,
         )
         self._pp, self._ps, self._pst = C.byref(self._params), C.byref(self._cseries), C.byref(self._cstate)
+        self._pm = self._alloc_metrics() if self.track_metrics else None
         if self.random_reset == "last" and base + N == total:
             # :253-257 the extra (evaluation) env starts on a drawn day
             r = _lib.philox(self.seed, total - 1, 0, 1)
@@ -320,12 +331,54 @@ class TimeSeriesEnv(BaseObject):
         elif self.random_reset == "all":
             self._launch_reset_all(redraw=True)
 
+    def _alloc_metrics(self):
+        N, dev = self.num_envs, self._dev
+        cap = self._metrics_capacity
+        cap = int((N if self.evaluate else max(8 * N, 1 << 16)) if cap is None else cap)
+        if cap < 1:
+            raise ValueError("metrics_capacity must be >= 1")
+        self.metrics_capacity = cap
+        # running state (FeMetricsState): sum, mean, m2, peak, mdd, mdd_rel as f64 rows; len, pos as int32 rows
+        self._m_f64 = torch.zeros((6, N), dtype=torch.float64, device=dev)
+        self._m_i32 = torch.zeros((2, N), dtype=torch.int32, device=dev)
+        self._m_emitted = torch.zeros(N, dtype=torch.uint8, device=dev) if self.evaluate else None
+        self._m_summary = torch.zeros(_lib.METRICS_SUMMARY_BYTES // 8, dtype=torch.int64, device=dev)
+        # finished-episode list: key, env (i64); len (i32); return, sharpe, mdd, mdd_rel, hit_rate (f64)
+        self._m_fin_i64 = torch.empty((2, cap), dtype=torch.int64, device=dev)
+        self._m_fin_len = torch.empty(cap, dtype=torch.int32, device=dev)
+        self._m_fin_f64 = torch.empty((5, cap), dtype=torch.float64, device=dev)
+        f, i, L = self._m_f64, self._m_i32, self._m_fin_f64
+        self._cmetrics = _lib.FeMetricsState(
+            i[0].data_ptr(), i[1].data_ptr(), *(f[k].data_ptr() for k in range(6)),
+            self._m_emitted.data_ptr() if self._m_emitted is not None else None,
+            self._m_fin_i64[0].data_ptr(), self._m_fin_i64[1].data_ptr(), self._m_fin_len.data_ptr(),
+            *(L[k].data_ptr() for k in range(5)), self._m_summary.data_ptr())
+        return C.byref(self._cmetrics)
+
+    def _launch_metrics(self, rewards_ptr: int, dones_ptr: int, counter_ptr: Optional[int] = None) -> None:
+        """fe_episode_metrics on one step's device rewards / dones (track_metrics=True; a no-op otherwise).  The step
+        ordinal is step_count, or *counter_ptr inside a CapturedRollout."""
+        if self._pm is None:
+            return
+        _lib.check(self._L.fe_episode_metrics(self._pp, self._pm, rewards_ptr, dones_ptr, self.step_count, counter_ptr,
+                                              self.metrics_capacity, self._stream()), "fe_episode_metrics")
+
+    def _zero_metrics_running(self) -> None:
+        self._m_f64.zero_()
+        self._m_i32.zero_()
+        if self._m_emitted is not None:
+            self._m_emitted.zero_()
+
     def reset_evaluation_metrics(self) -> None:
-        """:271-275"""
-        # in place: CapturedRollout graphs and FeState hold these device addresses
+        """:271-275; with track_metrics also the episode metrics (running state, "first episode recorded" flags, list
+        and summary), so that the next evaluation records each env's first episode afresh."""
+        # in place: CapturedRollout graphs and FeState / FeMetricsState hold these device addresses
         self._terminated.zero_()
         self._ep_return.zero_()
         self._stats.zero_()
+        if self._pm is not None:
+            self._zero_metrics_running()
+            self._m_summary.zero_()
 
     # reference-named views of the state (same memory; reference shapes (N,1) / (N,))
     @property
@@ -418,6 +471,7 @@ class TimeSeriesEnv(BaseObject):
                             self.step_count, self._stream()),
             "fe_step",
         )
+        self._launch_metrics(rewards.data_ptr(), dones.data_ptr())
 
     def _new_lazy(self) -> LazyObs:
         if self.num_assets != 1:
@@ -446,6 +500,7 @@ class TimeSeriesEnv(BaseObject):
                                  self.step_count, self._stream()),
             "fe_step_lazy",
         )
+        self._launch_metrics(rewards.data_ptr(), dones.data_ptr())
         info_dict = self.record_evaluation_metrics() if self.evaluate else {}
         return (lo, rewards, dones, info_dict)
 
@@ -488,6 +543,7 @@ class TimeSeriesEnv(BaseObject):
                                      rewards.data_ptr(), dones.data_ptr(), self._stats_ptr, self.step_count, self._stream()),
                 "fe_step_lazy",
             )
+            self._launch_metrics(rewards.data_ptr(), dones.data_ptr())
         shape = ((self.num_envs, self.num_intervals * self.num_obs) if self.flat_obs
                  else (self.num_envs, self.num_intervals, self.num_obs))
         obs = torch.empty(shape, dtype=self.obs_dtype, device=self._dev)
@@ -527,6 +583,7 @@ class TimeSeriesEnv(BaseObject):
                p_bh if packed_dones else p_dh, self._stats_ptr, self.step_count, self._stream()),
             "fe_step_host_packed" if packed_dones else "fe_step_host",
         )
+        self._launch_metrics(p_r, p_d)   # the device copies of rewards and dones (int32 flags with either wire format)
         info_dict = self.record_evaluation_metrics() if self.evaluate else {}
         return (obs, rewards, out_dones, info_dict)
 
@@ -545,7 +602,8 @@ class TimeSeriesEnv(BaseObject):
     def _observe_into(self, obs: torch.Tensor) -> None:
         _lib.check(self._L.fe_observe(self._pp, self._ps, self._pst, obs.data_ptr(), self._stream()), "fe_observe")
 
-    _STATE_FIELDS = ("_seg", "_ptr", "_cash", "_long", "_short", "_margin", "_terminated", "_ep_return", "_ep_len", "_stats")
+    _STATE_FIELDS = ("_seg", "_ptr", "_cash", "_long", "_short", "_margin", "_terminated", "_ep_return", "_ep_len", "_stats",
+                     "_m_f64", "_m_i32", "_m_emitted", "_m_summary")
 
     def state_snapshot(self) -> dict:
         """Copy of the per-env state (device tensors) + the step ordinal; load_state_snapshot() restores it in place."""
@@ -569,9 +627,11 @@ class TimeSeriesEnv(BaseObject):
         """The reference's evaluation loop (PPO_LSTM_testing_SPY.py:43-52: step until info has "returns") with the
         "all envs terminated" test (:531) read once per `steps_per_replay` graph-replayed steps instead of once per
         step.  Terminated envs collect zero reward (:527-528), so running past the end changes nothing: the returned
-        {"returns": (N,) f32} equals what the per-step loop returns.  Metrics are reset afterwards (:532-534) — in
-        place, so `rollout` (a CapturedRollout of this env, e.g. the one returned in the result) can be passed back
-        in to evaluate the next checkpoint of the same policy object without capturing again."""
+        {"returns": (N,) f32} equals what the per-step loop returns.  With track_metrics the result also holds
+        "metrics": each env's first episode (the backtest report of the checkpoint), per-env tensors in env order.
+        Metrics are reset afterwards (:532-534) — in place, so `rollout` (a CapturedRollout of this env, e.g. the one
+        returned in the result) can be passed back in to evaluate the next checkpoint of the same policy object
+        without capturing again."""
         if not self.evaluate:
             raise RuntimeError("evaluate_policy needs an env constructed with evaluate=True")
         roll = rollout if rollout is not None else self.capture_rollout(policy, steps_per_replay)
@@ -583,9 +643,9 @@ class TimeSeriesEnv(BaseObject):
             steps += roll.num_steps
             if int(self._stats[1].item()) >= self.num_envs:
                 info = {"returns": self._ep_return.clone(), "steps": steps, "rollout": roll}
-                self._terminated.zero_()
-                self._ep_return.zero_()
-                self._stats.zero_()
+                if self._pm is not None:
+                    info["metrics"] = self._first_episode_metrics()
+                self.reset_evaluation_metrics()
                 return info
         return {"steps": steps, "rollout": roll}
 
@@ -595,6 +655,8 @@ class TimeSeriesEnv(BaseObject):
         n_terminated = int(self._stats[1].item())
         if n_terminated >= self.num_envs:
             info_dict = {"returns": self._ep_return.clone()}   # the reference hands out the old tensor and rebinds (:532-534)
+            if self._pm is not None:
+                info_dict["metrics"] = self._first_episode_metrics()
             self.reset_evaluation_metrics()
             return info_dict
         return {}
@@ -612,6 +674,8 @@ class TimeSeriesEnv(BaseObject):
         self._launch_reset_all(redraw)
         if self._stats is not None:
             self._stats.zero_()
+        if self._pm is not None:   # fe_reset_all also clears the terminated flags the emitted flags follow
+            self._zero_metrics_running()
         return self.reset_lazy() if lazy else self.reset()
 
     def kernel_name(self) -> str:
@@ -629,3 +693,44 @@ class TimeSeriesEnv(BaseObject):
     def clear_stats(self) -> None:
         if self._stats is not None:
             self._stats.zero_()
+
+    # ------------------------------------------------------------------ episode metrics (track_metrics) ----
+    def _require_metrics(self) -> None:
+        if self._pm is None:
+            raise RuntimeError("construct the env with track_metrics=True")
+
+    def episode_metrics(self) -> Dict[str, torch.Tensor]:
+        """Every episode finished since the last clear_metrics() (evaluate mode: since the last metric reset), sorted
+        by key = step ordinal * total_envs + global env id, i.e. in (step, env) order: {"key", "env" (global id),
+        "len", "return" (cumulative P&L), "sharpe" (per-step mean / std of the rewards, not annualised), "mdd" (max
+        drawdown of the cumulative P&L), "mdd_rel" (the same relative to peak equity starting_balance + peak),
+        "hit_rate" (share of steps with a positive reward)}.  Reads the episode count (one host sync); raises
+        RuntimeError when more episodes finished than metrics_capacity."""
+        self._require_metrics()
+        n = int(self._m_summary[0].item())
+        if n > self.metrics_capacity:
+            raise RuntimeError(f"{n} episodes finished but metrics_capacity={self.metrics_capacity}")
+        order = torch.argsort(self._m_fin_i64[0, :n])
+        f = self._m_fin_f64[:, :n][:, order]
+        return {"key": self._m_fin_i64[0, :n][order], "env": self._m_fin_i64[1, :n][order],
+                "len": self._m_fin_len[:n][order], "return": f[0], "sharpe": f[1], "mdd": f[2], "mdd_rel": f[3],
+                "hit_rate": f[4]}
+
+    def _first_episode_metrics(self) -> Dict[str, torch.Tensor]:
+        """evaluate: every env has recorded exactly its first episode; the records in env order."""
+        m = self.episode_metrics()
+        order = torch.argsort(m["env"])
+        return {k: v[order] for k, v in m.items()}
+
+    def metrics_summary(self) -> Dict[str, torch.Tensor]:
+        """Aggregates of every episode recorded since the last clear (no list needed, overflowed episodes included):
+        device scalars episodes, sum_len (int64) and sum_return, sum_sharpe, sum_sharpe_sq, sum_mdd, max_mdd,
+        sum_hit_rate (f64).  finenvs_b200.parallel.all_reduce_episode_metrics combines them over ranks."""
+        self._require_metrics()
+        s, f = self._m_summary, self._m_summary.view(torch.float64)
+        return {k: (s[j] if j < 2 else f[j]) for j, k in enumerate(_lib.METRICS_SUMMARY_KEYS)}
+
+    def clear_metrics(self) -> None:
+        """Empty the finished-episode list and zero the summary (episodes in progress keep their running state)."""
+        self._require_metrics()
+        self._m_summary.zero_()

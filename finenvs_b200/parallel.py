@@ -8,6 +8,7 @@ over envs:
 
   * episode statistics at log points  (replaces the means/stds of PPO_agent.py:143-145 and
     evo_agent.py:116-123)                    -> all_reduce(sum) of a 5-vector
+  * per-episode trading metrics (TimeSeriesEnv.metrics_summary)  -> all_reduce(sum) + all_reduce(max)
   * evaluate mode's "all envs terminated"    (time_series_env.py:531)  -> all_reduce(min)
   * ES fitness (evo_agent.py:173-191: a GLOBAL argsort -> centred ranks)  -> all_gather
 """
@@ -96,6 +97,20 @@ def all_reduce_episode_stats(vec: torch.Tensor, group=None) -> Dict[str, float]:
     var = max(sq / n - mean * mean, 0.0) if n else 0.0
     return {"episodes": n, "terminated": nt, "mean_return": mean, "std_return": var ** 0.5,
             "mean_length": sl / n if n else 0.0}
+
+
+def all_reduce_episode_metrics(summary: Dict[str, torch.Tensor], group=None) -> Dict[str, float]:
+    """TimeSeriesEnv.metrics_summary() of every rank combined: the sums add, max_mdd is the maximum.  Counts come
+    back as ints (exact below 2^53)."""
+    keys = [k for k in summary if k != "max_mdd"]
+    vec = torch.stack([summary[k].to(torch.float64) for k in keys])
+    mx = summary["max_mdd"].to(torch.float64).reshape(1).clone()
+    if dist.is_initialized() and dist.get_world_size(group) > 1:
+        dist.all_reduce(vec, op=dist.ReduceOp.SUM, group=group)
+        dist.all_reduce(mx, op=dist.ReduceOp.MAX, group=group)
+    out = {k: (int(v) if k in ("episodes", "sum_len") else v) for k, v in zip(keys, vec.tolist())}
+    out["max_mdd"] = float(mx.item())
+    return out
 
 
 def all_terminated(local_flag: torch.Tensor, group=None) -> bool:

@@ -233,6 +233,63 @@ int fe_returns_advantages(const void *rewards_dev, int32_t rewards_f64, const in
                           const float *last_values_dev, int64_t num_envs, int32_t num_steps, double gamma,
                           float *returns_dev, float *advantages_dev, void *stream);
 
+/* ---- per-episode trading metrics (extension; DESIGN.md §4.11) ---------------------------------------------
+ * An episode of env i runs from a reset to the step whose done flag is 1, that step's reward included.  r is the
+ * reward the step returned (float or double, promoted to double); all accumulation is in double, per step in this order:
+ *     len += 1;  sum += r  (cumulative P&L);
+ *     d = r - mean;  mean += d / len;  m2 += d * (r - mean)   (Welford);
+ *     pos += (r > 0);  peak = max(peak, sum)  (peak starts at 0);
+ *     mdd = max(mdd, peak - sum);  mdd_rel = max(mdd_rel, (peak - sum) / (starting_balance + peak)).
+ * At done one record is emitted and the running state is zeroed:
+ *     key = step_ordinal * total_envs + global env id (sorting by key gives (step, env) order, as fe_es_store);
+ *     sharpe = mean / sqrt(m2 / len), 0 when len < 2 or m2 == 0 — the per-step ratio, not annualised;
+ *     hit_rate = pos / len.
+ * With FeParams.evaluate an env records only its first episode after its `emitted` flag was cleared (terminated envs
+ * keep stepping with zero reward and must not record again).  Every product, quotient and sum is one IEEE-rounded f64
+ * operation (no FMA contraction), so a numpy restatement with the same operations in the same order matches bit for
+ * bit. */
+typedef struct FeMetricsSummary {
+    unsigned long long episodes; /* finished episodes recorded since the last clear; also the next list slot (> capacity:
+                                    the list overflowed, the entries past capacity were not written) */
+    unsigned long long sum_len;
+    double sum_return;
+    double sum_sharpe;
+    double sum_sharpe_sq;
+    double sum_mdd;
+    double max_mdd;              /* atomic max on the bit pattern (mdd >= 0) */
+    double sum_hit_rate;
+} FeMetricsSummary;
+
+typedef struct FeMetricsState {
+    /* running state of the current episode, (N,) each, zero-initialised */
+    int32_t *len;
+    int32_t *pos;
+    double *sum;
+    double *mean;
+    double *m2;
+    double *peak;
+    double *mdd;
+    double *mdd_rel;
+    uint8_t *emitted;            /* (N,) evaluate only: the env has recorded its first episode (may be NULL otherwise) */
+    /* finished-episode list, `capacity` entries each, filled in slot order (sort by key for (step, env) order) */
+    int64_t *fin_key;
+    int64_t *fin_env;            /* global env id */
+    int32_t *fin_len;
+    double *fin_return;          /* sum */
+    double *fin_sharpe;
+    double *fin_mdd;
+    double *fin_mdd_rel;
+    double *fin_hit_rate;
+    FeMetricsSummary *summary;   /* aggregates of every recorded episode, overflowed ones included */
+} FeMetricsState;
+
+/* Advance the metrics of p->num_envs envs by one step's rewards (float, or double when p->out_f64) and dones (int32),
+ * the device outputs of any step entry point.  The step ordinal is *step_counter_dev when that is not NULL (the counter
+ * fe_step_captured increments, so the launch can be captured in a CUDA graph right after it), else step_counter.
+ * Finished episodes take slots with one atomic per 1024-env block; slots >= capacity are counted, not written. */
+int fe_episode_metrics(const FeParams *p, const FeMetricsState *m, const void *rewards_dev, const int32_t *dones_dev,
+                       uint64_t step_counter, const uint64_t *step_counter_dev, int64_t capacity, void *stream);
+
 /* ---- ES rollout path (finenvs/agents/networks/parallel_mlp.py, finenvs/agents/ES/evo_agent.py) -------------
  * Population layout of the reference (parallel_mlp.py:121-136): envs [0, T/2) use theta + sigma*eps[p], envs
  * [T/2, T) use theta - sigma*eps[p - T/2] (T = num_envs - num_eval_envs, even), the last num_eval_envs envs use
