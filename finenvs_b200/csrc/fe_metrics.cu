@@ -7,10 +7,12 @@
 // aggregate block, with one atomic per block and field: all of them land on one 64-byte line, and one atomic per warp
 // and field (the fe_es_store_kernel scheme) serialised there (c2, 1 Mi envs: ~5 000 warps with a finished episode per
 // step).
-// The definition (op order) is in include/finenvs_b200.h; every product, quotient and sum is an explicit __d*_rn
-// intrinsic (the TU is also built with -fmad=false), so a numpy restatement reproduces the records bit for bit.
+// The definition (op order) is in include/finenvs_b200.h and its one implementation in fe_metrics.cuh (fe_backtest_kernel
+// uses it too); every product, quotient and sum is an explicit __d*_rn intrinsic (the TU is also built with -fmad=false),
+// so a numpy restatement reproduces the records bit for bit.
 #include "finenvs_b200.h"
 #include "fe_common.cuh"
+#include "fe_metrics.cuh"
 
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -40,30 +42,19 @@ fe_episode_metrics_kernel(const RewT *__restrict__ rewards, const int32_t *__res
     double sum = 0.0, sharpe = 0.0, mdd = 0.0, mdd_rel = 0.0, hit = 0.0;
     if (i < N) {
         const double r = (double)rewards[i];
-        len = m.len[i] + 1;
-        const double dlen = (double)len;
-        sum = __dadd_rn(m.sum[i], r);
-        const double d = __dsub_rn(r, m.mean[i]);
-        const double mean = __dadd_rn(m.mean[i], __ddiv_rn(d, dlen));
-        const double m2 = __dadd_rn(m.m2[i], __dmul_rn(d, __dsub_rn(r, mean)));
-        const int32_t pos = m.pos[i] + (r > 0.0 ? 1 : 0);
-        const double peak = fmax(m.peak[i], sum);
-        const double dd = __dsub_rn(peak, sum);
-        mdd = fmax(m.mdd[i], dd);
-        mdd_rel = fmax(m.mdd_rel[i], __ddiv_rn(dd, __dadd_rn(starting_balance, peak)));
+        const EpisodeRun e = episode_advance(RunInMemory{m, i}, r, starting_balance);
+        len = e.len; sum = e.sum; mdd = e.mdd; mdd_rel = e.mdd_rel;
         if (dones[i] != 0) {
             emit = 1;
             if (m.emitted) {   // evaluate: only the first episode after the flags were cleared
                 emit = !m.emitted[i];
                 m.emitted[i] = 1;
             }
-            sharpe = (len < 2 || m2 == 0.0) ? 0.0 : __ddiv_rn(mean, __dsqrt_rn(__ddiv_rn(m2, dlen)));
-            hit = __ddiv_rn((double)pos, dlen);
-            m.len[i] = 0; m.pos[i] = 0;
-            m.sum[i] = 0.0; m.mean[i] = 0.0; m.m2[i] = 0.0; m.peak[i] = 0.0; m.mdd[i] = 0.0; m.mdd_rel[i] = 0.0;
+            sharpe = episode_sharpe(e);
+            hit = episode_hit_rate(e);
+            episode_store(m, i, EpisodeRun{});
         } else {
-            m.len[i] = len; m.pos[i] = pos;
-            m.sum[i] = sum; m.mean[i] = mean; m.m2[i] = m2; m.peak[i] = peak; m.mdd[i] = mdd; m.mdd_rel[i] = mdd_rel;
+            episode_store(m, i, e);
         }
     }
     __shared__ double s_sum[6][kWarps];                 // return, sharpe, sharpe^2, mdd, hit_rate, max mdd
@@ -134,14 +125,7 @@ fe_episode_metrics_kernel(const RewT *__restrict__ rewards, const int32_t *__res
         if (slot < capacity) {
             const uint64_t step = step_counter_dev ? *step_counter_dev : step_counter;
             const int64_t gid = env_id_base + i;
-            m.fin_key[slot] = (int64_t)step * total_envs + gid;
-            m.fin_env[slot] = gid;
-            m.fin_len[slot] = len;
-            m.fin_return[slot] = sum;
-            m.fin_sharpe[slot] = sharpe;
-            m.fin_mdd[slot] = mdd;
-            m.fin_mdd_rel[slot] = mdd_rel;
-            m.fin_hit_rate[slot] = hit;
+            episode_write_record(m, slot, (int64_t)step * total_envs + gid, gid, len, sum, sharpe, mdd, mdd_rel, hit);
         }
     }
 }
@@ -151,13 +135,8 @@ fe_episode_metrics_kernel(const RewT *__restrict__ rewards, const int32_t *__res
 extern "C" int fe_episode_metrics(const FeParams *p, const FeMetricsState *m, const void *rewards_dev,
                                   const int32_t *dones_dev, uint64_t step_counter, const uint64_t *step_counter_dev,
                                   int64_t capacity, void *stream) {
-    if (!p || !m || !rewards_dev || !dones_dev || p->num_envs <= 0 || capacity < 0) return FE_EINVAL;
-    if (!m->len || !m->pos || !m->sum || !m->mean || !m->m2 || !m->peak || !m->mdd || !m->mdd_rel || !m->summary)
-        return FE_EINVAL;
-    if (!m->fin_key || !m->fin_env || !m->fin_len || !m->fin_return || !m->fin_sharpe || !m->fin_mdd || !m->fin_mdd_rel ||
-        !m->fin_hit_rate)
-        return FE_EINVAL;
-    if (p->evaluate && !m->emitted) return FE_EINVAL;
+    if (!p || !rewards_dev || !dones_dev || p->num_envs <= 0) return FE_EINVAL;
+    if (int rc = check_metrics_state(p, m, capacity)) return rc;
     DeviceGuard guard(p->device);
     if (guard.rc) return guard.rc;
     FeMetricsState ms = *m;

@@ -19,6 +19,7 @@
 // The C ABI is declared in include/finenvs_b200.h.
 #include "finenvs_b200.h"
 #include "fe_common.cuh"
+#include "fe_metrics.cuh"
 
 #include <cuda.h> // CUtensorMap (types only; cuTensorMapEncodeTiled is resolved at run time, libcuda is not linked)
 #include <cuda_runtime.h>
@@ -157,10 +158,13 @@ __device__ __forceinline__ EnvBar env_load_bar(const FeParams &p, const FeSeries
     return b;
 }
 
-template <typename OutT>
-__device__ __forceinline__ EnvResult env_compute(const FeParams &p, const FeSeries &s, const FeState &st, const Consts &k,
-                                                 int64_t i, const EnvLoads &ld, const EnvBar &bar, OutT *__restrict__ rewards,
-                                                 int32_t *__restrict__ dones, bool track, uint64_t step) {
+// The trading arithmetic of one env-step, written once.  Whatever it reads or writes besides `ld` / `bar` goes through
+// `io`: GlobalEnvIO (the state arrays and outputs, for the step kernels) or BacktestEnvIO (registers across the K steps
+// of fe_backtest_kernel).
+template <typename IO>
+__device__ __forceinline__ EnvResult env_compute_core(const FeParams &p, const FeSeries &s, const Consts &k, int64_t i,
+                                                      const EnvLoads &ld, const EnvBar &bar, bool track, uint64_t step,
+                                                      IO &io) {
     EnvResult res;
     const int W = p.window;
     // :298-302 action -> integer share delta (round half to even, then clamp)
@@ -254,29 +258,57 @@ __device__ __forceinline__ EnvResult env_compute(const FeParams &p, const FeSeri
         const int64_t gid = p.env_id_base + i;
         if (p.reset_mode == FE_RESET_ALL || (p.reset_mode == FE_RESET_LAST && gid == p.total_envs - 1)) {
             draw_segment(p, s, gid, step, 0u, seg, ptr);
-            st.seg[i] = seg;
+            io.set_seg(seg);
         }
     }
     res.done = done;
     res.newly_terminated = 0; res.fin_return = 0.0; res.fin_len = 0;
     if (p.evaluate) { // :523-536
-        const int was = st.terminated[i];
+        const int was = io.terminated();
         if (was) rew = 0.0;                                             // :527-528
-        if (done && !was) { st.terminated[i] = 1; res.newly_terminated = 1; } // :529
-        st.ep_return[i] = d2f(dadd((double)st.ep_return[i], rew));      // :530  f32 += f64
+        if (done && !was) { io.set_terminated(); res.newly_terminated = 1; } // :529
+        io.set_ep_return(d2f(dadd((double)io.ep_return(), rew)));       // :530  f32 += f64
     } else if (track) { // extension: running episode return / length for the NCCL-reduced statistics
-        const float er = d2f(dadd((double)st.ep_return[i], rew));
-        const int32_t el = st.ep_len[i] + 1;
+        const float er = d2f(dadd((double)io.ep_return(), rew));
+        const int32_t el = io.ep_len() + 1;
         if (done) { res.fin_return = (double)er; res.fin_len = el; }
-        st.ep_return[i] = done ? 0.0f : er;
-        st.ep_len[i] = done ? 0 : el;
+        io.set_ep_return(done ? 0.0f : er);
+        io.set_ep_len(done ? 0 : el);
     }
-    st.ptr[i] = ptr; st.cash[i] = cash; st.long_sh[i] = lng; st.short_sh[i] = sht; st.margin[i] = margin;
-    rewards[i] = (OutT)rew;
-    dones[i] = done; // :296 dones.int()
-    if (k.rewards_mirror) reinterpret_cast<OutT *>(k.rewards_mirror)[i] = (OutT)rew;
-    if (k.dones_mirror) k.dones_mirror[i] = done;
+    io.finish(ptr, cash, lng, sht, margin, rew, done);
     return res;
+}
+
+// the step kernels' accessor: env i's slots of the state arrays, its reward / done outputs (and their mirrors)
+template <typename OutT>
+struct GlobalEnvIO {
+    const FeState &st;
+    const Consts &k;
+    const int64_t i;
+    OutT *__restrict__ rewards;
+    int32_t *__restrict__ dones;
+    __device__ __forceinline__ void set_seg(int32_t v) { st.seg[i] = v; }
+    __device__ __forceinline__ int terminated() const { return st.terminated[i]; }
+    __device__ __forceinline__ void set_terminated() { st.terminated[i] = 1; }
+    __device__ __forceinline__ float ep_return() const { return st.ep_return[i]; }
+    __device__ __forceinline__ void set_ep_return(float v) { st.ep_return[i] = v; }
+    __device__ __forceinline__ int32_t ep_len() const { return st.ep_len[i]; }
+    __device__ __forceinline__ void set_ep_len(int32_t v) { st.ep_len[i] = v; }
+    __device__ __forceinline__ void finish(int32_t ptr, float cash, float lng, float sht, double margin, double rew, int done) {
+        st.ptr[i] = ptr; st.cash[i] = cash; st.long_sh[i] = lng; st.short_sh[i] = sht; st.margin[i] = margin;
+        rewards[i] = (OutT)rew;
+        dones[i] = done; // :296 dones.int()
+        if (k.rewards_mirror) reinterpret_cast<OutT *>(k.rewards_mirror)[i] = (OutT)rew;
+        if (k.dones_mirror) k.dones_mirror[i] = done;
+    }
+};
+
+template <typename OutT>
+__device__ __forceinline__ EnvResult env_compute(const FeParams &p, const FeSeries &s, const FeState &st, const Consts &k,
+                                                 int64_t i, const EnvLoads &ld, const EnvBar &bar, OutT *__restrict__ rewards,
+                                                 int32_t *__restrict__ dones, bool track, uint64_t step) {
+    GlobalEnvIO<OutT> io{st, k, i, rewards, dones};
+    return env_compute_core(p, s, k, i, ld, bar, track, step, io);
 }
 
 template <typename OutT>
@@ -2134,6 +2166,198 @@ int gather_obs(const FeParams &p, const FeSeries &s, const int64_t *row0, const 
 // step ordinal kept on the device (fe_step_captured): one thread bumps it ahead of the step kernel
 __global__ void fe_bump_kernel(uint64_t *counter) { *counter += 1; }
 
+// ------------------------------------------------------------------------------------------
+// signal backtest (fe_backtest): K steps of every env in one launch, one thread per env.  The action of each step is
+// read from the env's column of a signal table; the step is env_compute_core (the trading arithmetic of every step
+// kernel) and the metrics update is the one of fe_episode_metrics_kernel (fe_metrics.cuh).  The env state and the
+// metrics' running state stay in registers for the whole launch and are written back once; no observation is built.
+// ------------------------------------------------------------------------------------------
+constexpr int kBtThreads = 256;
+constexpr int kBtWarps = kBtThreads / 32;
+
+// env i's state in registers (env_compute_core's accessor for the backtest), plus the reward / done of the last step
+struct BacktestEnvIO {
+    int32_t seg, ptr;
+    float cash, lng, sht;
+    double margin;
+    int term;
+    float eret;
+    int32_t elen;
+    double rew;
+    int done;
+    __device__ __forceinline__ void set_seg(int32_t v) { seg = v; }
+    __device__ __forceinline__ int terminated() const { return term; }
+    __device__ __forceinline__ void set_terminated() { term = 1; }
+    __device__ __forceinline__ float ep_return() const { return eret; }
+    __device__ __forceinline__ void set_ep_return(float v) { eret = v; }
+    __device__ __forceinline__ int32_t ep_len() const { return elen; }
+    __device__ __forceinline__ void set_ep_len(int32_t v) { elen = v; }
+    __device__ __forceinline__ void finish(int32_t ptr_, float cash_, float lng_, float sht_, double margin_, double rew_,
+                                           int done_) {
+        ptr = ptr_; cash = cash_; lng = lng_; sht = sht_; margin = margin_; rew = rew_; done = done_;
+    }
+};
+
+// reduction over the block; the result is valid in thread 0.  Every thread of the block must call it.
+template <typename T, typename Op>
+__device__ __forceinline__ T bt_block_reduce(T v, Op op, T *sh) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v = op(v, __shfl_xor_sync(0xFFFFFFFFu, v, o));
+    __syncthreads();   // the previous call's readers are done with sh
+    if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = v;
+    __syncthreads();
+    if (threadIdx.x == 0)
+        for (int w = 1; w < kBtWarps; ++w) v = op(v, sh[w]);
+    return v;
+}
+
+template <typename OutT>
+__global__ void __launch_bounds__(kBtThreads)
+fe_backtest_kernel(const FeParams p, const FeSeries s, const FeState st, const Consts k, const FeMetricsState m,
+                   const int64_t capacity, FeStats *stats, const float *__restrict__ signal, const int32_t *__restrict__ column,
+                   const uint64_t first_step, const int K, OutT *__restrict__ rewards, int32_t *__restrict__ dones,
+                   const int history) {
+    constexpr unsigned kAll = 0xFFFFFFFFu;
+    const int64_t N = p.num_envs;
+    const int64_t i = (int64_t)blockIdx.x * kBtThreads + threadIdx.x;
+    const int64_t gid = p.env_id_base + i;
+    const bool active = i < N;
+    const bool track = stats != nullptr;
+    const int lane = threadIdx.x & 31;
+    BacktestEnvIO e{};
+    EpisodeRun run{};
+    int emitted = 0;
+    const float *sig = signal;
+    if (active) {
+        e.seg = st.seg[i]; e.ptr = st.ptr[i]; e.cash = st.cash[i]; e.lng = st.long_sh[i]; e.sht = st.short_sh[i];
+        e.margin = st.margin[i];
+        if (p.evaluate) e.term = st.terminated[i];
+        if (p.evaluate || track) e.eret = st.ep_return[i];
+        if (!p.evaluate && track) e.elen = st.ep_len[i];
+        run.len = m.len[i]; run.pos = m.pos[i];
+        run.sum = m.sum[i]; run.mean = m.mean[i]; run.m2 = m.m2[i]; run.peak = m.peak[i]; run.mdd = m.mdd[i];
+        run.mdd_rel = m.mdd_rel[i];
+        if (m.emitted) emitted = m.emitted[i];
+        sig = signal + (int64_t)column[i] * p.num_rows;
+    }
+    // FeStats and FeMetricsSummary contributions, flushed once per block after the loop; only the slot counter
+    // (summary->episodes) is touched inside it, once per warp and step with a finished episode
+    unsigned long long st_done = 0, st_term = 0, st_len = 0;
+    double st_ret = 0.0, st_sq = 0.0;
+    unsigned long long ms_cnt = 0, ms_len = 0;
+    double ms_ret = 0.0, ms_sh = 0.0, ms_sh2 = 0.0, ms_mdd = 0.0, ms_hit = 0.0, ms_max = 0.0;
+    for (int t = 0; t < K; ++t) {
+        const uint64_t step = first_step + (uint64_t)t;
+        int emit = 0;
+        int32_t len = 0;
+        double sum = 0.0, sharpe = 0.0, mdd = 0.0, mdd_rel = 0.0, hit = 0.0;
+        if (active) {
+            EnvLoads ld;
+            ld.seg = e.seg; ld.ptr = e.ptr; ld.cash = e.cash; ld.lng = e.lng; ld.sht = e.sht; ld.margin = e.margin;
+            const EnvBar bar = env_load_bar(p, s, ld);
+            // row seg_start + ptr + W - 1: the last row of the window the env observed before this step (bar.row0 is the
+            // window after the advance).  The trade executes at the next row's Open: no look-ahead.
+            ld.act = __ldg(sig + bar.row0 + p.window - 2);
+            const EnvResult r = env_compute_core(p, s, k, i, ld, bar, track, step, e);
+            const OutT ro = (OutT)e.rew;
+            if (history) {
+                rewards[(int64_t)t * N + i] = ro;
+                dones[(int64_t)t * N + i] = e.done;
+            } else if (t == K - 1) {
+                rewards[i] = ro;
+                dones[i] = e.done;
+            }
+            if (track && r.done) {   // accumulate_stats
+                st_done += 1;
+                st_len += (unsigned long long)r.fin_len;
+                st_ret += r.fin_return;
+                st_sq += r.fin_return * r.fin_return;
+            }
+            st_term += (unsigned long long)r.newly_terminated;
+            const EpisodeRun nx = episode_advance(RunInRegisters{run}, (double)ro, p.starting_balance);
+            len = nx.len; sum = nx.sum; mdd = nx.mdd; mdd_rel = nx.mdd_rel;
+            if (e.done) {
+                emit = 1;
+                if (m.emitted) {   // evaluate: only the first episode after the flags were cleared
+                    emit = !emitted;
+                    emitted = 1;
+                }
+                sharpe = episode_sharpe(nx);
+                hit = episode_hit_rate(nx);
+                run = EpisodeRun{};
+            } else {
+                run = nx;
+            }
+        }
+        const unsigned ballot = __ballot_sync(kAll, emit);
+        if (ballot) {
+            const int leader = __ffs(ballot) - 1;
+            unsigned long long base = 0;
+            if (lane == leader) base = atomicAdd(&m.summary->episodes, (unsigned long long)__popc(ballot));
+            base = __shfl_sync(kAll, base, leader);
+            if (emit) {
+                const int64_t slot = (int64_t)base + __popc(ballot & ((1u << lane) - 1u));
+                if (slot < capacity)
+                    episode_write_record(m, slot, (int64_t)step * p.total_envs + gid, gid, len, sum, sharpe, mdd, mdd_rel, hit);
+                ms_cnt += 1;
+                ms_len += (unsigned long long)len;
+                ms_ret = __dadd_rn(ms_ret, sum);
+                ms_sh = __dadd_rn(ms_sh, sharpe);
+                ms_sh2 = __dadd_rn(ms_sh2, __dmul_rn(sharpe, sharpe));
+                ms_mdd = __dadd_rn(ms_mdd, mdd);
+                ms_hit = __dadd_rn(ms_hit, hit);
+                ms_max = fmax(ms_max, mdd);
+            }
+        }
+    }
+    if (active) {
+        st.seg[i] = e.seg; st.ptr[i] = e.ptr; st.cash[i] = e.cash; st.long_sh[i] = e.lng; st.short_sh[i] = e.sht;
+        st.margin[i] = e.margin;
+        if (p.evaluate) st.terminated[i] = (uint8_t)e.term;
+        if (p.evaluate || track) st.ep_return[i] = e.eret;
+        if (!p.evaluate && track) st.ep_len[i] = e.elen;
+        episode_store(m, i, run);
+        if (m.emitted) m.emitted[i] = (uint8_t)emitted;
+    }
+    __shared__ unsigned long long sh_u[kBtWarps];
+    __shared__ double sh_d[kBtWarps];
+    const auto add_u = [](unsigned long long a, unsigned long long b) { return a + b; };
+    const auto add_d = [](double a, double b) { return __dadd_rn(a, b); };
+    const auto max_d = [](double a, double b) { return fmax(a, b); };
+    if (track) {
+        const unsigned long long nd = bt_block_reduce(st_done, add_u, sh_u);
+        const unsigned long long nt = bt_block_reduce(st_term, add_u, sh_u);
+        const unsigned long long sl = bt_block_reduce(st_len, add_u, sh_u);
+        const double sr = bt_block_reduce(st_ret, add_d, sh_d);
+        const double sq = bt_block_reduce(st_sq, add_d, sh_d);
+        if (threadIdx.x == 0) {
+            if (nd) atomicAdd(&stats->n_done, nd);
+            if (nt) atomicAdd(&stats->n_terminated, nt);
+            if (sl) atomicAdd(&stats->sum_len, sl);
+            if (nd) { atomicAdd(&stats->sum_return, sr); atomicAdd(&stats->sum_return_sq, sq); }
+        }
+    }
+    const unsigned long long cnt = bt_block_reduce(ms_cnt, add_u, sh_u);
+    const unsigned long long blen = bt_block_reduce(ms_len, add_u, sh_u);
+    const double bret = bt_block_reduce(ms_ret, add_d, sh_d);
+    const double bsh = bt_block_reduce(ms_sh, add_d, sh_d);
+    const double bsh2 = bt_block_reduce(ms_sh2, add_d, sh_d);
+    const double bmdd = bt_block_reduce(ms_mdd, add_d, sh_d);
+    const double bhit = bt_block_reduce(ms_hit, add_d, sh_d);
+    const double bmax = bt_block_reduce(ms_max, max_d, sh_d);
+    if (threadIdx.x == 0 && cnt) {
+        FeMetricsSummary *sm = m.summary;
+        atomicAdd(&sm->sum_len, blen);
+        atomicAdd(&sm->sum_return, bret);
+        atomicAdd(&sm->sum_sharpe, bsh);
+        atomicAdd(&sm->sum_sharpe_sq, bsh2);
+        atomicAdd(&sm->sum_mdd, bmdd);
+        atomicAdd(&sm->sum_hit_rate, bhit);
+        // mdd >= 0: the order of non-negative doubles is the order of their bit patterns
+        atomicMax(reinterpret_cast<unsigned long long *>(&sm->max_mdd), (unsigned long long)__double_as_longlong(bmax));
+    }
+}
+
 // side streams of fe_step_host (created once per device, never destroyed: they live as long as the process)
 constexpr int kHostStreams = 3;
 struct HostPipe {
@@ -2334,6 +2558,33 @@ int fe_step_lazy(const FeParams *p, const FeSeries *s, const FeState *st, const 
         fe_lazy_kernel<float, false><<<blocks, kThreads, 0, (cudaStream_t)stream>>>(
             *p, *s, *st, k, actions_dev, obs_row0_dev, (float *)obs_posfeat_dev, (float *)rewards_dev, dones_dev, stats_dev,
             step_counter, nullptr);
+    return (int)cudaGetLastError();
+}
+
+int fe_backtest(const FeParams *p, const FeSeries *s, const FeState *st, const FeMetricsState *m, int64_t metrics_capacity,
+                FeStats *stats_dev, const float *signal_dev, int32_t num_signals, const int32_t *column_dev,
+                uint64_t first_step, int32_t num_steps, void *rewards_dev, int32_t *dones_dev, int32_t history, void *stream) {
+    int rc = check_common(p, s, st);
+    if (rc) return rc;
+    if (p->num_assets != 1 || !signal_dev || num_signals < 1 || !column_dev || num_steps < 1 || !rewards_dev || !dones_dev)
+        return FE_EINVAL;
+    if (stats_dev && !p->evaluate && (!st->ep_return || !st->ep_len)) return FE_EINVAL;
+    if ((rc = check_metrics_state(p, m, metrics_capacity))) return rc;
+    DeviceGuard guard(p->device);
+    if (guard.rc) return guard.rc;
+    const Consts k = make_consts(*p);
+    FeMetricsState ms = *m;
+    if (!p->evaluate) ms.emitted = nullptr;
+    const unsigned blocks = (unsigned)((p->num_envs + kBtThreads - 1) / kBtThreads);
+    cudaStream_t q = (cudaStream_t)stream;
+    if (p->out_f64)
+        fe_backtest_kernel<double><<<blocks, kBtThreads, 0, q>>>(*p, *s, *st, k, ms, metrics_capacity, stats_dev, signal_dev,
+                                                                 column_dev, first_step, num_steps, (double *)rewards_dev,
+                                                                 dones_dev, history);
+    else
+        fe_backtest_kernel<float><<<blocks, kBtThreads, 0, q>>>(*p, *s, *st, k, ms, metrics_capacity, stats_dev, signal_dev,
+                                                                column_dev, first_step, num_steps, (float *)rewards_dev,
+                                                                dones_dev, history);
     return (int)cudaGetLastError();
 }
 

@@ -39,6 +39,19 @@ _VARIANTS = {"auto": _lib.VARIANT_AUTO, "tile": _lib.VARIANT_TILE, "direct": _li
              "gather": _lib.VARIANT_GATHER}
 
 
+def default_signal_columns(env_id_base: int, num_envs: int, num_segments: int, num_signals: int) -> torch.Tensor:
+    """The signal column each env of the shard [env_id_base, env_id_base + num_envs) trades in TimeSeriesEnv.backtest()
+    by default: global id // num_segments.  Env g starts on segment g % num_segments, so with total_envs = S x D every
+    (strategy, day) pair is one env, whatever the sharding.  (num_envs,) int32 on the CPU; ValueError when a column
+    falls outside [0, num_signals)."""
+    gid = torch.arange(int(env_id_base), int(env_id_base) + int(num_envs), dtype=torch.int64)
+    cols = gid // int(num_segments)
+    if num_envs > 0 and int(cols[-1]) >= num_signals:
+        raise ValueError(f"the default columns (global id // {num_segments} segments) reach {int(cols[-1])}, but the "
+                         f"signal table has {num_signals} rows; pass columns= or more signals")
+    return cols.to(torch.int32)
+
+
 class LazyObs:
     """An observation that has not been materialised: obs[i, j, 0:4] = logret[row0[i] + j], obs[i, j, 4] = posfeat[i]
     (time_series_env.py:428-445).  12 bytes per env instead of W x 20; consumers that read the window straight from
@@ -734,3 +747,84 @@ class TimeSeriesEnv(BaseObject):
         """Empty the finished-episode list and zero the summary (episodes in progress keep their running state)."""
         self._require_metrics()
         self._m_summary.zero_()
+
+    # ------------------------------------------------------------------ signal backtests (DESIGN §4.12) ----
+    def backtest(self, signal: torch.Tensor, num_steps: int, columns: Optional[torch.Tensor] = None,
+                 history: bool = False) -> Dict:
+        """Advance every env `num_steps` steps with actions read from a signal table, in ONE launch (fe_backtest).
+
+        `signal` is a float32 (S, series.num_rows) tensor on the env's device: one row ("column") per rule-based
+        strategy, one action per row of the staged series, mapped like step()'s actions.  Env i trades column
+        `columns[i]` (default: default_signal_columns, global id // num_segments).  At every step env i's action is
+        signal[columns[i], seg_start[seg] + ptr + W - 1] with the state before the step: the last row of the window the
+        env observes.  The trade executes at the next bar's Open, so there is no look-ahead by construction.
+
+        The result is bit-identical to `num_steps` step_into() calls with those actions: per-env state, redraws, stats,
+        episode metrics (records, running state, summary counts; the f64 sums up to their order of addition).  Unlike
+        step() in evaluate mode it does not test for "all terminated" or reset the evaluation metrics on the way
+        (evaluate_signal() does that once, at the end).  Needs track_metrics=True and a single-asset series.  Records are
+        keyed by global env id, so shards of one population (env_id_base / total_envs) produce the records of the whole
+        and parallel.all_reduce_episode_metrics combines their summaries.
+
+        Returns {"steps": num_steps}, plus "rewards" / "dones" (num_steps, N) when history=True."""
+        self._require_metrics()
+        if self.num_assets != 1:
+            raise NotImplementedError("signal backtests are implemented for single-asset envs")
+        if self._obs_ring is not None or self._handle_ring is not None:
+            raise RuntimeError("a rollout buffer is bound to this env (bind_env): a backtest would leave the observation "
+                               "it holds stale")
+        K = int(num_steps)
+        if K < 1:
+            raise ValueError("num_steps must be >= 1")
+        if not torch.is_tensor(signal) or signal.dim() != 2 or signal.shape[1] != self.series.num_rows:
+            raise ValueError(f"signal must be a (S, {self.series.num_rows}) tensor (one row per strategy, one value per "
+                             f"series row); got {tuple(signal.shape) if torch.is_tensor(signal) else type(signal)}")
+        if signal.dtype != torch.float32 or signal.device != self._dev or not signal.is_contiguous():
+            raise ValueError(f"signal must be a contiguous float32 tensor on {self._dev}; got {signal.dtype} on "
+                             f"{signal.device}{'' if signal.is_contiguous() else ', not contiguous'}")
+        S = signal.shape[0]
+        if S < 1 or S > 0x7FFFFFFF:
+            raise ValueError("signal must have between 1 and 2**31 - 1 rows")
+        if columns is None:
+            cols = default_signal_columns(self.env_id_base, self.num_envs, self.series.num_segments, S).to(self._dev)
+        else:
+            if (not torch.is_tensor(columns) or columns.shape != (self.num_envs,) or columns.dtype.is_floating_point
+                    or columns.dtype.is_complex or columns.dtype == torch.bool):
+                raise ValueError(f"columns must be an integer ({self.num_envs},) tensor")
+            lo, hi = torch.stack(torch.aminmax(columns)).tolist()   # one host read
+            if lo < 0 or hi >= S:
+                raise ValueError(f"columns must lie in [0, {S}); got [{lo}, {hi}]")
+            cols = columns.to(device=self._dev, dtype=torch.int32).contiguous()
+        shape = (K, self.num_envs) if history else (self.num_envs,)
+        rewards = torch.empty(shape, dtype=self.obs_dtype, device=self._dev)
+        dones = torch.empty(shape, dtype=torch.int32, device=self._dev)
+        _lib.check(
+            self._L.fe_backtest(self._pp, self._ps, self._pst, self._pm, self.metrics_capacity, self._stats_ptr,
+                                signal.data_ptr(), S, cols.data_ptr(), self.step_count + 1, K, rewards.data_ptr(),
+                                dones.data_ptr(), int(bool(history)), self._stream()),
+            "fe_backtest",
+        )
+        self.step_count += K
+        self._epoch += 1   # a CapturedRollout's observation is stale now
+        out = {"steps": K}
+        if history:
+            out["rewards"], out["dones"] = rewards, dones
+        return out
+
+    def evaluate_signal(self, signal: torch.Tensor, columns: Optional[torch.Tensor] = None) -> Dict:
+        """The evaluate-mode report of a signal table, the counterpart of evaluate_policy(): one backtest() launch of
+        max(seg_len) - W steps (enough for every env to finish its current episode from any pointer; terminated envs
+        collect zero reward, so running past the end changes nothing), then one host read of the terminated count.
+        Returns {"returns": (N,) f32, "steps", "metrics": each env's first episode in env order} and resets the
+        evaluation metrics, as evaluate_policy() does.  Needs evaluate=True and track_metrics=True."""
+        if not self.evaluate:
+            raise RuntimeError("evaluate_signal needs an env constructed with evaluate=True")
+        self._require_metrics()
+        if getattr(self, "_signal_steps", None) is None:
+            self._signal_steps = int(self.series.seg_len.max().item()) - self.num_intervals
+        steps = self.backtest(signal, self._signal_steps, columns)["steps"]
+        if int(self._stats[1].item()) >= self.num_envs:
+            info = {"returns": self._ep_return.clone(), "steps": steps, "metrics": self._first_episode_metrics()}
+            self.reset_evaluation_metrics()
+            return info
+        return {"steps": steps}

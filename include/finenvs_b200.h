@@ -290,6 +290,25 @@ typedef struct FeMetricsState {
 int fe_episode_metrics(const FeParams *p, const FeMetricsState *m, const void *rewards_dev, const int32_t *dones_dev,
                        uint64_t step_counter, const uint64_t *step_counter_dev, int64_t capacity, void *stream);
 
+/* ---- signal backtests (extension; DESIGN.md §4.12) ----------------------------------------------------------
+ * A signal table signal_dev (num_signals, p->num_rows) float holds one row ("column") per rule-based strategy and one
+ * value per row of the staged flat series; values are actions, mapped exactly like fe_step's (rint(a * (max_shares +
+ * 0.5)), clamped).  Env i trades column column_dev[i] in [0, num_signals) (the caller's responsibility, like
+ * fe_gather_obs' index).  fe_backtest advances every env num_steps steps in ONE launch and is bit-identical to
+ * num_steps calls of fe_step + fe_episode_metrics with step ordinals first_step, first_step + 1, ... in which env i's
+ * action at each step is
+ *     a_i = signal[column[i], seg_start[seg_i] + ptr_i + W - 1]        (seg_i, ptr_i: the state BEFORE the step)
+ * i.e. the last row of the window the env observes; the trade executes at the next row's Open, so a signal computed from
+ * rows <= r never trades on row r's prices: no look-ahead by construction.  Identical are the per-env state, the Philox
+ * redraws, the FeStats counts, the metrics' running state, the records of the finished-episode list (same keys and values;
+ * which records win a slot on overflow depends on warp timing, as with fe_episode_metrics) and the summary counts and
+ * max_mdd; f64 sums are the same values added in another order.  rewards_dev / dones_dev: (num_steps, N) histories when
+ * history != 0, else (N,) holding the last step.  No observation is written.  Single-asset series only (num_assets == 1);
+ * evaluate mode needs m->emitted, FeStats (stats_dev, may be NULL) as fe_step. */
+int fe_backtest(const FeParams *p, const FeSeries *s, const FeState *st, const FeMetricsState *m, int64_t metrics_capacity,
+                FeStats *stats_dev, const float *signal_dev, int32_t num_signals, const int32_t *column_dev,
+                uint64_t first_step, int32_t num_steps, void *rewards_dev, int32_t *dones_dev, int32_t history, void *stream);
+
 /* ---- ES rollout path (finenvs/agents/networks/parallel_mlp.py, finenvs/agents/ES/evo_agent.py) -------------
  * Population layout of the reference (parallel_mlp.py:121-136): envs [0, T/2) use theta + sigma*eps[p], envs
  * [T/2, T) use theta - sigma*eps[p - T/2] (T = num_envs - num_eval_envs, even), the last num_eval_envs envs use
