@@ -77,6 +77,9 @@ METRICS_SUMMARY_KEYS = ("episodes", "sum_len", "sum_return", "sum_sharpe", "sum_
                         "sum_hit_rate")
 METRICS_SUMMARY_BYTES = 64
 
+# FE_TARGET_MAX_SHARES: the largest max_shares of a target-position backtest (the D -> action -> D round trip is exact)
+TARGET_MAX_SHARES = 1 << 20
+
 
 class FeMetricsState(C.Structure):
     _fields_ = [(name, C.c_void_p) for name in (
@@ -122,6 +125,9 @@ _PROTOTYPES = {
     "fe_backtest": (C.c_int, [C.POINTER(FeParams), C.POINTER(FeSeries), C.POINTER(FeState), C.POINTER(FeMetricsState),
                               C.c_int64, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_uint64, C.c_int32, C.c_void_p,
                               C.c_void_p, C.c_int32, C.c_void_p]),
+    "fe_backtest_targets": (C.c_int, [C.POINTER(FeParams), C.POINTER(FeSeries), C.POINTER(FeState),
+                                      C.POINTER(FeMetricsState), C.c_int64, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p,
+                                      C.c_void_p, C.c_uint64, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
     "fe_es_params_padded": (C.c_int64, [C.POINTER(FeEsNet)]),
     "fe_es_packed_index": (C.c_int64, [C.POINTER(FeEsNet), C.c_int32, C.c_int32, C.c_int32]),
     "fe_es_perturb": (C.c_int, [C.POINTER(FeEsNet), C.c_uint64, C.c_uint64, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p]),

@@ -2167,8 +2167,9 @@ int gather_obs(const FeParams &p, const FeSeries &s, const int64_t *row0, const 
 __global__ void fe_bump_kernel(uint64_t *counter) { *counter += 1; }
 
 // ------------------------------------------------------------------------------------------
-// signal backtest (fe_backtest): K steps of every env in one launch, one thread per env.  The action of each step is
-// read from the env's column of a signal table; the step is env_compute_core (the trading arithmetic of every step
+// signal backtest (fe_backtest, fe_backtest_targets): K steps of every env in one launch, one thread per env.  The
+// action of each step comes from the env's column of a signal table: the value itself (TradeRule) or the delta to a
+// target position (TargetRule); the step is env_compute_core (the trading arithmetic of every step
 // kernel) and the metrics update is the one of fe_episode_metrics_kernel (fe_metrics.cuh).  The env state and the
 // metrics' running state stay in registers for the whole launch and are written back once; no observation is built.
 // ------------------------------------------------------------------------------------------
@@ -2211,12 +2212,36 @@ __device__ __forceinline__ T bt_block_reduce(T v, Op op, T *sh) {
     return v;
 }
 
-template <typename OutT>
-__global__ void __launch_bounds__(kBtThreads)
-fe_backtest_kernel(const FeParams p, const FeSeries s, const FeState st, const Consts k, const FeMetricsState m,
-                   const int64_t capacity, FeStats *stats, const float *__restrict__ signal, const int32_t *__restrict__ column,
-                   const uint64_t first_step, const int K, OutT *__restrict__ rewards, int32_t *__restrict__ dones,
-                   const int history) {
+// The action rules of a backtest step: the table value v of env i's column at the step's row -> the action fed to
+// env_compute_core.  load(c) runs once per launch with env i's column c.
+struct TradeRule {   // fe_backtest: v is the action
+    __device__ __forceinline__ void load(int32_t) {}
+    __device__ __forceinline__ float action(float v, const BacktestEnvIO &, const EpisodeRun &) const { return v; }
+};
+struct TargetRule {  // fe_backtest_targets: v is a target net position (include/finenvs_b200.h)
+    const double *__restrict__ exits;   // (num_signals, 2) trailing stop, take-profit; nullptr: no exits
+    float ms, scale;
+    double stop, take;
+    __device__ __forceinline__ void load(int32_t c) {
+        if (exits) { stop = __ldg(exits + 2 * (int64_t)c); take = __ldg(exits + 2 * (int64_t)c + 1); }
+    }
+    __device__ __forceinline__ float action(float v, const BacktestEnvIO &e, const EpisodeRun &run) const {
+        float T = rintf(fmul(v, scale));
+        T = T < -ms ? -ms : (T > ms ? ms : T);
+        if (exits && (dsub(run.peak, run.sum) >= stop || run.sum >= take)) T = 0.0f;
+        // env_compute_core maps the quotient back to exactly D (the header's round-trip bound, max_shares <= 2^20)
+        return __fdiv_rn(fsub(T, fsub(e.lng, e.sht)), scale);
+    }
+};
+
+// the backtest loop of both entry points; Rule turns each step's table value into the action.  The structs are taken
+// by value: with references the compiler numbered fe_backtest_kernel's accumulators differently and its SASS changed.
+template <typename OutT, typename Rule>
+__device__ __forceinline__ void
+backtest_run(const FeParams p, const FeSeries s, const FeState st, const Consts k, const FeMetricsState m,
+             const int64_t capacity, FeStats *stats, const float *__restrict__ signal, const int32_t *__restrict__ column,
+             const uint64_t first_step, const int K, OutT *__restrict__ rewards, int32_t *__restrict__ dones,
+             const int history, Rule rule) {
     constexpr unsigned kAll = 0xFFFFFFFFu;
     const int64_t N = p.num_envs;
     const int64_t i = (int64_t)blockIdx.x * kBtThreads + threadIdx.x;
@@ -2238,7 +2263,9 @@ fe_backtest_kernel(const FeParams p, const FeSeries s, const FeState st, const C
         run.sum = m.sum[i]; run.mean = m.mean[i]; run.m2 = m.m2[i]; run.peak = m.peak[i]; run.mdd = m.mdd[i];
         run.mdd_rel = m.mdd_rel[i];
         if (m.emitted) emitted = m.emitted[i];
-        sig = signal + (int64_t)column[i] * p.num_rows;
+        const int32_t c = column[i];
+        sig = signal + (int64_t)c * p.num_rows;
+        rule.load(c);
     }
     // FeStats and FeMetricsSummary contributions, flushed once per block after the loop; only the slot counter
     // (summary->episodes) is touched inside it, once per warp and step with a finished episode
@@ -2257,7 +2284,7 @@ fe_backtest_kernel(const FeParams p, const FeSeries s, const FeState st, const C
             const EnvBar bar = env_load_bar(p, s, ld);
             // row seg_start + ptr + W - 1: the last row of the window the env observed before this step (bar.row0 is the
             // window after the advance).  The trade executes at the next row's Open: no look-ahead.
-            ld.act = __ldg(sig + bar.row0 + p.window - 2);
+            ld.act = rule.action(__ldg(sig + bar.row0 + p.window - 2), e, run);
             const EnvResult r = env_compute_core(p, s, k, i, ld, bar, track, step, e);
             const OutT ro = (OutT)e.rew;
             if (history) {
@@ -2356,6 +2383,25 @@ fe_backtest_kernel(const FeParams p, const FeSeries s, const FeState st, const C
         // mdd >= 0: the order of non-negative doubles is the order of their bit patterns
         atomicMax(reinterpret_cast<unsigned long long *>(&sm->max_mdd), (unsigned long long)__double_as_longlong(bmax));
     }
+}
+
+template <typename OutT>
+__global__ void __launch_bounds__(kBtThreads)
+fe_backtest_kernel(const FeParams p, const FeSeries s, const FeState st, const Consts k, const FeMetricsState m,
+                   const int64_t capacity, FeStats *stats, const float *__restrict__ signal, const int32_t *__restrict__ column,
+                   const uint64_t first_step, const int K, OutT *__restrict__ rewards, int32_t *__restrict__ dones,
+                   const int history) {
+    backtest_run<OutT>(p, s, st, k, m, capacity, stats, signal, column, first_step, K, rewards, dones, history, TradeRule{});
+}
+
+template <typename OutT>
+__global__ void __launch_bounds__(kBtThreads)
+fe_backtest_targets_kernel(const FeParams p, const FeSeries s, const FeState st, const Consts k, const FeMetricsState m,
+                           const int64_t capacity, FeStats *stats, const float *__restrict__ signal,
+                           const int32_t *__restrict__ column, const double *__restrict__ exits, const uint64_t first_step,
+                           const int K, OutT *__restrict__ rewards, int32_t *__restrict__ dones, const int history) {
+    const TargetRule rule{exits, k.ms, k.scale, 0.0, 0.0};
+    backtest_run<OutT>(p, s, st, k, m, capacity, stats, signal, column, first_step, K, rewards, dones, history, rule);
 }
 
 // side streams of fe_step_host (created once per device, never destroyed: they live as long as the process)
@@ -2585,6 +2631,36 @@ int fe_backtest(const FeParams *p, const FeSeries *s, const FeState *st, const F
         fe_backtest_kernel<float><<<blocks, kBtThreads, 0, q>>>(*p, *s, *st, k, ms, metrics_capacity, stats_dev, signal_dev,
                                                                 column_dev, first_step, num_steps, (float *)rewards_dev,
                                                                 dones_dev, history);
+    return (int)cudaGetLastError();
+}
+
+int fe_backtest_targets(const FeParams *p, const FeSeries *s, const FeState *st, const FeMetricsState *m,
+                        int64_t metrics_capacity, FeStats *stats_dev, const float *signal_dev, int32_t num_signals,
+                        const int32_t *column_dev, const double *exits_dev, uint64_t first_step, int32_t num_steps,
+                        void *rewards_dev, int32_t *dones_dev, int32_t history, void *stream) {
+    int rc = check_common(p, s, st);
+    if (rc) return rc;
+    if (p->num_assets != 1 || !signal_dev || num_signals < 1 || !column_dev || num_steps < 1 || !rewards_dev || !dones_dev)
+        return FE_EINVAL;
+    if (p->max_shares < 1 || p->max_shares > FE_TARGET_MAX_SHARES) return FE_EINVAL;
+    if ((uintptr_t)exits_dev & 7) return FE_EALIGN;
+    if (stats_dev && !p->evaluate && (!st->ep_return || !st->ep_len)) return FE_EINVAL;
+    if ((rc = check_metrics_state(p, m, metrics_capacity))) return rc;
+    DeviceGuard guard(p->device);
+    if (guard.rc) return guard.rc;
+    const Consts k = make_consts(*p);
+    FeMetricsState ms = *m;
+    if (!p->evaluate) ms.emitted = nullptr;
+    const unsigned blocks = (unsigned)((p->num_envs + kBtThreads - 1) / kBtThreads);
+    cudaStream_t q = (cudaStream_t)stream;
+    if (p->out_f64)
+        fe_backtest_targets_kernel<double><<<blocks, kBtThreads, 0, q>>>(*p, *s, *st, k, ms, metrics_capacity, stats_dev,
+                                                                         signal_dev, column_dev, exits_dev, first_step,
+                                                                         num_steps, (double *)rewards_dev, dones_dev, history);
+    else
+        fe_backtest_targets_kernel<float><<<blocks, kBtThreads, 0, q>>>(*p, *s, *st, k, ms, metrics_capacity, stats_dev,
+                                                                        signal_dev, column_dev, exits_dev, first_step,
+                                                                        num_steps, (float *)rewards_dev, dones_dev, history);
     return (int)cudaGetLastError();
 }
 

@@ -750,7 +750,7 @@ class TimeSeriesEnv(BaseObject):
 
     # ------------------------------------------------------------------ signal backtests (DESIGN §4.12) ----
     def backtest(self, signal: torch.Tensor, num_steps: int, columns: Optional[torch.Tensor] = None,
-                 history: bool = False) -> Dict:
+                 history: bool = False, *, targets: bool = False, exits: Optional[torch.Tensor] = None) -> Dict:
         """Advance every env `num_steps` steps with actions read from a signal table, in ONE launch (fe_backtest).
 
         `signal` is a float32 (S, series.num_rows) tensor on the env's device: one row ("column") per rule-based
@@ -759,12 +759,24 @@ class TimeSeriesEnv(BaseObject):
         signal[columns[i], seg_start[seg] + ptr + W - 1] with the state before the step: the last row of the window the
         env observes.  The trade executes at the next bar's Open, so there is no look-ahead by construction.
 
-        The result is bit-identical to `num_steps` step_into() calls with those actions: per-env state, redraws, stats,
-        episode metrics (records, running state, summary counts; the f64 sums up to their order of addition).  Unlike
-        step() in evaluate mode it does not test for "all terminated" or reset the evaluation metrics on the way
-        (evaluate_signal() does that once, at the end).  Needs track_metrics=True and a single-asset series.  Records are
-        keyed by global env id, so shards of one population (env_id_base / total_envs) produce the records of the whole
-        and parallel.all_reduce_episode_metrics combines their summaries.
+        With targets=True (fe_backtest_targets) that value v is the net position to hold instead of a trade:
+        T = clamp(rint(v * (max_shares + 0.5)), +-max_shares) shares, and the action is the delta (T - (long - short)) /
+        (max_shares + 0.5), which step() maps back to exactly that delta (clamped to +-max_shares).  So +1 everywhere is
+        buy-and-hold wherever the episode starts, and sign(momentum) is "long while momentum is positive".  `exits`, a
+        contiguous float64 (S, 2) tensor on the env's device, adds per column a trailing stop [:, 0] and a take-profit
+        [:, 1] in reward units: T is 0 on every step at which the episode's P&L is that far below its running peak
+        (peak starts at 0), or at least the take-profit.  Thresholds must be > 0; +inf disables one.  The exit is not
+        latched, but once flat the rewards are 0, so the env stays flat until its episode ends.  The env's rules still
+        apply: a flip from long to short takes two steps, and an entry the cash cannot pay for is retried.  Needs
+        max_shares <= 2**20.
+
+        The result is bit-identical to `num_steps` step_into() calls with those actions (for targets, computed from the
+        env's state before each step in the same f32 / f64 operations): per-env state, redraws, stats, episode metrics
+        (records, running state, summary counts; the f64 sums up to their order of addition).  Unlike step() in evaluate
+        mode it does not test for "all terminated" or reset the evaluation metrics on the way (evaluate_signal() does
+        that once, at the end).  Needs track_metrics=True and a single-asset series.  Records are keyed by global env id,
+        so shards of one population (env_id_base / total_envs) produce the records of the whole and
+        parallel.all_reduce_episode_metrics combines their summaries.
 
         Returns {"steps": num_steps}, plus "rewards" / "dones" (num_steps, N) when history=True."""
         self._require_metrics()
@@ -795,15 +807,37 @@ class TimeSeriesEnv(BaseObject):
             if lo < 0 or hi >= S:
                 raise ValueError(f"columns must lie in [0, {S}); got [{lo}, {hi}]")
             cols = columns.to(device=self._dev, dtype=torch.int32).contiguous()
+        if exits is not None:
+            if not targets:
+                raise ValueError("exits need targets=True (they flatten a target position)")
+            if not torch.is_tensor(exits) or exits.shape != (S, 2):
+                raise ValueError(f"exits must be a ({S}, 2) tensor (trailing stop, take-profit per signal row); got "
+                                 f"{tuple(exits.shape) if torch.is_tensor(exits) else type(exits)}")
+            if exits.dtype != torch.float64 or exits.device != self._dev or not exits.is_contiguous():
+                raise ValueError(f"exits must be a contiguous float64 tensor on {self._dev}; got {exits.dtype} on "
+                                 f"{exits.device}{'' if exits.is_contiguous() else ', not contiguous'}")
+            if not bool((exits > 0).all()):   # one host read; NaN fails the comparison too
+                raise ValueError("exit thresholds must be > 0 (+inf disables one); got a value <= 0 or NaN")
+        if targets and not 1 <= self.max_shares <= _lib.TARGET_MAX_SHARES:
+            raise ValueError(f"target backtests need 1 <= max_shares <= {_lib.TARGET_MAX_SHARES}")
         shape = (K, self.num_envs) if history else (self.num_envs,)
         rewards = torch.empty(shape, dtype=self.obs_dtype, device=self._dev)
         dones = torch.empty(shape, dtype=torch.int32, device=self._dev)
-        _lib.check(
-            self._L.fe_backtest(self._pp, self._ps, self._pst, self._pm, self.metrics_capacity, self._stats_ptr,
-                                signal.data_ptr(), S, cols.data_ptr(), self.step_count + 1, K, rewards.data_ptr(),
-                                dones.data_ptr(), int(bool(history)), self._stream()),
-            "fe_backtest",
-        )
+        if targets:
+            _lib.check(
+                self._L.fe_backtest_targets(self._pp, self._ps, self._pst, self._pm, self.metrics_capacity,
+                                            self._stats_ptr, signal.data_ptr(), S, cols.data_ptr(),
+                                            exits.data_ptr() if exits is not None else None, self.step_count + 1, K,
+                                            rewards.data_ptr(), dones.data_ptr(), int(bool(history)), self._stream()),
+                "fe_backtest_targets",
+            )
+        else:
+            _lib.check(
+                self._L.fe_backtest(self._pp, self._ps, self._pst, self._pm, self.metrics_capacity, self._stats_ptr,
+                                    signal.data_ptr(), S, cols.data_ptr(), self.step_count + 1, K, rewards.data_ptr(),
+                                    dones.data_ptr(), int(bool(history)), self._stream()),
+                "fe_backtest",
+            )
         self.step_count += K
         self._epoch += 1   # a CapturedRollout's observation is stale now
         out = {"steps": K}
@@ -811,10 +845,12 @@ class TimeSeriesEnv(BaseObject):
             out["rewards"], out["dones"] = rewards, dones
         return out
 
-    def evaluate_signal(self, signal: torch.Tensor, columns: Optional[torch.Tensor] = None) -> Dict:
+    def evaluate_signal(self, signal: torch.Tensor, columns: Optional[torch.Tensor] = None, *, targets: bool = False,
+                        exits: Optional[torch.Tensor] = None) -> Dict:
         """The evaluate-mode report of a signal table, the counterpart of evaluate_policy(): one backtest() launch of
         max(seg_len) - W steps (enough for every env to finish its current episode from any pointer; terminated envs
         collect zero reward, so running past the end changes nothing), then one host read of the terminated count.
+        `targets` / `exits` are backtest()'s (target positions, trailing stop and take-profit per signal row).
         Returns {"returns": (N,) f32, "steps", "metrics": each env's first episode in env order} and resets the
         evaluation metrics, as evaluate_policy() does.  Needs evaluate=True and track_metrics=True."""
         if not self.evaluate:
@@ -822,7 +858,7 @@ class TimeSeriesEnv(BaseObject):
         self._require_metrics()
         if getattr(self, "_signal_steps", None) is None:
             self._signal_steps = int(self.series.seg_len.max().item()) - self.num_intervals
-        steps = self.backtest(signal, self._signal_steps, columns)["steps"]
+        steps = self.backtest(signal, self._signal_steps, columns, targets=targets, exits=exits)["steps"]
         if int(self._stats[1].item()) >= self.num_envs:
             info = {"returns": self._ep_return.clone(), "steps": steps, "metrics": self._first_episode_metrics()}
             self.reset_evaluation_metrics()

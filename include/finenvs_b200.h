@@ -309,6 +309,30 @@ int fe_backtest(const FeParams *p, const FeSeries *s, const FeState *st, const F
                 FeStats *stats_dev, const float *signal_dev, int32_t num_signals, const int32_t *column_dev,
                 uint64_t first_step, int32_t num_steps, void *rewards_dev, int32_t *dones_dev, int32_t history, void *stream);
 
+/* Target-position backtests: as fe_backtest, but the table value v = signal[column[i], row] (same row) is the net
+ * position env i should hold, and exits_dev (num_signals, 2) double, or NULL, holds per column c a trailing stop
+ * exits[c][0] and a take-profit exits[c][1] in reward units (the episode's P&L).  Per env and step, on the state before
+ * the step, f32 unless noted (scale = (float)(max_shares + 0.5), ms = max_shares; sum, peak: the metrics' running
+ * state of the current episode):
+ *     T = clamp(rintf(v * scale), -ms, ms)                          target net position in shares
+ *     if exits_dev && ((peak - sum) >= exits[c][0] || sum >= exits[c][1])   (f64)
+ *         T = +0.0f                                                  go flat
+ *     D = T - (long - short)                                         share delta that reaches the target
+ *     a = D / scale                                                  (IEEE-rounded), the action of the step
+ * The step maps a back to clamp(rint(a * scale), -ms, ms) = clamp(D, -ms, ms): for |D| <= 2^21 the two rounding errors
+ * stay below 2^21 * 2^-23 = 0.25 shares (max_shares <= FE_TARGET_MAX_SHARES keeps scale exact; larger max_shares are
+ * FE_EINVAL), and beyond that bound they cannot bring |a * scale| below ms.  So a target backtest is bit-identical to
+ * fe_step calls with these actions computed by the caller, and follows the env's rules: a flip from +ms to -ms takes two
+ * steps (the first sells the longs, the short entry sees no sell order), an entry the cash cannot pay for is retried on
+ * the next step, and the exit rule is evaluated every step without latching: once flat the rewards are 0, sum and peak
+ * stay put and the env stays flat until its episode ends; the next episode trades again.  A threshold of +inf never
+ * triggers.  exits_dev must be 8-byte aligned (FE_EALIGN); the other checks are fe_backtest's. */
+#define FE_TARGET_MAX_SHARES (1 << 20)
+int fe_backtest_targets(const FeParams *p, const FeSeries *s, const FeState *st, const FeMetricsState *m,
+                        int64_t metrics_capacity, FeStats *stats_dev, const float *signal_dev, int32_t num_signals,
+                        const int32_t *column_dev, const double *exits_dev, uint64_t first_step, int32_t num_steps,
+                        void *rewards_dev, int32_t *dones_dev, int32_t history, void *stream);
+
 /* ---- ES rollout path (finenvs/agents/networks/parallel_mlp.py, finenvs/agents/ES/evo_agent.py) -------------
  * Population layout of the reference (parallel_mlp.py:121-136): envs [0, T/2) use theta + sigma*eps[p], envs
  * [T/2, T) use theta - sigma*eps[p - T/2] (T = num_envs - num_eval_envs, even), the last num_eval_envs envs use
