@@ -5,6 +5,9 @@
 #include <stdint.h>
 #include <stdlib.h>
 
+#include <atomic>
+#include <type_traits>
+
 namespace {
 
 // ------------------------------------------------------------------------------------------
@@ -152,6 +155,43 @@ inline int pointer_device(const void *ptr) {
     }
     return a.device;
 }
+
+// ------------------------------------------------------------------------------------------
+// host side: kernel set-up
+// ------------------------------------------------------------------------------------------
+// dynamic shared memory every large-smem kernel opts in to
+constexpr int kSmemMax = 226 * 1024;
+
+// SM count of `device`, queried once per device
+inline int device_sm_count(int device, int *out) {
+    static std::atomic<int> num_sms[16];
+    const int dev = device & 15;
+    int n = num_sms[dev].load(std::memory_order_relaxed);
+    if (!n) {
+        cudaError_t e = cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, device);
+        if (e != cudaSuccess) return (int)e;
+        num_sms[dev].store(n, std::memory_order_relaxed);
+    }
+    *out = n;
+    return 0;
+}
+
+// cudaFuncSetAttribute(max dynamic shared memory) once per (kernel instantiation, device); safe to race: the attribute
+// call is idempotent and the flag is only set after it succeeded
+template <auto Kern> int opt_in_smem(int device) {
+    static std::atomic<uint32_t> done_mask{0};
+    const uint32_t bit = 1u << (device & 15);
+    if (done_mask.load(std::memory_order_acquire) & bit) return 0;
+    cudaError_t e = cudaFuncSetAttribute(Kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax);
+    if (e != cudaSuccess) return (int)e;
+    done_mask.fetch_or(bit, std::memory_order_release);
+    return 0;
+}
+
+// Template arguments chosen at run time: f is called with a value of the chosen type (f(float{}) / f(double{}) for the
+// output dtype, f(std::true_type{}) / f(std::false_type{}) for a flag), so the launch it makes is written once.
+template <class F> int with_out_type(bool f64, F &&f) { return f64 ? f(double{}) : f(float{}); }
+template <class F> int with_flag(bool b, F &&f) { return b ? f(std::true_type{}) : f(std::false_type{}); }
 
 // tuning overrides exist only in experiment builds (-DFE_EXPERIMENTS, tools/build_*_variants.sh); the shipped library
 // reads no environment variable

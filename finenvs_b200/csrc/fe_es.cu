@@ -29,8 +29,6 @@
 #include <stdio.h>
 #include <stdlib.h>
 
-#include <atomic>
-
 namespace {
 
 constexpr int kEsWarps = 8;
@@ -866,7 +864,7 @@ EsRoute route_forward(const EsLayout &lay, const bool lazy, const bool obs_align
         f.tail_in_regs = lay.L == 2 && lay.out[1] <= 8;
         f.theta_bytes = (int)((P * 4 + 127) & ~(int64_t)127);
         rt.smem = fast_smem_bytes(f);
-        if (rt.smem <= 226 * 1024) {
+        if (rt.smem <= kSmemMax) {
             rt.kern = ES_FAST;
             return rt;
         }
@@ -891,9 +889,9 @@ EsRoute route_forward(const EsLayout &lay, const bool lazy, const bool obs_align
         f.strideA = (a + 1) & ~1;
         f.strideB = (b + 1) & ~1;
         f.U = kStMaxU;
-        while (f.U > 1 && stream_smem_bytes(f) > 226 * 1024) --f.U;
+        while (f.U > 1 && stream_smem_bytes(f) > kSmemMax) --f.U;
         rt.smem = stream_smem_bytes(f);
-        if (rt.smem <= 226 * 1024) {
+        if (rt.smem <= kSmemMax) {
             rt.kern = ES_STREAM;
             return rt;
         }
@@ -903,7 +901,7 @@ EsRoute route_forward(const EsLayout &lay, const bool lazy, const bool obs_align
     const size_t act_bytes = (size_t)kEsWarps * 4 * stride * sizeof(float);
     rt.theta_smem = act_bytes + (size_t)P * sizeof(float) <= 100 * 1024;
     rt.smem = act_bytes + (rt.theta_smem ? (size_t)P * sizeof(float) : 0);
-    rt.kern = rt.smem <= 226 * 1024 ? ES_GENERIC : ES_ERR_SMEM;
+    rt.kern = rt.smem <= kSmemMax ? ES_GENERIC : ES_ERR_SMEM;
     return rt;
 }
 
@@ -953,52 +951,50 @@ int fe_es_forward(const FeEsNet *net, const float *theta_packed_dev, const void 
     if (((uintptr_t)eps_dev | (uintptr_t)theta_packed_dev) & 15) return FE_EALIGN;
     const EsRoute rt = route_forward(lay, lazy, lazy || ((uintptr_t)obs_dev & 15) == 0);
     if (rt.kern == ES_ERR_SMEM) return FE_ESMEM;
-    cudaError_t e;
     DeviceGuard guard(device);
     if (guard.rc) return guard.rc;
-    static std::atomic<int> num_sms_cache[16];
-    const int dev = device & 15;
-    int num_sms[16];
-    num_sms[dev] = num_sms_cache[dev].load(std::memory_order_relaxed);
-    if (!num_sms[dev]) {
-        if ((e = cudaDeviceGetAttribute(&num_sms[dev], cudaDevAttrMultiProcessorCount, device)) != cudaSuccess) return (int)e;
-        num_sms_cache[dev].store(num_sms[dev], std::memory_order_relaxed);
-    }
+    int num_sms = 0;
+    if (const int rc = device_sm_count(device, &num_sms)) return rc;
     const int64_t units = train / 2 + num_eval_envs;
-    if (rt.kern == ES_FAST) {
-        auto kern = lazy ? fe_es_forward_fast_kernel<true> : fe_es_forward_fast_kernel<false>;
-        if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rt.smem)) != cudaSuccess) return (int)e;
-        int64_t blocks = (units + kFastWarps - 1) / kFastWarps;
-        if (blocks > num_sms[dev]) blocks = num_sms[dev];
-        kern<<<(unsigned)blocks, kFastThreads, rt.smem, (cudaStream_t)stream>>>(
-            lay, rt.fast, theta_packed_dev, (const __half *)eps_dev, sigma, train / 2, num_eval_envs, obs_dev,
-            (const float *)logret_dev, obs_row0_dev, obs_posfeat_dev, action_noise_std, seed, step_counter, env_id_base,
-            actions_dev);
-        return (int)cudaGetLastError();
-    }
-    if (rt.kern == ES_STREAM) {
-        auto kern = lazy ? fe_es_forward_stream_kernel<true> : fe_es_forward_stream_kernel<false>;
-        if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rt.smem)) != cudaSuccess) return (int)e;
-        int64_t blocks = (units + (int64_t)kStWarps * rt.stream.U - 1) / ((int64_t)kStWarps * rt.stream.U);
-        if (blocks > num_sms[dev]) blocks = num_sms[dev];
-        kern<<<(unsigned)blocks, kStThreads, rt.smem, (cudaStream_t)stream>>>(
-            lay, rt.stream, theta_packed_dev, (const __half *)eps_dev, sigma, train / 2, num_eval_envs, obs_dev,
-            (const float *)logret_dev, obs_row0_dev, obs_posfeat_dev, window, action_noise_std, seed, step_counter,
-            env_id_base, actions_dev);
-        return (int)cudaGetLastError();
-    }
-    auto kern = lazy ? (rt.theta_smem ? fe_es_forward_kernel<true, true> : fe_es_forward_kernel<true, false>)
-                     : (rt.theta_smem ? fe_es_forward_kernel<false, true> : fe_es_forward_kernel<false, false>);
-    if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rt.smem)) != cudaSuccess) return (int)e;
-    int per_sm = (int)((226 * 1024) / (rt.smem + 1024));
-    if (per_sm > 8) per_sm = 8;
-    if (per_sm < 1) per_sm = 1;
-    int64_t blocks = (units + kEsWarps - 1) / kEsWarps;
-    if (blocks > (int64_t)num_sms[dev] * per_sm) blocks = (int64_t)num_sms[dev] * per_sm;
-    kern<<<(unsigned)blocks, kEsThreads, rt.smem, (cudaStream_t)stream>>>(
-        lay, theta_packed_dev, (const __half *)eps_dev, sigma, train / 2, num_eval_envs, obs_dev, (const float *)logret_dev,
-        obs_row0_dev, obs_posfeat_dev, window, action_noise_std, seed, step_counter, env_id_base, actions_dev);
-    return (int)cudaGetLastError();
+    return with_flag(lazy, [&](auto lazy_obs) {
+        constexpr bool kLazy = decltype(lazy_obs)::value;
+        if (rt.kern == ES_FAST) {
+            constexpr auto kern = fe_es_forward_fast_kernel<kLazy>;
+            if (const int rc = opt_in_smem<kern>(device)) return rc;
+            int64_t blocks = (units + kFastWarps - 1) / kFastWarps;
+            if (blocks > num_sms) blocks = num_sms;
+            kern<<<(unsigned)blocks, kFastThreads, rt.smem, (cudaStream_t)stream>>>(
+                lay, rt.fast, theta_packed_dev, (const __half *)eps_dev, sigma, train / 2, num_eval_envs, obs_dev,
+                (const float *)logret_dev, obs_row0_dev, obs_posfeat_dev, action_noise_std, seed, step_counter, env_id_base,
+                actions_dev);
+            return (int)cudaGetLastError();
+        }
+        if (rt.kern == ES_STREAM) {
+            constexpr auto kern = fe_es_forward_stream_kernel<kLazy>;
+            if (const int rc = opt_in_smem<kern>(device)) return rc;
+            int64_t blocks = (units + (int64_t)kStWarps * rt.stream.U - 1) / ((int64_t)kStWarps * rt.stream.U);
+            if (blocks > num_sms) blocks = num_sms;
+            kern<<<(unsigned)blocks, kStThreads, rt.smem, (cudaStream_t)stream>>>(
+                lay, rt.stream, theta_packed_dev, (const __half *)eps_dev, sigma, train / 2, num_eval_envs, obs_dev,
+                (const float *)logret_dev, obs_row0_dev, obs_posfeat_dev, window, action_noise_std, seed, step_counter,
+                env_id_base, actions_dev);
+            return (int)cudaGetLastError();
+        }
+        return with_flag(rt.theta_smem, [&](auto theta_smem) {
+            constexpr auto kern = fe_es_forward_kernel<kLazy, decltype(theta_smem)::value>;
+            if (const int rc = opt_in_smem<kern>(device)) return rc;
+            int per_sm = (int)(kSmemMax / (rt.smem + 1024));
+            if (per_sm > 8) per_sm = 8;
+            if (per_sm < 1) per_sm = 1;
+            int64_t blocks = (units + kEsWarps - 1) / kEsWarps;
+            if (blocks > (int64_t)num_sms * per_sm) blocks = (int64_t)num_sms * per_sm;
+            kern<<<(unsigned)blocks, kEsThreads, rt.smem, (cudaStream_t)stream>>>(
+                lay, theta_packed_dev, (const __half *)eps_dev, sigma, train / 2, num_eval_envs, obs_dev,
+                (const float *)logret_dev, obs_row0_dev, obs_posfeat_dev, window, action_noise_std, seed, step_counter,
+                env_id_base, actions_dev);
+            return (int)cudaGetLastError();
+        });
+    });
 }
 
 const char *fe_es_forward_kernel_name(const FeEsNet *net, int32_t lazy, int32_t obs_aligned) {
@@ -1058,15 +1054,13 @@ int fe_es_store(const void *rewards_dev, int32_t rewards_f64, const int32_t *don
     DeviceGuard guard(pointer_device(rewards_dev));
     if (guard.rc) return guard.rc;
     const unsigned blocks = (unsigned)((num_envs + 255) / 256);
-    if (rewards_f64)
-        fe_es_store_kernel<double><<<blocks, 256, 0, (cudaStream_t)stream>>>(
-            (const double *)rewards_dev, dones_dev, num_envs, env_id_base, total_envs, step_ordinal, cur_returns_dev,
+    return with_out_type(rewards_f64 != 0, [&](auto rew_type) {
+        using RewT = decltype(rew_type);
+        fe_es_store_kernel<RewT><<<blocks, 256, 0, (cudaStream_t)stream>>>(
+            (const RewT *)rewards_dev, dones_dev, num_envs, env_id_base, total_envs, step_ordinal, cur_returns_dev,
             cur_steps_dev, capacity, counters_dev, fin_key_dev, fin_env_dev, fin_ret_dev);
-    else
-        fe_es_store_kernel<float><<<blocks, 256, 0, (cudaStream_t)stream>>>(
-            (const float *)rewards_dev, dones_dev, num_envs, env_id_base, total_envs, step_ordinal, cur_returns_dev,
-            cur_steps_dev, capacity, counters_dev, fin_key_dev, fin_env_dev, fin_ret_dev);
-    return (int)cudaGetLastError();
+        return (int)cudaGetLastError();
+    });
 }
 
 } // extern "C"

@@ -143,13 +143,11 @@ extern "C" int fe_episode_metrics(const FeParams *p, const FeMetricsState *m, co
     if (!p->evaluate) ms.emitted = nullptr;
     const unsigned blocks = (unsigned)((p->num_envs + kThreads - 1) / kThreads);
     cudaStream_t q = (cudaStream_t)stream;
-    if (p->out_f64)
-        fe_episode_metrics_kernel<double><<<blocks, kThreads, 0, q>>>((const double *)rewards_dev, dones_dev, p->num_envs,
-                                                                 p->env_id_base, p->total_envs, p->starting_balance, ms,
-                                                                 step_counter, step_counter_dev, capacity);
-    else
-        fe_episode_metrics_kernel<float><<<blocks, kThreads, 0, q>>>((const float *)rewards_dev, dones_dev, p->num_envs,
-                                                                p->env_id_base, p->total_envs, p->starting_balance, ms,
-                                                                step_counter, step_counter_dev, capacity);
-    return (int)cudaGetLastError();
+    return with_out_type(p->out_f64, [&](auto out_type) {
+        using OutT = decltype(out_type);
+        fe_episode_metrics_kernel<OutT><<<blocks, kThreads, 0, q>>>((const OutT *)rewards_dev, dones_dev, p->num_envs,
+                                                                    p->env_id_base, p->total_envs, p->starting_balance, ms,
+                                                                    step_counter, step_counter_dev, capacity);
+        return (int)cudaGetLastError();
+    });
 }

@@ -78,11 +78,10 @@ extern "C" int fe_returns_advantages(const void *rewards_dev, int32_t rewards_f6
     if (guard.rc) return guard.rc;
     const unsigned blocks = (unsigned)((num_envs + 255) / 256);
     cudaStream_t q = (cudaStream_t)stream;
-    if (rewards_f64)
-        fe_returns_kernel<double><<<blocks, 256, 0, q>>>((const double *)rewards_dev, dones_dev, values_dev, last_values_dev,
-                                                         num_envs, num_steps, (float)gamma, returns_dev, advantages_dev);
-    else
-        fe_returns_kernel<float><<<blocks, 256, 0, q>>>((const float *)rewards_dev, dones_dev, values_dev, last_values_dev,
-                                                        num_envs, num_steps, (float)gamma, returns_dev, advantages_dev);
-    return (int)cudaGetLastError();
+    return with_out_type(rewards_f64 != 0, [&](auto rew_type) {
+        using RewT = decltype(rew_type);
+        fe_returns_kernel<RewT><<<blocks, 256, 0, q>>>((const RewT *)rewards_dev, dones_dev, values_dev, last_values_dev,
+                                                       num_envs, num_steps, (float)gamma, returns_dev, advantages_dev);
+        return (int)cudaGetLastError();
+    });
 }

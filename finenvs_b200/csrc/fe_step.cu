@@ -26,7 +26,6 @@
 #include <stdint.h>
 #include <stdlib.h>
 
-#include <atomic>
 #include <mutex>
 #include <vector>
 
@@ -35,7 +34,6 @@ namespace {
 constexpr int kThreads = 128;          // threads per block (both variants)
 constexpr int kMaxTileEnvs = kThreads; // one bookkeeping thread per env of the tile
 constexpr int kSmemHeader = 16;        // mbarrier (8 B) + pad
-constexpr int kSmemMax = 226 * 1024;
 
 // ------------------------------------------------------------------------------------------
 // exact (never contracted) arithmetic helpers
@@ -1821,6 +1819,14 @@ int check_common(const FeParams *p, const FeSeries *s, const FeState *st) {
     return 0;
 }
 
+// check_common for the entry points that step: accumulating FeStats outside evaluate mode reads and writes the
+// episode returns and lengths
+int check_step(const FeParams *p, const FeSeries *s, const FeState *st, const FeStats *stats) {
+    const int rc = check_common(p, s, st);
+    if (rc) return rc;
+    return stats && !p->evaluate && (!st->ep_return || !st->ep_len) ? FE_EINVAL : 0;
+}
+
 // Tile shape.  Measured on B200 (tools/sweep_tile.sh, 1 Mi envs, W=60): the step is latency-bound per
 // block (state loads -> table lookup -> window copy -> interleave -> store), so MANY SMALL blocks in
 // flight beat few large ones: 4 envs x 32 threads (23 blocks/SM) runs 0.35 ms where 32 envs x 128
@@ -1867,19 +1873,6 @@ int pick_gather_stages(int W, bool f64) {
 }
 // the observation-layout table is worth reading only while it stays L2-resident next to the observation stream
 bool gather_table_resident(const FeParams &p, bool f64) { return ga_table_bytes(p.num_rows, p.window, f64) <= ((size_t)64 << 20); }
-
-int device_sm_count(int device, int *out) {
-    static std::atomic<int> num_sms[16];
-    const int dev = device & 15;
-    int n = num_sms[dev].load(std::memory_order_relaxed);
-    if (!n) {
-        cudaError_t e = cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, device);
-        if (e != cudaSuccess) return (int)e;
-        num_sms[dev].store(n, std::memory_order_relaxed);
-    }
-    *out = n;
-    return 0;
-}
 
 // Which kernel a launch uses.  `auto`: portfolio when A > 1; for populations that give every SM a few tiles and windows
 // of >= 24 rows a persistent kernel — gather when the caller staged the observation-layout table (FeSeries.obs_table),
@@ -1937,19 +1930,9 @@ StepChoice choose_kernel(const FeParams &p, bool gather_ready, bool f64, int sms
     return c;
 }
 
-// cudaFuncSetAttribute(max dynamic shared memory) once per (kernel instantiation, device); safe to race: the attribute
-// call is idempotent and the flag is only set after it succeeded
-template <typename Kern> int opt_in_smem(Kern kern, std::atomic<uint32_t> &done_mask, int device) {
-    const uint32_t bit = 1u << (device & 15);
-    if (done_mask.load(std::memory_order_acquire) & bit) return 0;
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemMax);
-    if (e != cudaSuccess) return (int)e;
-    done_mask.fetch_or(bit, std::memory_order_release);
-    return 0;
-}
-
-// Tensor map of the observation-layout table (gather variant): rows of `inner_bytes` at an 80-byte pitch — the rows
-// overlap, row i is the window starting i pitches into a shifted copy.  Encoded by the driver (cuTensorMapEncodeTiled,
+// Geometry and tensor map of the observation-layout table, shared by the gather step and gather_obs: `rpp` tensor rows
+// per shifted copy, each window read in `parts` box rows of `inner_bytes` at an 80-byte pitch — the rows overlap, row i
+// is the window starting i pitches into a shifted copy.  The map is encoded by the driver (cuTensorMapEncodeTiled,
 // resolved through the runtime so that libcuda is not a link dependency) and cached: a step costs no driver call.
 typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
                                   const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
@@ -1960,13 +1943,24 @@ struct TmapEntry {
     int inner_bytes, device;
     CUtensorMap map;
 };
-int gather_tensor_map(const void *table, int64_t total_rows, int inner_bytes, int device, CUtensorMap *out) {
+struct ObsTableMap {
+    CUtensorMap map;
+    int64_t rpp;
+    int parts;
+};
+int gather_tensor_map(const FeParams &p, const FeSeries &s, bool f64, ObsTableMap *out) {
+    out->rpp = ga_rows_per_phase(p.num_rows, p.window, f64);
+    out->parts = ga_parts(p.window, f64);
+    const int64_t total_rows = out->rpp << ga_phase_shift(f64);
+    if (total_rows >= ((int64_t)1 << 31)) return FE_EINVAL;
+    const void *table = s.obs_table;
+    const int inner_bytes = ga_row_bytes(f64) * p.window / out->parts, device = p.device;
     static std::mutex mu;
     static std::vector<TmapEntry> cache;
     static EncodeTiledFn encode = nullptr;
     std::lock_guard<std::mutex> lock(mu);
     for (const TmapEntry &e : cache)
-        if (e.base == table && e.rows == total_rows && e.inner_bytes == inner_bytes && e.device == device) { *out = e.map; return 0; }
+        if (e.base == table && e.rows == total_rows && e.inner_bytes == inner_bytes && e.device == device) { out->map = e.map; return 0; }
     if (!encode) {
         void *fn = nullptr;
         cudaDriverEntryPointQueryResult q;
@@ -1986,7 +1980,7 @@ int gather_tensor_map(const void *table, int64_t total_rows, int inner_bytes, in
     if (r != CUDA_SUCCESS) return FE_EDRIVER;
     if (cache.size() >= 64) cache.erase(cache.begin());
     cache.push_back(n);
-    *out = n.map;
+    out->map = n.map;
     return 0;
 }
 
@@ -2024,9 +2018,8 @@ int launch(const FeParams &p, const FeSeries &s, const FeState &st, const float 
         if (CH > ((P + 3) & ~3)) CH = (P + 3) & ~3;
         const size_t smem = port_smem_bytes<OutT>(CH);
         if (smem > (size_t)kSmemMax) return FE_ESMEM;
-        auto skern = fe_portfolio_stream_kernel<OutT>;
-        static std::atomic<uint32_t> configured{0};
-        if ((rc = opt_in_smem(skern, configured, p.device))) return rc;
+        constexpr auto skern = fe_portfolio_stream_kernel<OutT>;
+        if ((rc = opt_in_smem<skern>(p.device))) return rc;
         fe_portfolio_book_kernel<OutT, kObserve><<<(unsigned)((p.num_envs + kBookWarps - 1) / kBookWarps), kBookWarps * 32, 0, stream>>>(
             p, s, st, k, actions, (OutT *)obs, (OutT *)rewards, dones, stats, step, step_dev);
         skern<<<(unsigned)p.num_envs, kPortThreads, smem, stream>>>(p, s, (OutT *)obs, CH);
@@ -2045,56 +2038,36 @@ int launch(const FeParams &p, const FeSeries &s, const FeState &st, const float 
     }
     case K_GATHER: {
         if ((uintptr_t)obs & 15) return FE_EALIGN;
-        constexpr bool f64 = sizeof(OutT) == 8;
-        const int64_t rpp = ga_rows_per_phase(p.num_rows, p.window, f64);
-        const int64_t total_rows = rpp << ga_phase_shift(f64);
-        if (total_rows >= ((int64_t)1 << 31)) return FE_EINVAL;
-        const int parts = ga_parts(p.window, f64);
-        CUtensorMap tmap;
-        if ((rc = gather_tensor_map(s.obs_table, total_rows, ga_row_bytes(f64) * p.window / parts, p.device, &tmap))) return rc;
+        ObsTableMap tab;
+        if ((rc = gather_tensor_map(p, s, sizeof(OutT) == 8, &tab))) return rc;
         const int64_t ntiles = (p.num_envs + 31) / 32;
         const unsigned blocks = (unsigned)(ntiles < sms ? ntiles : sms);
         const size_t smem = gather_smem_bytes<OutT>(p.window, c.S);
-        if (parts == 1) {
-            auto kern = fe_gather_kernel<OutT, kObserve, 1>;
-            static std::atomic<uint32_t> configured{0};
-            if ((rc = opt_in_smem(kern, configured, p.device))) return rc;
-            kern<<<blocks, kGaThreads, smem, stream>>>(tmap, p, s, st, k, actions, (OutT *)obs, (OutT *)rewards, dones, stats, step,
-                                                       step_dev, c.S, (int)rpp, st.sched);
-        } else {
-            auto kern = fe_gather_kernel<OutT, kObserve, 2>;
-            static std::atomic<uint32_t> configured{0};
-            if ((rc = opt_in_smem(kern, configured, p.device))) return rc;
-            kern<<<blocks, kGaThreads, smem, stream>>>(tmap, p, s, st, k, actions, (OutT *)obs, (OutT *)rewards, dones, stats, step,
-                                                       step_dev, c.S, (int)rpp, st.sched);
-        }
-        break;
+        return with_flag(tab.parts == 2, [&](auto two_parts) {
+            constexpr auto kern = fe_gather_kernel<OutT, kObserve, decltype(two_parts)::value ? 2 : 1>;
+            if (const int r = opt_in_smem<kern>(p.device)) return r;
+            kern<<<blocks, kGaThreads, smem, stream>>>(tab.map, p, s, st, k, actions, (OutT *)obs, (OutT *)rewards, dones, stats,
+                                                       step, step_dev, c.S, (int)tab.rpp, st.sched);
+            return (int)cudaGetLastError();
+        });
     }
     case K_PIPE: {
         if ((uintptr_t)obs & 15) return FE_EALIGN;
         const int64_t ntiles = (p.num_envs + c.te - 1) / c.te;
         const unsigned blocks = (unsigned)(ntiles < sms ? ntiles : sms);
-        if (c.sin == 0) {
-            auto kern = fe_pipe_kernel<OutT, kObserve, 0>;
-            static std::atomic<uint32_t> configured{0};
-            if ((rc = opt_in_smem(kern, configured, p.device))) return rc;
+        return with_flag(c.sin != 0, [&](auto stream_flavour) {
+            constexpr auto kern = fe_pipe_kernel<OutT, kObserve, decltype(stream_flavour)::value ? kPipeSInStream : 0>;
+            if (const int r = opt_in_smem<kern>(p.device)) return r;
             kern<<<blocks, kPipeThreads, pipe_smem_bytes<OutT>(c.te, p.window, c.sin), stream>>>(
                 p, s, st, k, actions, (OutT *)obs, (OutT *)rewards, dones, stats, step, step_dev, c.te);
-        } else {
-            auto kern = fe_pipe_kernel<OutT, kObserve, kPipeSInStream>;
-            static std::atomic<uint32_t> configured{0};
-            if ((rc = opt_in_smem(kern, configured, p.device))) return rc;
-            kern<<<blocks, kPipeThreads, pipe_smem_bytes<OutT>(c.te, p.window, c.sin), stream>>>(
-                p, s, st, k, actions, (OutT *)obs, (OutT *)rewards, dones, stats, step, step_dev, c.te);
-        }
-        break;
+            return (int)cudaGetLastError();
+        });
     }
     case K_TILE: {
         if ((uintptr_t)obs & 15) return FE_EALIGN;
         const size_t smem = tile_smem_bytes<OutT>(c.te, p.window);
-        auto kern = fe_tile_kernel<OutT, kObserve>;
-        static std::atomic<uint32_t> configured{0};
-        if ((rc = opt_in_smem(kern, configured, p.device))) return rc;
+        constexpr auto kern = fe_tile_kernel<OutT, kObserve>;
+        if ((rc = opt_in_smem<kern>(p.device))) return rc;
         const int64_t blocks = (p.num_envs + c.te - 1) / c.te;
         kern<<<(unsigned)blocks, c.threads, smem, stream>>>(p, s, st, k, actions, (OutT *)obs, (OutT *)rewards, dones,
                                                              stats, step, step_dev, c.te);
@@ -2133,11 +2106,8 @@ int gather_obs(const FeParams &p, const FeSeries &s, const int64_t *row0, const 
     int sms = 0;
     int rc = device_sm_count(p.device, &sms);
     if (rc) return rc;
-    const int64_t rpp = ga_rows_per_phase(p.num_rows, p.window, f64);
-    const int parts = ga_parts(p.window, f64);
-    CUtensorMap tmap;
-    if ((rc = gather_tensor_map(s.obs_table, rpp << ga_phase_shift(f64), ga_row_bytes(f64) * p.window / parts, p.device, &tmap)))
-        return rc;
+    ObsTableMap tab;
+    if ((rc = gather_tensor_map(p, s, f64, &tab))) return rc;
     // 3 slots per warp when at least 8 warps of them fit in shared memory, else 2; up to 16 warps per block and, for short
     // windows whose rings are small, up to 4 blocks per SM
     const size_t pitch = ga_slot_pitch(p.window, f64), room = (size_t)kSmemMax - kGoBarBytes;
@@ -2149,18 +2119,13 @@ int gather_obs(const FeParams &p, const FeSeries &s, const int64_t *row0, const 
     per_sm = per_sm < 1 ? 1 : per_sm > 4 ? 4 : per_sm;
     const int64_t need = ((count + 31) / 32 + warps - 1) / warps;
     const unsigned blocks = (unsigned)(need < (int64_t)sms * per_sm ? need : (int64_t)sms * per_sm);
-    if (parts == 1) {
-        auto kern = fe_gather_obs_kernel<OutT, 1>;
-        static std::atomic<uint32_t> configured{0};
-        if ((rc = opt_in_smem(kern, configured, p.device))) return rc;
-        kern<<<blocks, warps * 32, smem, stream>>>(tmap, count, p.window, row0, (const OutT *)pf, index, (OutT *)obs, S, (int)rpp);
-    } else {
-        auto kern = fe_gather_obs_kernel<OutT, 2>;
-        static std::atomic<uint32_t> configured{0};
-        if ((rc = opt_in_smem(kern, configured, p.device))) return rc;
-        kern<<<blocks, warps * 32, smem, stream>>>(tmap, count, p.window, row0, (const OutT *)pf, index, (OutT *)obs, S, (int)rpp);
-    }
-    return (int)cudaGetLastError();
+    return with_flag(tab.parts == 2, [&](auto two_parts) {
+        constexpr auto kern = fe_gather_obs_kernel<OutT, decltype(two_parts)::value ? 2 : 1>;
+        if (const int r = opt_in_smem<kern>(p.device)) return r;
+        kern<<<blocks, warps * 32, smem, stream>>>(tab.map, count, p.window, row0, (const OutT *)pf, index, (OutT *)obs, S,
+                                                   (int)tab.rpp);
+        return (int)cudaGetLastError();
+    });
 }
 
 // step ordinal kept on the device (fe_step_captured): one thread bumps it ahead of the step kernel
@@ -2404,6 +2369,37 @@ fe_backtest_targets_kernel(const FeParams p, const FeSeries s, const FeState st,
     backtest_run<OutT>(p, s, st, k, m, capacity, stats, signal, column, first_step, K, rewards, dones, history, rule);
 }
 
+// fe_backtest (kTargets = false, exits == nullptr) and fe_backtest_targets: validation and launch
+template <bool kTargets>
+int backtest_entry(const FeParams *p, const FeSeries *s, const FeState *st, const FeMetricsState *m, int64_t capacity,
+                   FeStats *stats, const float *signal, int32_t num_signals, const int32_t *column, const double *exits,
+                   uint64_t first_step, int32_t num_steps, void *rewards, int32_t *dones, int32_t history, void *stream) {
+    int rc = check_step(p, s, st, stats);
+    if (rc) return rc;
+    if (p->num_assets != 1 || !signal || num_signals < 1 || !column || num_steps < 1 || !rewards || !dones) return FE_EINVAL;
+    if (kTargets && (p->max_shares < 1 || p->max_shares > FE_TARGET_MAX_SHARES)) return FE_EINVAL;
+    if ((uintptr_t)exits & 7) return FE_EALIGN;
+    if ((rc = check_metrics_state(p, m, capacity))) return rc;
+    DeviceGuard guard(p->device);
+    if (guard.rc) return guard.rc;
+    const Consts k = make_consts(*p);
+    FeMetricsState ms = *m;
+    if (!p->evaluate) ms.emitted = nullptr;
+    const unsigned blocks = (unsigned)((p->num_envs + kBtThreads - 1) / kBtThreads);
+    cudaStream_t q = (cudaStream_t)stream;
+    return with_out_type(p->out_f64, [&](auto out_type) {
+        using OutT = decltype(out_type);
+        if constexpr (kTargets)
+            fe_backtest_targets_kernel<OutT><<<blocks, kBtThreads, 0, q>>>(*p, *s, *st, k, ms, capacity, stats, signal, column,
+                                                                           exits, first_step, num_steps, (OutT *)rewards, dones,
+                                                                           history);
+        else
+            fe_backtest_kernel<OutT><<<blocks, kBtThreads, 0, q>>>(*p, *s, *st, k, ms, capacity, stats, signal, column,
+                                                                   first_step, num_steps, (OutT *)rewards, dones, history);
+        return (int)cudaGetLastError();
+    });
+}
+
 // side streams of fe_step_host (created once per device, never destroyed: they live as long as the process)
 constexpr int kHostStreams = 3;
 struct HostPipe {
@@ -2504,9 +2500,11 @@ int fe_obs_table_build(const void *logret_dev, int64_t num_rows, int32_t window,
     const int64_t rpp = ga_rows_per_phase(num_rows, window, f64);
     const int64_t threads = num_rows << ga_phase_shift(f64);
     const unsigned blocks = (unsigned)((threads + 255) / 256);
-    if (f64) fe_obs_table_kernel<double><<<blocks, 256, 0, q>>>((const double *)logret_dev, num_rows, rpp, (unsigned char *)table_dev);
-    else fe_obs_table_kernel<float><<<blocks, 256, 0, q>>>((const float *)logret_dev, num_rows, rpp, (unsigned char *)table_dev);
-    return (int)cudaGetLastError();
+    return with_out_type(f64, [&](auto out_type) {
+        using OutT = decltype(out_type);
+        fe_obs_table_kernel<OutT><<<blocks, 256, 0, q>>>((const OutT *)logret_dev, num_rows, rpp, (unsigned char *)table_dev);
+        return (int)cudaGetLastError();
+    });
 }
 
 int fe_log_returns(const double *prices_dev, int64_t num_rows, int32_t num_assets, double *logret64_dev,
@@ -2533,38 +2531,37 @@ int fe_observe(const FeParams *p, const FeSeries *s, const FeState *st, void *ob
     if (!obs_dev) return FE_EINVAL;
     DeviceGuard guard(p->device);
     if (guard.rc) return guard.rc;
-    return p->out_f64 ? launch<double, true>(*p, *s, *st, nullptr, obs_dev, nullptr, nullptr, nullptr, 0, (cudaStream_t)stream)
-                      : launch<float, true>(*p, *s, *st, nullptr, obs_dev, nullptr, nullptr, nullptr, 0, (cudaStream_t)stream);
+    return with_out_type(p->out_f64, [&](auto out_type) {
+        return launch<decltype(out_type), true>(*p, *s, *st, nullptr, obs_dev, nullptr, nullptr, nullptr, 0, (cudaStream_t)stream);
+    });
 }
 
 int fe_step(const FeParams *p, const FeSeries *s, const FeState *st, const float *actions_dev, void *obs_dev,
             void *rewards_dev, int32_t *dones_dev, FeStats *stats_dev, uint64_t step_counter, void *stream) {
-    int rc = check_common(p, s, st);
+    int rc = check_step(p, s, st, stats_dev);
     if (rc) return rc;
     if (!actions_dev || !obs_dev || !rewards_dev || !dones_dev) return FE_EINVAL;
-    if (stats_dev && !p->evaluate && (!st->ep_return || !st->ep_len)) return FE_EINVAL;
     DeviceGuard guard(p->device);
     if (guard.rc) return guard.rc;
-    return p->out_f64 ? launch<double, false>(*p, *s, *st, actions_dev, obs_dev, rewards_dev, dones_dev, stats_dev,
-                                              step_counter, (cudaStream_t)stream)
-                      : launch<float, false>(*p, *s, *st, actions_dev, obs_dev, rewards_dev, dones_dev, stats_dev,
-                                             step_counter, (cudaStream_t)stream);
+    return with_out_type(p->out_f64, [&](auto out_type) {
+        return launch<decltype(out_type), false>(*p, *s, *st, actions_dev, obs_dev, rewards_dev, dones_dev, stats_dev,
+                                                 step_counter, (cudaStream_t)stream);
+    });
 }
 
 int fe_step_captured(const FeParams *p, const FeSeries *s, const FeState *st, const float *actions_dev, void *obs_dev,
                      void *rewards_dev, int32_t *dones_dev, FeStats *stats_dev, uint64_t *step_counter_dev, void *stream) {
-    int rc = check_common(p, s, st);
+    int rc = check_step(p, s, st, stats_dev);
     if (rc) return rc;
     if (!actions_dev || !obs_dev || !rewards_dev || !dones_dev || !step_counter_dev) return FE_EINVAL;
-    if (stats_dev && !p->evaluate && (!st->ep_return || !st->ep_len)) return FE_EINVAL;
     DeviceGuard guard(p->device);
     if (guard.rc) return guard.rc;
     fe_bump_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(step_counter_dev);
     if ((rc = (int)cudaGetLastError())) return rc;
-    return p->out_f64 ? launch<double, false>(*p, *s, *st, actions_dev, obs_dev, rewards_dev, dones_dev, stats_dev, 0,
-                                              (cudaStream_t)stream, step_counter_dev)
-                      : launch<float, false>(*p, *s, *st, actions_dev, obs_dev, rewards_dev, dones_dev, stats_dev, 0,
-                                             (cudaStream_t)stream, step_counter_dev);
+    return with_out_type(p->out_f64, [&](auto out_type) {
+        return launch<decltype(out_type), false>(*p, *s, *st, actions_dev, obs_dev, rewards_dev, dones_dev, stats_dev, 0,
+                                                 (cudaStream_t)stream, step_counter_dev);
+    });
 }
 
 int fe_observe_lazy(const FeParams *p, const FeSeries *s, const FeState *st, int64_t *obs_row0_dev, void *obs_posfeat_dev,
@@ -2576,92 +2573,46 @@ int fe_observe_lazy(const FeParams *p, const FeSeries *s, const FeState *st, int
     if (guard.rc) return guard.rc;
     const Consts k = make_consts(*p);
     const unsigned blocks = (unsigned)((p->num_envs + kThreads - 1) / kThreads);
-    if (p->out_f64)
-        fe_lazy_kernel<double, true><<<blocks, kThreads, 0, (cudaStream_t)stream>>>(
-            *p, *s, *st, k, nullptr, obs_row0_dev, (double *)obs_posfeat_dev, nullptr, nullptr, nullptr, 0, nullptr);
-    else
-        fe_lazy_kernel<float, true><<<blocks, kThreads, 0, (cudaStream_t)stream>>>(
-            *p, *s, *st, k, nullptr, obs_row0_dev, (float *)obs_posfeat_dev, nullptr, nullptr, nullptr, 0, nullptr);
-    return (int)cudaGetLastError();
+    return with_out_type(p->out_f64, [&](auto out_type) {
+        using OutT = decltype(out_type);
+        fe_lazy_kernel<OutT, true><<<blocks, kThreads, 0, (cudaStream_t)stream>>>(
+            *p, *s, *st, k, nullptr, obs_row0_dev, (OutT *)obs_posfeat_dev, nullptr, nullptr, nullptr, 0, nullptr);
+        return (int)cudaGetLastError();
+    });
 }
 
 int fe_step_lazy(const FeParams *p, const FeSeries *s, const FeState *st, const float *actions_dev, int64_t *obs_row0_dev,
                  void *obs_posfeat_dev, void *rewards_dev, int32_t *dones_dev, FeStats *stats_dev, uint64_t step_counter,
                  void *stream) {
-    int rc = check_common(p, s, st);
+    int rc = check_step(p, s, st, stats_dev);
     if (rc) return rc;
     if (!actions_dev || !obs_row0_dev || !obs_posfeat_dev || !rewards_dev || !dones_dev || p->num_assets != 1) return FE_EINVAL;
-    if (stats_dev && !p->evaluate && (!st->ep_return || !st->ep_len)) return FE_EINVAL;
     DeviceGuard guard(p->device);
     if (guard.rc) return guard.rc;
     const Consts k = make_consts(*p);
     const unsigned blocks = (unsigned)((p->num_envs + kThreads - 1) / kThreads);
-    if (p->out_f64)
-        fe_lazy_kernel<double, false><<<blocks, kThreads, 0, (cudaStream_t)stream>>>(
-            *p, *s, *st, k, actions_dev, obs_row0_dev, (double *)obs_posfeat_dev, (double *)rewards_dev, dones_dev, stats_dev,
+    return with_out_type(p->out_f64, [&](auto out_type) {
+        using OutT = decltype(out_type);
+        fe_lazy_kernel<OutT, false><<<blocks, kThreads, 0, (cudaStream_t)stream>>>(
+            *p, *s, *st, k, actions_dev, obs_row0_dev, (OutT *)obs_posfeat_dev, (OutT *)rewards_dev, dones_dev, stats_dev,
             step_counter, nullptr);
-    else
-        fe_lazy_kernel<float, false><<<blocks, kThreads, 0, (cudaStream_t)stream>>>(
-            *p, *s, *st, k, actions_dev, obs_row0_dev, (float *)obs_posfeat_dev, (float *)rewards_dev, dones_dev, stats_dev,
-            step_counter, nullptr);
-    return (int)cudaGetLastError();
+        return (int)cudaGetLastError();
+    });
 }
 
 int fe_backtest(const FeParams *p, const FeSeries *s, const FeState *st, const FeMetricsState *m, int64_t metrics_capacity,
                 FeStats *stats_dev, const float *signal_dev, int32_t num_signals, const int32_t *column_dev,
                 uint64_t first_step, int32_t num_steps, void *rewards_dev, int32_t *dones_dev, int32_t history, void *stream) {
-    int rc = check_common(p, s, st);
-    if (rc) return rc;
-    if (p->num_assets != 1 || !signal_dev || num_signals < 1 || !column_dev || num_steps < 1 || !rewards_dev || !dones_dev)
-        return FE_EINVAL;
-    if (stats_dev && !p->evaluate && (!st->ep_return || !st->ep_len)) return FE_EINVAL;
-    if ((rc = check_metrics_state(p, m, metrics_capacity))) return rc;
-    DeviceGuard guard(p->device);
-    if (guard.rc) return guard.rc;
-    const Consts k = make_consts(*p);
-    FeMetricsState ms = *m;
-    if (!p->evaluate) ms.emitted = nullptr;
-    const unsigned blocks = (unsigned)((p->num_envs + kBtThreads - 1) / kBtThreads);
-    cudaStream_t q = (cudaStream_t)stream;
-    if (p->out_f64)
-        fe_backtest_kernel<double><<<blocks, kBtThreads, 0, q>>>(*p, *s, *st, k, ms, metrics_capacity, stats_dev, signal_dev,
-                                                                 column_dev, first_step, num_steps, (double *)rewards_dev,
-                                                                 dones_dev, history);
-    else
-        fe_backtest_kernel<float><<<blocks, kBtThreads, 0, q>>>(*p, *s, *st, k, ms, metrics_capacity, stats_dev, signal_dev,
-                                                                column_dev, first_step, num_steps, (float *)rewards_dev,
-                                                                dones_dev, history);
-    return (int)cudaGetLastError();
+    return backtest_entry<false>(p, s, st, m, metrics_capacity, stats_dev, signal_dev, num_signals, column_dev, nullptr,
+                                 first_step, num_steps, rewards_dev, dones_dev, history, stream);
 }
 
 int fe_backtest_targets(const FeParams *p, const FeSeries *s, const FeState *st, const FeMetricsState *m,
                         int64_t metrics_capacity, FeStats *stats_dev, const float *signal_dev, int32_t num_signals,
                         const int32_t *column_dev, const double *exits_dev, uint64_t first_step, int32_t num_steps,
                         void *rewards_dev, int32_t *dones_dev, int32_t history, void *stream) {
-    int rc = check_common(p, s, st);
-    if (rc) return rc;
-    if (p->num_assets != 1 || !signal_dev || num_signals < 1 || !column_dev || num_steps < 1 || !rewards_dev || !dones_dev)
-        return FE_EINVAL;
-    if (p->max_shares < 1 || p->max_shares > FE_TARGET_MAX_SHARES) return FE_EINVAL;
-    if ((uintptr_t)exits_dev & 7) return FE_EALIGN;
-    if (stats_dev && !p->evaluate && (!st->ep_return || !st->ep_len)) return FE_EINVAL;
-    if ((rc = check_metrics_state(p, m, metrics_capacity))) return rc;
-    DeviceGuard guard(p->device);
-    if (guard.rc) return guard.rc;
-    const Consts k = make_consts(*p);
-    FeMetricsState ms = *m;
-    if (!p->evaluate) ms.emitted = nullptr;
-    const unsigned blocks = (unsigned)((p->num_envs + kBtThreads - 1) / kBtThreads);
-    cudaStream_t q = (cudaStream_t)stream;
-    if (p->out_f64)
-        fe_backtest_targets_kernel<double><<<blocks, kBtThreads, 0, q>>>(*p, *s, *st, k, ms, metrics_capacity, stats_dev,
-                                                                         signal_dev, column_dev, exits_dev, first_step,
-                                                                         num_steps, (double *)rewards_dev, dones_dev, history);
-    else
-        fe_backtest_targets_kernel<float><<<blocks, kBtThreads, 0, q>>>(*p, *s, *st, k, ms, metrics_capacity, stats_dev,
-                                                                        signal_dev, column_dev, exits_dev, first_step,
-                                                                        num_steps, (float *)rewards_dev, dones_dev, history);
-    return (int)cudaGetLastError();
+    return backtest_entry<true>(p, s, st, m, metrics_capacity, stats_dev, signal_dev, num_signals, column_dev, exits_dev,
+                                first_step, num_steps, rewards_dev, dones_dev, history, stream);
 }
 
 int fe_materialize(const FeParams *p, const FeSeries *s, const int64_t *obs_row0_dev, const void *obs_posfeat_dev,
@@ -2670,8 +2621,10 @@ int fe_materialize(const FeParams *p, const FeSeries *s, const int64_t *obs_row0
     if (p->num_envs <= 0 || p->window <= 0 || p->num_assets != 1) return FE_EINVAL;
     DeviceGuard guard(p->device);
     if (guard.rc) return guard.rc;
-    return p->out_f64 ? gather_obs<double>(*p, *s, obs_row0_dev, obs_posfeat_dev, nullptr, p->num_envs, obs_dev, (cudaStream_t)stream)
-                      : gather_obs<float>(*p, *s, obs_row0_dev, obs_posfeat_dev, nullptr, p->num_envs, obs_dev, (cudaStream_t)stream);
+    return with_out_type(p->out_f64, [&](auto out_type) {
+        return gather_obs<decltype(out_type)>(*p, *s, obs_row0_dev, obs_posfeat_dev, nullptr, p->num_envs, obs_dev,
+                                              (cudaStream_t)stream);
+    });
 }
 
 int fe_gather_obs(const FeParams *p, const FeSeries *s, const int64_t *row0_dev, const void *posfeat_dev,
@@ -2682,8 +2635,9 @@ int fe_gather_obs(const FeParams *p, const FeSeries *s, const int64_t *row0_dev,
     if (count == 0) return 0;
     DeviceGuard guard(p->device);
     if (guard.rc) return guard.rc;
-    return p->out_f64 ? gather_obs<double>(*p, *s, row0_dev, posfeat_dev, index_dev, count, obs_dev, (cudaStream_t)stream)
-                      : gather_obs<float>(*p, *s, row0_dev, posfeat_dev, index_dev, count, obs_dev, (cudaStream_t)stream);
+    return with_out_type(p->out_f64, [&](auto out_type) {
+        return gather_obs<decltype(out_type)>(*p, *s, row0_dev, posfeat_dev, index_dev, count, obs_dev, (cudaStream_t)stream);
+    });
 }
 
 const char *fe_gather_obs_kernel_name(const FeParams *p, const FeSeries *s) {
@@ -2706,10 +2660,9 @@ static int step_host_impl(const FeParams *p, const FeSeries *s, const FeState *s
                           void *obs_dev, void *rewards_dev, int32_t *dones_dev, void *rewards_host, int32_t *dones_host,
                           uint32_t *dones_bits_host, FeStats *stats_dev, uint64_t step_counter, void *stream) {
     if (!p || !s || !st || !actions_host || !actions_dev || !rewards_host || (!dones_host == !dones_bits_host)) return FE_EINVAL;
-    int rc = check_common(p, s, st);
+    int rc = check_step(p, s, st, stats_dev);
     if (rc) return rc;
     if (!obs_dev || !rewards_dev || !dones_dev) return FE_EINVAL;
-    if (stats_dev && !p->evaluate && (!st->ep_return || !st->ep_len)) return FE_EINVAL;
     DeviceGuard guard(p->device);
     if (guard.rc) return guard.rc;
     cudaStream_t q = (cudaStream_t)stream;
@@ -2754,10 +2707,10 @@ static int step_host_impl(const FeParams *p, const FeSeries *s, const FeState *s
             // the actions are read from the host: actions_dev (>= 4 bytes per env) is free to stage the packed bits
             uint32_t *stage = reinterpret_cast<uint32_t *>(actions_dev);
             int packed_inline = 0;
-            rc = p->out_f64 ? launch<double, false>(*p, *s, *st, a, obs_dev, rewards_dev, dones_dev, stats_dev, step_counter, q,
-                                                    nullptr, ar.devicePointer, dmirror, bmirror, stage, &packed_inline)
-                            : launch<float, false>(*p, *s, *st, a, obs_dev, rewards_dev, dones_dev, stats_dev, step_counter, q,
-                                                   nullptr, ar.devicePointer, dmirror, bmirror, stage, &packed_inline);
+            rc = with_out_type(p->out_f64, [&](auto out_type) {
+                return launch<decltype(out_type), false>(*p, *s, *st, a, obs_dev, rewards_dev, dones_dev, stats_dev, step_counter,
+                                                         q, nullptr, ar.devicePointer, dmirror, bmirror, stage, &packed_inline);
+            });
             if (rc) return rc;
             if (dones_bits_host && packed_inline != 1) {
                 const int64_t nwords = (n + 31) / 32;
@@ -2805,10 +2758,10 @@ static int step_host_impl(const FeParams *p, const FeSeries *s, const FeState *s
         if (sc.ep_return) sc.ep_return += off;
         if (sc.ep_len) sc.ep_len += off;
         const size_t obs_off = (size_t)off * p->window * 5 * A * osz;
-        rc = p->out_f64 ? launch<double, false>(pc, *s, sc, actions_dev + off * A, (char *)obs_dev + obs_off, (char *)rewards_dev + off * osz,
-                                                dones_dev + off, stats_dev, step_counter, cs)
-                        : launch<float, false>(pc, *s, sc, actions_dev + off * A, (char *)obs_dev + obs_off, (char *)rewards_dev + off * osz,
-                                               dones_dev + off, stats_dev, step_counter, cs);
+        rc = with_out_type(p->out_f64, [&](auto out_type) {
+            return launch<decltype(out_type), false>(pc, *s, sc, actions_dev + off * A, (char *)obs_dev + obs_off,
+                                                     (char *)rewards_dev + off * osz, dones_dev + off, stats_dev, step_counter, cs);
+        });
         if (rc) return rc;
         e = cudaMemcpyAsync((char *)rewards_host + off * osz, (char *)rewards_dev + off * osz, (size_t)cnt * osz,
                             cudaMemcpyDeviceToHost, cs);

@@ -72,8 +72,7 @@ class LazyObs:
 
     @property
     def shape(self):
-        e = self.env
-        return (e.num_envs, e.num_intervals * e.num_obs) if e.flat_obs else (e.num_envs, e.num_intervals, e.num_obs)
+        return self.env._obs_shape
 
     def materialize(self) -> torch.Tensor:
         """The tensor step() would have returned for this observation."""
@@ -99,8 +98,7 @@ class CapturedRollout:
             raise ValueError("num_steps must be >= 1")
         self.env, self.policy, self.num_steps = env, policy, int(num_steps)
         dev, N = env._dev, env.num_envs
-        shape = (N, env.num_intervals * env.num_obs) if env.flat_obs else (N, env.num_intervals, env.num_obs)
-        self.obs = torch.empty(shape, dtype=env.obs_dtype, device=dev)
+        self.obs = torch.empty(env._obs_shape, dtype=env.obs_dtype, device=dev)
         self.rewards = torch.empty((num_steps, N), dtype=env.obs_dtype, device=dev)
         self.dones = torch.empty((num_steps, N), dtype=torch.int32, device=dev)
         self.actions = torch.empty((num_steps, N, env.num_acts), dtype=torch.float32, device=dev)
@@ -128,8 +126,7 @@ class CapturedRollout:
             self.actions[t].copy_(a.reshape(env.num_envs, env.num_acts))
             _lib.check(
                 env._L.fe_step_captured(env._pp, env._ps, env._pst, self.actions[t].data_ptr(), self.obs.data_ptr(),
-                                        self.rewards[t].data_ptr(), self.dones[t].data_ptr(),
-                                        env._stats.data_ptr() if env._stats is not None else None,
+                                        self.rewards[t].data_ptr(), self.dones[t].data_ptr(), env._stats_ptr,
                                         self._counter.data_ptr(), env._stream()),
                 "fe_step_captured",
             )
@@ -435,21 +432,25 @@ class TimeSeriesEnv(BaseObject):
     def _stream(self) -> int:
         return torch.cuda.current_stream(self._dev).cuda_stream
 
+    @property
+    def _obs_shape(self) -> Tuple[int, ...]:
+        """(N, W * num_obs) with flat_obs, else (N, W, num_obs)."""
+        W = self.num_intervals
+        return (self.num_envs, W * self.num_obs) if self.flat_obs else (self.num_envs, W, self.num_obs)
+
     def _new_obs(self, for_reset: bool = False) -> torch.Tensor:
         # a fresh tensor every call: the PPO buffer keeps references to past observations (buffer.py:44-56)
-        shape = ((self.num_envs, self.num_intervals * self.num_obs) if self.flat_obs
-                 else (self.num_envs, self.num_intervals, self.num_obs))
         ring = getattr(self, "_obs_ring", None)
         if ring is not None:  # a rollout buffer bound with Buffer.bind_env: write straight into its storage
-            return ring.next_obs_slot(shape, self.obs_dtype, for_reset)
-        return torch.empty(shape, dtype=self.obs_dtype, device=self._dev)
+            return ring.next_obs_slot(self._obs_shape, self.obs_dtype, for_reset)
+        return torch.empty(self._obs_shape, dtype=self.obs_dtype, device=self._dev)
 
     def reset(self) -> torch.Tensor:
         """:423-435 — materialises the current observation; touches no state (reference semantics)."""
         if self._handle_ring is not None:
             return self._observe_via_handle(None, for_reset=True)
         obs = self._new_obs(for_reset=True)
-        _lib.check(self._L.fe_observe(self._pp, self._ps, self._pst, obs.data_ptr(), self._stream()), "fe_observe")
+        self._observe_into(obs)
         return obs
 
     def _prepare_actions(self, actions: torch.Tensor) -> torch.Tensor:
@@ -480,8 +481,7 @@ class TimeSeriesEnv(BaseObject):
         self.step_count += 1
         _lib.check(
             self._L.fe_step(self._pp, self._ps, self._pst, actions.data_ptr(), obs.data_ptr(), rewards.data_ptr(),
-                            dones.data_ptr(), self._stats.data_ptr() if self._stats is not None else None,
-                            self.step_count, self._stream()),
+                            dones.data_ptr(), self._stats_ptr, self.step_count, self._stream()),
             "fe_step",
         )
         self._launch_metrics(rewards.data_ptr(), dones.data_ptr())
@@ -492,11 +492,24 @@ class TimeSeriesEnv(BaseObject):
         return LazyObs(self, torch.empty(self.num_envs, dtype=torch.int64, device=self._dev),
                        torch.empty(self.num_envs, dtype=self.obs_dtype, device=self._dev))
 
+    def _observe_lazy(self, row0: torch.Tensor, posfeat: torch.Tensor) -> None:
+        _lib.check(self._L.fe_observe_lazy(self._pp, self._ps, self._pst, row0.data_ptr(), posfeat.data_ptr(),
+                                           self._stream()), "fe_observe_lazy")
+
+    def _step_lazy(self, actions: torch.Tensor, row0: torch.Tensor, posfeat: torch.Tensor, rewards: torch.Tensor,
+                   dones: torch.Tensor) -> None:
+        self.step_count += 1
+        _lib.check(
+            self._L.fe_step_lazy(self._pp, self._ps, self._pst, actions.data_ptr(), row0.data_ptr(), posfeat.data_ptr(),
+                                 rewards.data_ptr(), dones.data_ptr(), self._stats_ptr, self.step_count, self._stream()),
+            "fe_step_lazy",
+        )
+        self._launch_metrics(rewards.data_ptr(), dones.data_ptr())
+
     def reset_lazy(self) -> LazyObs:
         """reset() returning a LazyObs handle instead of the tensor."""
         lo = self._new_lazy()
-        _lib.check(self._L.fe_observe_lazy(self._pp, self._ps, self._pst, lo.row0.data_ptr(), lo.posfeat.data_ptr(),
-                                           self._stream()), "fe_observe_lazy")
+        self._observe_lazy(lo.row0, lo.posfeat)
         return lo
 
     def step_lazy(self, actions: torch.Tensor) -> Tuple[LazyObs, torch.Tensor, torch.Tensor, dict]:
@@ -506,14 +519,7 @@ class TimeSeriesEnv(BaseObject):
         lo = self._new_lazy()
         rewards = torch.empty(self.num_envs, dtype=self.obs_dtype, device=self._dev)
         dones = torch.empty(self.num_envs, dtype=torch.int32, device=self._dev)
-        self.step_count += 1
-        _lib.check(
-            self._L.fe_step_lazy(self._pp, self._ps, self._pst, actions.data_ptr(), lo.row0.data_ptr(), lo.posfeat.data_ptr(),
-                                 rewards.data_ptr(), dones.data_ptr(), self._stats.data_ptr() if self._stats is not None else None,
-                                 self.step_count, self._stream()),
-            "fe_step_lazy",
-        )
-        self._launch_metrics(rewards.data_ptr(), dones.data_ptr())
+        self._step_lazy(actions, lo.row0, lo.posfeat, rewards, dones)
         info_dict = self.record_evaluation_metrics() if self.evaluate else {}
         return (lo, rewards, dones, info_dict)
 
@@ -546,20 +552,11 @@ class TimeSeriesEnv(BaseObject):
     def _observe_via_handle(self, step_args, for_reset: bool) -> torch.Tensor:
         row0, posfeat = self._handle_ring.next_handle_slot(self.num_envs, self.obs_dtype, for_reset)
         if step_args is None:
-            _lib.check(self._L.fe_observe_lazy(self._pp, self._ps, self._pst, row0.data_ptr(), posfeat.data_ptr(),
-                                               self._stream()), "fe_observe_lazy")
+            self._observe_lazy(row0, posfeat)
         else:
             actions, rewards, dones = step_args
-            self.step_count += 1
-            _lib.check(
-                self._L.fe_step_lazy(self._pp, self._ps, self._pst, actions.data_ptr(), row0.data_ptr(), posfeat.data_ptr(),
-                                     rewards.data_ptr(), dones.data_ptr(), self._stats_ptr, self.step_count, self._stream()),
-                "fe_step_lazy",
-            )
-            self._launch_metrics(rewards.data_ptr(), dones.data_ptr())
-        shape = ((self.num_envs, self.num_intervals * self.num_obs) if self.flat_obs
-                 else (self.num_envs, self.num_intervals, self.num_obs))
-        obs = torch.empty(shape, dtype=self.obs_dtype, device=self._dev)
+            self._step_lazy(actions, row0, posfeat, rewards, dones)
+        obs = torch.empty(self._obs_shape, dtype=self.obs_dtype, device=self._dev)
         self.gather_obs(row0, posfeat, None, obs)
         self._handle_ring.hand_out(obs)
         return obs
