@@ -10,8 +10,7 @@ import ctypes as C
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# FINENVS_B200_LIB: alternative build of the same library (kernel tuning experiments only)
-LIB_PATH = os.environ.get("FINENVS_B200_LIB") or os.path.join(_HERE, "libfinenvs_b200.so")
+LIB_PATH = os.path.join(_HERE, "libfinenvs_b200.so")
 
 RESET_KEEP, RESET_LAST, RESET_ALL = 0, 1, 2
 VARIANT_AUTO, VARIANT_TILE, VARIANT_DIRECT, VARIANT_PORTFOLIO, VARIANT_PIPE, VARIANT_SPLIT, VARIANT_GATHER = 0, 1, 2, 3, 4, 6, 8

@@ -3,7 +3,6 @@
 #define FE_COMMON_CUH
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdlib.h>
 
 #include <atomic>
 #include <type_traits>
@@ -104,14 +103,9 @@ __device__ __forceinline__ uint64_t l2_policy_evict_last() {
     return pol;
 }
 __device__ __forceinline__ void bulk_store_hint(void *dst, uint32_t src_smem, uint32_t bytes, uint64_t policy) {
-#ifdef FE_NO_L2_HINTS
-    (void)policy;
-    bulk_store(dst, src_smem, bytes);
-#else
     asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;" ::"l"(dst), "r"(src_smem),
                  "r"(bytes), "l"(policy)
                  : "memory");
-#endif
 }
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_read_all() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
@@ -192,17 +186,6 @@ template <auto Kern> int opt_in_smem(int device) {
 // output dtype, f(std::true_type{}) / f(std::false_type{}) for a flag), so the launch it makes is written once.
 template <class F> int with_out_type(bool f64, F &&f) { return f64 ? f(double{}) : f(float{}); }
 template <class F> int with_flag(bool b, F &&f) { return b ? f(std::true_type{}) : f(std::false_type{}); }
-
-// tuning overrides exist only in experiment builds (-DFE_EXPERIMENTS, tools/build_*_variants.sh); the shipped library
-// reads no environment variable
-#ifdef FE_EXPERIMENTS
-inline int env_override(const char *name) {
-    const char *v = getenv(name);
-    return v ? atoi(v) : 0;
-}
-#else
-constexpr int env_override(const char *) { return 0; }
-#endif
 
 } // namespace
 #endif // FE_COMMON_CUH

@@ -26,8 +26,6 @@
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdio.h>
-#include <stdlib.h>
 
 namespace {
 
@@ -251,15 +249,9 @@ fe_es_forward_kernel(const EsLayout lay, const float *__restrict__ theta, const 
 // The remaining (tiny) layers read theta from shared memory and eps from the stage.  Dense observations take the
 // same path (their rows are 5 consecutive floats), with the same FMA order, so lazy == dense bit for bit.
 // ------------------------------------------------------------------------------------------
-#ifndef FE_ES_FAST_WARPS
-#define FE_ES_FAST_WARPS 12
-#endif
-#ifndef FE_ES_FAST_STAGES
-#define FE_ES_FAST_STAGES 2
-#endif
-constexpr int kFastWarps = FE_ES_FAST_WARPS;
+constexpr int kFastWarps = 12;
 constexpr int kFastThreads = kFastWarps * 32;
-constexpr int kFastStages = FE_ES_FAST_STAGES;
+constexpr int kFastStages = 2;
 
 struct FastShape {
     int rows;        // R: window rows (in[0] == 5 * R)
@@ -550,20 +542,11 @@ fe_es_forward_fast_kernel(const EsLayout lay, const FastShape fs, const float *_
 //     warp's ring, issued kStStages-1 (pair, chunk) steps ahead, completing on the stage's mbarrier;
 //   * activations of the U pairs live in shared memory as (x+, x-) float2 per input.
 // ------------------------------------------------------------------------------------------
-#ifndef FE_ES_ST_WARPS
-#define FE_ES_ST_WARPS 12
-#endif
-#ifndef FE_ES_ST_STAGES
-#define FE_ES_ST_STAGES 2
-#endif
-#ifndef FE_ES_ST_MAXU
-#define FE_ES_ST_MAXU 4
-#endif
-constexpr int kStWarps = FE_ES_ST_WARPS;
+constexpr int kStWarps = 12;
 constexpr int kStThreads = kStWarps * 32;
-constexpr int kStStages = FE_ES_ST_STAGES;
+constexpr int kStStages = 2;
 constexpr int kStRows = 10;   // rows per lane: in + 1 <= 320
-constexpr int kStMaxU = FE_ES_ST_MAXU;
+constexpr int kStMaxU = 4;
 
 struct StreamShape {
     int U;            // pairs per warp per group
@@ -850,8 +833,7 @@ EsRoute route_forward(const EsLayout &lay, const bool lazy, const bool obs_align
     EsRoute rt{};
     const int64_t P = lay.off[lay.L];
     // ---- fast path: 5R -> <= 8 first layer (R <= 63), inputs 16-byte granular, ring fits in shared memory
-    const bool no_fast = env_override("FE_ES_NO_FAST") != 0; // A/B runs (experiment builds only)
-    if (!no_fast && lay.out[0] <= 8 && lay.in[0] % 5 == 0 && lay.in[0] / 5 <= 63 &&
+    if (lay.out[0] <= 8 && lay.in[0] % 5 == 0 && lay.in[0] / 5 <= 63 &&
         (lazy || (lay.in[0] % 4 == 0 && obs_aligned))) {
         FastShape &f = rt.fast;
         f.rows = lay.in[0] / 5;
@@ -870,8 +852,7 @@ EsRoute route_forward(const EsLayout &lay, const bool lazy, const bool obs_align
         }
     }
     // ---- streaming path: every layer has <= 319 inputs, eps chunks 16-byte granular (always), ring + activations fit
-    const bool no_stream = env_override("FE_ES_NO_STREAM") != 0;
-    bool stream_ok = !no_stream;
+    bool stream_ok = true;
     for (int l = 0; l < lay.L; ++l) stream_ok = stream_ok && lay.in[l] + 1 <= 32 * kStRows;
     if (stream_ok) {
         StreamShape &f = rt.stream;
@@ -1002,18 +983,15 @@ const char *fe_es_forward_kernel_name(const FeEsNet *net, int32_t lazy, int32_t 
     if (!make_layout(net, lay)) return "";
     const bool lz = lazy != 0;
     const EsRoute rt = route_forward(lay, lz, lz || obs_aligned != 0);
-    // one name per (input form, U) for whatever kStMaxU the build uses (FE_ES_ST_MAXU); filled once, thread-safely
-    static const struct StreamNames {
-        char s[2][kStMaxU][48];
-        StreamNames() {
-            for (int l = 0; l < 2; ++l)
-                for (int u = 0; u < kStMaxU; ++u)
-                    snprintf(s[l][u], sizeof s[l][u], "fe_es_forward_stream_kernel<%s> U=%d", l ? "lazy" : "dense", u + 1);
-        }
-    } stream_names;
+    static_assert(kStMaxU == 4, "one streaming-kernel name per pairs-per-warp count");
+    static const char *const stream_names[2][4] = {
+        {"fe_es_forward_stream_kernel<dense> U=1", "fe_es_forward_stream_kernel<dense> U=2", "fe_es_forward_stream_kernel<dense> U=3",
+         "fe_es_forward_stream_kernel<dense> U=4"},
+        {"fe_es_forward_stream_kernel<lazy> U=1", "fe_es_forward_stream_kernel<lazy> U=2", "fe_es_forward_stream_kernel<lazy> U=3",
+         "fe_es_forward_stream_kernel<lazy> U=4"}};
     switch (rt.kern) {
     case ES_FAST: return lz ? "fe_es_forward_fast_kernel<lazy>" : "fe_es_forward_fast_kernel<dense>";
-    case ES_STREAM: return stream_names.s[lz][rt.stream.U - 1];
+    case ES_STREAM: return stream_names[lz][rt.stream.U - 1];
     case ES_GENERIC:
         return rt.theta_smem ? (lz ? "fe_es_forward_kernel<lazy,theta_smem>" : "fe_es_forward_kernel<dense,theta_smem>")
                              : (lz ? "fe_es_forward_kernel<lazy,theta_global>" : "fe_es_forward_kernel<dense,theta_global>");

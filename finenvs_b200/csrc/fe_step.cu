@@ -24,7 +24,6 @@
 #include <cuda.h> // CUtensorMap (types only; cuTensorMapEncodeTiled is resolved at run time, libcuda is not linked)
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdlib.h>
 
 #include <mutex>
 #include <vector>
@@ -452,34 +451,20 @@ fe_tile_kernel(const FeParams p, const FeSeries s, const FeState st, const Const
 // per SM whatever the stage counts (7085 copies per SM per step => 0.32 ms floor), the same wall the
 // tile variant hits.  Register gathers have no such per-copy cost and halve the shared-memory traffic.
 // ------------------------------------------------------------------------------------------
-#ifndef FE_PIPE_BOOK
-#define FE_PIPE_BOOK 6
-#endif
-#ifndef FE_PIPE_MOVE
-#define FE_PIPE_MOVE 8
-#endif
-#ifndef FE_PIPE_SOUT
-#define FE_PIPE_SOUT 2
-#endif
-#ifndef FE_PIPE_SIN
-#define FE_PIPE_SIN 4   /* in-ring stages of the "stream" flavour (series larger than L2) */
-#endif
-#ifndef FE_PIPE_RPT
-#define FE_PIPE_RPT 8   /* f32 rows per mover thread per tile (f64: half) */
-#endif
-constexpr int kPipeBook = FE_PIPE_BOOK;
-constexpr int kPipeMove = FE_PIPE_MOVE;
+constexpr int kPipeBook = 6;
+constexpr int kPipeMove = 8;
 constexpr int kPipeThreads = (kPipeBook + kPipeMove) * 32;
 constexpr int kMovers = kPipeMove * 32;
-constexpr int kPipeQ = 8;                // descriptor ring depth
-constexpr int kPipeSOut = FE_PIPE_SOUT;  // out-tile stages
+constexpr int kPipeQ = 8;    // descriptor ring depth
+constexpr int kPipeSOut = 2; // out-tile stages
+constexpr int kPipeRows = 8; // f32 rows per mover thread per tile (f64: half)
 // Two flavours, chosen per launch from the size of the log-return table (pick_pipe_stages):
 //   kSIn == 0  "cached": the table is L2-resident, one tile of register prefetch covers the L2 latency and the
 //              rows never touch shared memory on the way in (measured c2: 0.28 ms vs 0.35 ms for kSIn == 3);
 //   kSIn  > 0  "stream": the table lives in HBM; rows arrive through an in-ring of kSIn stages filled with
 //              16-byte cp.async (LDGSTS), ~kSIn x 30 KB in flight per SM (measured c4: 0.376 ms vs 0.43 ms).
-constexpr int kPipeSInStream = FE_PIPE_SIN;
-template <typename OutT> struct PipeRows { static constexpr int value = sizeof(OutT) == 4 ? FE_PIPE_RPT : (FE_PIPE_RPT + 1) / 2; }; // rows / thread / tile
+constexpr int kPipeSInStream = 4;
+template <typename OutT> struct PipeRows { static constexpr int value = sizeof(OutT) == 4 ? kPipeRows : (kPipeRows + 1) / 2; }; // rows / thread / tile
 
 // smem: [mbarriers desc_full[Q], desc_free[Q], in_full[S_IN]] (256 B) [descriptors Q x TE x (8 + 8) B]
 //       [in ring S_IN x TE*W*4 OutT] [out ring S_OUT x TE*W*5 OutT]
@@ -712,20 +697,10 @@ fe_pipe_kernel(const FeParams p, const FeSeries s, const FeState st, const Const
 //                               issues the bulk store, releases the descriptor, waits until the store has read the slot
 //                               and issues the gather of unit i + S into it.
 // ------------------------------------------------------------------------------------------
-#ifndef FE_GATHER_BOOK
-#define FE_GATHER_BOOK 6 /* measured c2: 6 -> 0.2525 ms, 8 -> 0.2655 ms (profiles/r02_gather_allwait.txt) */
-#endif
-#ifndef FE_GATHER_MOVE
-#define FE_GATHER_MOVE 12
-#endif
-#ifndef FE_GATHER_STAGES
-#define FE_GATHER_STAGES 3 /* slots per mover when they fit (else 2) */
-#endif
-#ifndef FE_GATHER_FLUSH_SPINS
-#define FE_GATHER_FLUSH_SPINS 2000 /* x 100 ns: how long a block waits for the grid's bookkeeping before it leaves the packed dones to the last block out */
-#endif
-constexpr int kGaBook = FE_GATHER_BOOK;
-constexpr int kGaMove = FE_GATHER_MOVE;
+constexpr int kGaBook = 6;    // measured c2: 6 -> 0.2525 ms, 8 -> 0.2655 ms (profiles/r02_gather_allwait.txt)
+constexpr int kGaMove = 12;
+constexpr int kGaStages = 3;  // slots per mover when they fit (else 2)
+constexpr int kGaFlushSpins = 2000; // x 100 ns: how long a block waits for the grid's bookkeeping before it leaves the packed dones to the last block out
 constexpr int kGaThreads = (kGaBook + kGaMove) * 32;
 constexpr int kGaQ = 32;          // descriptor ring depth in tiles (movers keep a descriptor until its unit is stored)
 constexpr int kGaMaxStages = 4;
@@ -776,22 +751,6 @@ __device__ __forceinline__ void tma_gather4(uint32_t dst_smem, const CUtensorMap
         : "memory");
 }
 
-#ifdef FE_GATHER_CLOCKS
-// experiment builds: cycles spent per phase by block 0's mover 0 / bookkeeper 0 (tools/gather_clocks.py)
-__device__ unsigned long long fe_gather_clk[16];
-__device__ unsigned long long fe_gather_block_ns[3 * 160]; // per block: start, all movers done, smid (globaltimer ns)
-__device__ __forceinline__ unsigned long long ga_globaltimer() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
-#define GA_CLK(var) const long long var = clock64()
-#define GA_ACC(slot, a, b) acc[slot] += (b) - (a)
-#else
-#define GA_CLK(var)
-#define GA_ACC(slot, a, b)
-#endif
-
 template <typename OutT, bool kObserve, int kParts>
 __global__ void __launch_bounds__(kGaThreads, 1)
 fe_gather_kernel(const __grid_constant__ CUtensorMap tmap, const FeParams p, const FeSeries s, const FeState st, const Consts k,
@@ -819,15 +778,6 @@ fe_gather_kernel(const __grid_constant__ CUtensorMap tmap, const FeParams p, con
     unsigned char *ring = smem + kGaBarBytes + gather_desc_bytes<OutT>();
     const uint32_t pitch = ga_slot_pitch(W, kF64);
 
-#ifdef FE_GATHER_CLOCKS
-    if (tid == 0 && blockIdx.x < 160) {
-        unsigned smid;
-        asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-        fe_gather_block_ns[3 * blockIdx.x] = ga_globaltimer();
-        fe_gather_block_ns[3 * blockIdx.x + 2] = smid;
-        fe_gather_block_ns[3 * blockIdx.x + 1] = 0;
-    }
-#endif
     if (tid == 0) {
         for (int q = 0; q < kGaQ; ++q) { mbar_init(desc_full(q), 1); mbar_init(desc_free(q), kTileUnits); }
         for (int m = 0; m < kGaMove; ++m)
@@ -845,10 +795,6 @@ fe_gather_kernel(const __grid_constant__ CUtensorMap tmap, const FeParams p, con
         // grid), taken together under a block-local lock so that sequence order = tile order: once a sequence slot says
         // "no more tiles", every later one does.
         const int shift = ga_phase_shift(kF64);
-#ifdef FE_GATHER_CLOCKS
-        long long acc[16] = {0};
-        int ntl = 0;
-#endif
         // With the actions in mapped host memory (fe_step_host: k.rewards_mirror is set) the action load is a PCIe read of
         // ~2 us.  There a claim is taken one tile AHEAD of the tile being computed and the first-hop loads of the claimed
         // tile (action and per-env state) are issued at once, in flight while the current tile is computed, so that the
@@ -885,11 +831,8 @@ fe_gather_kernel(const __grid_constant__ CUtensorMap tmap, const FeParams p, con
                 take_claim(n_next, t_next);
                 first_hop(t_next, ld_next);
             }
-            GA_CLK(c0);
             if (lane == 0) mbar_wait(desc_free(q), ((n / kGaQ) & 1) ^ 1); // first lap passes immediately
             __syncwarp();
-            GA_CLK(c1);
-            GA_ACC(8, c0, c1);
             if (t >= ntiles_all) { // nothing left: tell the movers and stop
                 if (lane == 0) { d_tile[q] = -1; mbar_arrive(desc_full(q)); }
                 break;
@@ -913,11 +856,6 @@ fe_gather_kernel(const __grid_constant__ CUtensorMap tmap, const FeParams p, con
             if (!kObserve) accumulate_stats(stats, r, active);
             __syncwarp();
             if (lane == 0) mbar_arrive(desc_full(q)); // release: descriptor visible to the movers
-            GA_CLK(c2);
-            GA_ACC(9, c1, c2);
-#ifdef FE_GATHER_CLOCKS
-            ++ntl;
-#endif
             if (ahead) { n = n_next; t = t_next; ld = ld_next; }
             else { take_claim(n, t); first_hop(t, ld); }
         }
@@ -940,7 +878,7 @@ fe_gather_kernel(const __grid_constant__ CUtensorMap tmap, const FeParams p, con
                     const unsigned want = gridDim.x * (unsigned)kGaBook;
                     int spins = 0;
                     while (ld_acquire_gpu(&sched[2]) < want) {
-                        if (++spins > FE_GATHER_FLUSH_SPINS) { ok = 0; break; }
+                        if (++spins > kGaFlushSpins) { ok = 0; break; }
                         __nanosleep(100);
                     }
                     if (!ok) atomicOr(&sched[3], 1u);
@@ -960,15 +898,8 @@ fe_gather_kernel(const __grid_constant__ CUtensorMap tmap, const FeParams p, con
                 }
             }
         }
-#ifdef FE_GATHER_CLOCKS
-        if (blockIdx.x == 0 && tid == 0) { fe_gather_clk[8] = acc[8]; fe_gather_clk[9] = acc[9]; fe_gather_clk[10] = ntl; }
-#endif
     } else {
         // ------------------------------------------------------------------ movers
-#ifdef FE_GATHER_CLOCKS
-        long long acc[16] = {0};
-        const long long mover_t0 = clock64();
-#endif
         const int m = warp - kGaBook;
         const uint32_t row_b = (uint32_t)ga_row_bytes(kF64) * W, unit_b = kUnitEnvs * row_b; // row_b: one window
         const int part_rows = (int)(row_b / 2) / kGaPitch; // two parts: tensor rows from a window's first half to its second
@@ -987,10 +918,7 @@ fe_gather_kernel(const __grid_constant__ CUtensorMap tmap, const FeParams p, con
         bool open = true;          // lane 0: more units may follow (no "no more tiles" slot seen yet)
         auto issue = [&]() {       // lane 0: gather of the next unit into slot iss_si
             const int n = iss_u >> kUnitShift, g = iss_u & (kTileUnits - 1), q = n & (kGaQ - 1);
-            GA_CLK(c0);
             mbar_wait(desc_full(q), (n / kGaQ) & 1);
-            GA_CLK(c1);
-            GA_ACC(4, c0, c1);
             if (d_tile[q] < 0) { open = false; return; }
             int4 rows4;
             if constexpr (kParts == 1) {
@@ -999,22 +927,12 @@ fe_gather_kernel(const __grid_constant__ CUtensorMap tmap, const FeParams p, con
                 const int2 r2 = *reinterpret_cast<const int2 *>(d_row + q * 32 + 2 * g);
                 rows4 = make_int4(r2.x, r2.x + part_rows, r2.y, r2.y + part_rows);
             }
-#ifdef FE_GATHER_NOLOAD
-            if (rows4.x == -12345)
-#endif
-            {
-                mbar_arrive_expect_tx(slot_full(m, iss_si), unit_b);
-                tma_gather4(smem_u32(slots + (size_t)iss_si * pitch), &tmap, rows4.x, rows4.y, rows4.z, rows4.w, slot_full(m, iss_si),
-                            keep);
-            }
-#ifdef FE_GATHER_NOLOAD
-            mbar_arrive(slot_full(m, iss_si));
-#endif
+            mbar_arrive_expect_tx(slot_full(m, iss_si), unit_b);
+            tma_gather4(smem_u32(slots + (size_t)iss_si * pitch), &tmap, rows4.x, rows4.y, rows4.z, rows4.w, slot_full(m, iss_si),
+                        keep);
             ++issued;
             iss_u += kGaMove;
             iss_si = iss_si + 1 == S ? 0 : iss_si + 1;
-            GA_CLK(c2);
-            GA_ACC(5, c1, c2);
         };
         if (lane == 0)
             for (int i = 0; i < S && open; ++i) issue();
@@ -1027,17 +945,11 @@ fe_gather_kernel(const __grid_constant__ CUtensorMap tmap, const FeParams p, con
         int n_iss = __shfl_sync(0xFFFFFFFFu, issued, 0);
         for (int i = 0; i < n_iss; ++i) {
             const int n = u >> kUnitShift, g = u & (kTileUnits - 1), q = n & (kGaQ - 1);
-            GA_CLK(c0);
             if (lane == 0) mbar_wait(slot_full(m, si), (slot_phase >> si) & 1u); // the unit's windows have landed
             __syncwarp();
-            GA_CLK(c1);
-            GA_ACC(0, c0, c1);
             unsigned char *slot = slots + (size_t)si * pitch;
             const OutT *pf = d_pf + q * 32 + kUnitEnvs * g;
             OutT *col = reinterpret_cast<OutT *>(slot) + 5 * lane + 4; // position-feature slot of row `lane` of env 0
-#ifdef FE_GATHER_NOPF
-            if (pf[0] == (OutT)12345.678)
-#endif
 #pragma unroll
             for (int e = 0; e < kUnitEnvs; ++e) {
                 const OutT v = pf[e];
@@ -1045,34 +957,19 @@ fe_gather_kernel(const __grid_constant__ CUtensorMap tmap, const FeParams p, con
                 for (int kk = 0; kk < kRounds; ++kk)
                     if (round_mask & (1u << kk)) col[e * env_stride + 160 * kk] = v;
             }
-            GA_CLK(c1b);
-            GA_ACC(1, c1, c1b);
-#ifndef FE_GATHER_NOFENCE
             fence_proxy_async_smem(); // generic-proxy writes -> visible to the bulk store
-#endif
             __syncwarp();
-            GA_CLK(c2);
-            GA_ACC(11, c1b, c2);
             if (lane == 0) {
                 const int64_t env0 = (int64_t)d_tile[q] * 32 + kUnitEnvs * g;
                 const int64_t left = p.num_envs - env0;
                 const int nv = left >= kUnitEnvs ? kUnitEnvs : (left > 0 ? (int)left : 0); // fewer only in the ragged last tile
-#ifdef FE_GATHER_NOSTORE
-                if (nv > 4)
-#else
-                if (nv > 0)
-#endif
-                {
+                if (nv > 0) {
                     bulk_store_hint(obs + (size_t)env0 * W * 5, smem_u32(slot), (uint32_t)nv * row_b, stream_out);
                     bulk_commit();
                 }
                 mbar_arrive(desc_free(q)); // this unit's descriptor entries are consumed
-                GA_CLK(c3);
-                GA_ACC(2, c2, c3);
                 if (open) {
                     bulk_wait_read_all(); // the store has read the slot: refill it
-                    GA_CLK(c4);
-                    GA_ACC(3, c3, c4);
                     issue();
                 }
             }
@@ -1083,10 +980,6 @@ fe_gather_kernel(const __grid_constant__ CUtensorMap tmap, const FeParams p, con
             si = si + 1 == S ? 0 : si + 1;
         }
         if (lane == 0) bulk_wait_read_all();
-#ifdef FE_GATHER_CLOCKS
-        if (lane == 0 && blockIdx.x < 160) atomicMax(&fe_gather_block_ns[3 * blockIdx.x + 1], ga_globaltimer());
-        if (blockIdx.x == 0 && m == 0 && lane == 0) { for (int c = 0; c < 6; ++c) fe_gather_clk[c] = acc[c]; fe_gather_clk[6] = issued; fe_gather_clk[11] = acc[11]; fe_gather_clk[12] = 0; fe_gather_clk[13] = clock64() - mover_t0; }
-#endif
     }
     // the last block out rewinds the counters for the next launch (every block's claims, and its wait on sched[2], precede
     // its arrival here)
@@ -1827,7 +1720,7 @@ int check_step(const FeParams *p, const FeSeries *s, const FeState *st, const Fe
     return stats && !p->evaluate && (!st->ep_return || !st->ep_len) ? FE_EINVAL : 0;
 }
 
-// Tile shape.  Measured on B200 (tools/sweep_tile.sh, 1 Mi envs, W=60): the step is latency-bound per
+// Tile shape.  Measured on B200 (profiles/r01_sweep_tile_shape.txt, 1 Mi envs, W=60): the step is latency-bound per
 // block (state loads -> table lookup -> window copy -> interleave -> store), so MANY SMALL blocks in
 // flight beat few large ones: 4 envs x 32 threads (23 blocks/SM) runs 0.35 ms where 32 envs x 128
 // threads (3 blocks/SM) runs 0.46 ms.  E is kept a multiple of 4 so that every full tile's byte count
@@ -1867,7 +1760,7 @@ int pick_pipe_stages(const FeParams &p, bool f64) {
 // slots per mover of the gather variant (3 when they fit, else 2); 0 = this window has no gather variant
 int pick_gather_stages(int W, bool f64) {
     if (!ga_window_ok(W, f64)) return 0;
-    for (int S = FE_GATHER_STAGES; S >= 2; --S)
+    for (int S = kGaStages; S >= 2; --S)
         if ((f64 ? gather_smem_bytes<double>(W, S) : gather_smem_bytes<float>(W, S)) <= (size_t)kSmemMax) return S;
     return 0;
 }
@@ -1901,15 +1794,13 @@ StepChoice choose_kernel(const FeParams &p, bool gather_ready, bool f64, int sms
             c.kern = !gather_ready ? K_ERR_TABLE : c.S == 0 ? K_ERR_SMEM : K_GATHER;
             return c;
         }
-        const bool no_gather = env_override("FE_NO_GATHER") != 0; // sweeps: "auto" never picks gather
-        if (!no_gather && gather_ready && c.S > 0 && worth_persistent && p.window >= 24 && gather_table_resident(p, f64)) {
+        if (gather_ready && c.S > 0 && worth_persistent && p.window >= 24 && gather_table_resident(p, f64)) {
             c.kern = K_GATHER;
             return c;
         }
     }
     if (p.variant == FE_VARIANT_PIPE || p.variant == FE_VARIANT_AUTO) {
-        const int ov_sin = env_override("FE_PIPE_FLAVOUR"); // sweeps: 1 = cached, 2 = stream
-        c.sin = ov_sin == 1 ? 0 : ov_sin == 2 ? kPipeSInStream : pick_pipe_stages(p, f64);
+        c.sin = pick_pipe_stages(p, f64);
         c.te = pick_pipe_envs(p.window, f64, c.sin);
         if (c.te == 0 && p.variant == FE_VARIANT_PIPE) { c.kern = K_ERR_SMEM; return c; }
         if (c.te > 0 && (p.variant == FE_VARIANT_PIPE || (worth_persistent && p.window >= 24))) { c.kern = K_PIPE; return c; }
@@ -1919,14 +1810,7 @@ StepChoice choose_kernel(const FeParams &p, bool gather_ready, bool f64, int sms
     }
     c.te = p.variant == FE_VARIANT_DIRECT ? 0 : pick_tile_envs(p.window, f64, &c.threads);
     if (p.variant == FE_VARIANT_TILE && c.te == 0) { c.kern = K_ERR_SMEM; return c; }
-    if (c.te > 0) {
-        const int ov_e = env_override("FE_TILE_ENVS"), ov_t = env_override("FE_TILE_THREADS");
-        const size_t sz = f64 ? 8 : 4;
-        if (ov_e >= 4 && kSmemHeader + 16 + (size_t)(ov_e & ~3) * (p.window * 9 * sz + sz) <= (size_t)kSmemMax) c.te = ov_e & ~3;
-        if (ov_t >= 32 && ov_t <= kThreads) c.threads = ov_t & ~31;
-        if (c.te > c.threads) c.te = c.threads;
-        c.kern = K_TILE;
-    }
+    if (c.te > 0) c.kern = K_TILE;
     return c;
 }
 
@@ -1999,13 +1883,12 @@ int launch(const FeParams &p, const FeSeries &s, const FeState &st, const float 
     // the persistent kernels with 32-env tiles pack the dones themselves (one ballot per tile); otherwise the caller runs
     // fe_pack_dones_kernel after the step
     const bool inline_pack = dones_bits_mirror && dones_bits_stage && (c.kern == K_GATHER || (c.kern == K_PIPE && c.te == 32));
-    const int pack_mode = env_override("FE_PACK_MODE"); // sweeps: 1 = words straight to the host, 2 = flush by a second kernel
     if (inline_pack) {
-        k.dones_bits_out = pack_mode == 1 ? dones_bits_mirror : dones_bits_stage;
-        if (c.kern == K_GATHER && pack_mode == 0) k.dones_bits_host = dones_bits_mirror; // sent by the kernel itself
+        k.dones_bits_out = dones_bits_stage;
+        if (c.kern == K_GATHER) k.dones_bits_host = dones_bits_mirror; // sent by the kernel itself
     }
     // 0: the caller packs dones_dev after the step; 1: packed and already sent to the host; 2: packed into the staging buffer
-    if (packed_inline) *packed_inline = !inline_pack ? 0 : (pack_mode == 1 || (c.kern == K_GATHER && pack_mode == 0)) ? 1 : 2;
+    if (packed_inline) *packed_inline = !inline_pack ? 0 : c.kern == K_GATHER ? 1 : 2;
     switch (c.kern) {
     case K_ERR_SMEM: return FE_ESMEM;
     case K_ERR_TABLE: return FE_EINVAL;
@@ -2013,8 +1896,6 @@ int launch(const FeParams &p, const FeSeries &s, const FeState &st, const float 
         if ((uintptr_t)obs & 15) return FE_EALIGN;
         const int P = p.window * p.num_assets;
         int CH = 512; // pairs per chunk (8 KB in + 10 KB out, x2 stages); C3: 128 -> 1.492 ms, 256 -> 1.480, 512 -> 1.472, 1024 -> 1.471
-        const int ov_ch = env_override("FE_PORT_CHUNK");
-        if (ov_ch >= 4) CH = ov_ch & ~3;
         if (CH > ((P + 3) & ~3)) CH = (P + 3) & ~3;
         const size_t smem = port_smem_bytes<OutT>(CH);
         if (smem > (size_t)kSmemMax) return FE_ESMEM;
@@ -2029,8 +1910,7 @@ int launch(const FeParams &p, const FeSeries &s, const FeState &st, const float 
         if ((uintptr_t)obs & 7) return FE_EALIGN;
         fe_book_kernel<OutT, kObserve><<<(unsigned)((p.num_envs + kThreads - 1) / kThreads), kThreads, 0, stream>>>(
             p, s, st, k, actions, (OutT *)obs, (OutT *)rewards, dones, stats, step, step_dev);
-        const int ov_b = env_override("FE_STREAM_BLOCKS_PER_SM");
-        int64_t blocks = (int64_t)sms * (ov_b > 0 ? ov_b : 6); // 48 warps per SM
+        int64_t blocks = (int64_t)sms * 6; // 48 warps per SM
         const int64_t need = (p.num_envs * 32 + kStreamThreads - 1) / kStreamThreads;
         if (blocks > need) blocks = need;
         fe_stream_kernel<OutT><<<(unsigned)blocks, kStreamThreads, 0, stream>>>(p.num_envs, p.window, (const OutT *)s.logret, (OutT *)obs);
@@ -2682,52 +2562,49 @@ static int step_host_impl(const FeParams *p, const FeSeries *s, const FeState *s
     // serialises launches (ncu, CUDA_LAUNCH_BLOCKING=1) — dropped.)
     int sms = 0;
     if ((rc = device_sm_count(p->device, &sms))) return rc;
-    if (!env_override("FE_HOST_NO_ZEROCOPY")) {
-        cudaPointerAttributes aa, ar, ad;
-        const bool ok = cudaPointerGetAttributes(&aa, actions_host) == cudaSuccess && aa.type == cudaMemoryTypeHost &&
-                        aa.devicePointer && cudaPointerGetAttributes(&ar, rewards_host) == cudaSuccess &&
-                        ar.type == cudaMemoryTypeHost && ar.devicePointer &&
-                        cudaPointerGetAttributes(&ad, dones_any) == cudaSuccess && ad.type == cudaMemoryTypeHost &&
-                        ad.devicePointer;
-        (void)cudaGetLastError(); // an unregistered pointer leaves a sticky-free error on old drivers
-        // Only for the persistent (and the portfolio) kernels: their bookkeeper warps run tiles ahead, which hides the
-        // PCIe read latency, and they write rewards / dones 32 envs (128 bytes) per store.  A tile / direct block would
-        // sit on its shared memory while it waits for its actions and write 16-byte PCIe packets (measured W = 60,
-        // 1 Mi envs: 1.04 ms zero-copy, 0.77 ms with a copy-engine upload + zero-copy writes, vs 0.36 ms
-        // device-resident): those take the chunked copy pipeline below.
-        // Small populations are the exception: there the whole step is a few microseconds and the three copies, two events
-        // and their stream hops of the chunked path cost more than the PCIe round trips (1024 envs: C call 25.6 -> 20.0 us, bit-packed
-        // 35.0 -> 24.8 us; profiles/r02_e2e_probe_small_populations.txt), so tile / direct launches of <= 32 Ki envs go zero-copy too.
-        const StepKernel kk = choose_kernel(*p, s->obs_table && st->sched, p->out_f64 != 0, sms).kern;
-        const bool small = n <= 32768;
-        if (ok && ((kk != K_TILE && kk != K_DIRECT) || small)) {
-            const float *a = (const float *)aa.devicePointer;
-            int32_t *dmirror = dones_host ? (int32_t *)ad.devicePointer : nullptr;
-            uint32_t *bmirror = dones_bits_host ? (uint32_t *)ad.devicePointer : nullptr;
-            // the actions are read from the host: actions_dev (>= 4 bytes per env) is free to stage the packed bits
-            uint32_t *stage = reinterpret_cast<uint32_t *>(actions_dev);
-            int packed_inline = 0;
-            rc = with_out_type(p->out_f64, [&](auto out_type) {
-                return launch<decltype(out_type), false>(*p, *s, *st, a, obs_dev, rewards_dev, dones_dev, stats_dev, step_counter,
-                                                         q, nullptr, ar.devicePointer, dmirror, bmirror, stage, &packed_inline);
-            });
-            if (rc) return rc;
-            if (dones_bits_host && packed_inline != 1) {
-                const int64_t nwords = (n + 31) / 32;
-                if (packed_inline == 0 && small) { // a handful of words: straight to the host, one launch less
-                    fe_pack_dones_kernel<<<(unsigned)((n + 255) / 256), 256, 0, q>>>(dones_dev, n, (uint32_t *)ad.devicePointer);
-                } else {
-                    if (packed_inline == 0)
-                        fe_pack_dones_kernel<<<(unsigned)((n + 255) / 256), 256, 0, q>>>(dones_dev, n, stage);
-                    fe_flush_bits_kernel<<<(unsigned)((nwords + 255) / 256), 256, 0, q>>>(stage, nwords, (uint32_t *)ad.devicePointer);
-                }
-                if ((rc = (int)cudaGetLastError())) return rc;
+    cudaPointerAttributes aa, ar, ad;
+    const bool ok = cudaPointerGetAttributes(&aa, actions_host) == cudaSuccess && aa.type == cudaMemoryTypeHost &&
+                    aa.devicePointer && cudaPointerGetAttributes(&ar, rewards_host) == cudaSuccess &&
+                    ar.type == cudaMemoryTypeHost && ar.devicePointer &&
+                    cudaPointerGetAttributes(&ad, dones_any) == cudaSuccess && ad.type == cudaMemoryTypeHost &&
+                    ad.devicePointer;
+    (void)cudaGetLastError(); // an unregistered pointer leaves a sticky-free error on old drivers
+    // Only for the persistent (and the portfolio) kernels: their bookkeeper warps run tiles ahead, which hides the
+    // PCIe read latency, and they write rewards / dones 32 envs (128 bytes) per store.  A tile / direct block would
+    // sit on its shared memory while it waits for its actions and write 16-byte PCIe packets (measured W = 60,
+    // 1 Mi envs: 1.04 ms zero-copy, 0.77 ms with a copy-engine upload + zero-copy writes, vs 0.36 ms
+    // device-resident): those take the chunked copy pipeline below.
+    // Small populations are the exception: there the whole step is a few microseconds and the three copies, two events
+    // and their stream hops of the chunked path cost more than the PCIe round trips (1024 envs: C call 25.6 -> 20.0 us, bit-packed
+    // 35.0 -> 24.8 us; profiles/r02_e2e_probe_small_populations.txt), so tile / direct launches of <= 32 Ki envs go zero-copy too.
+    const StepKernel kk = choose_kernel(*p, s->obs_table && st->sched, p->out_f64 != 0, sms).kern;
+    const bool small = n <= 32768;
+    if (ok && ((kk != K_TILE && kk != K_DIRECT) || small)) {
+        const float *a = (const float *)aa.devicePointer;
+        int32_t *dmirror = dones_host ? (int32_t *)ad.devicePointer : nullptr;
+        uint32_t *bmirror = dones_bits_host ? (uint32_t *)ad.devicePointer : nullptr;
+        // the actions are read from the host: actions_dev (>= 4 bytes per env) is free to stage the packed bits
+        uint32_t *stage = reinterpret_cast<uint32_t *>(actions_dev);
+        int packed_inline = 0;
+        rc = with_out_type(p->out_f64, [&](auto out_type) {
+            return launch<decltype(out_type), false>(*p, *s, *st, a, obs_dev, rewards_dev, dones_dev, stats_dev, step_counter,
+                                                     q, nullptr, ar.devicePointer, dmirror, bmirror, stage, &packed_inline);
+        });
+        if (rc) return rc;
+        if (dones_bits_host && packed_inline != 1) {
+            const int64_t nwords = (n + 31) / 32;
+            if (packed_inline == 0 && small) { // a handful of words: straight to the host, one launch less
+                fe_pack_dones_kernel<<<(unsigned)((n + 255) / 256), 256, 0, q>>>(dones_dev, n, (uint32_t *)ad.devicePointer);
+            } else {
+                if (packed_inline == 0)
+                    fe_pack_dones_kernel<<<(unsigned)((n + 255) / 256), 256, 0, q>>>(dones_dev, n, stage);
+                fe_flush_bits_kernel<<<(unsigned)((nwords + 255) / 256), 256, 0, q>>>(stage, nwords, (uint32_t *)ad.devicePointer);
             }
-            return (int)cudaStreamSynchronize(q);
+            if ((rc = (int)cudaGetLastError())) return rc;
         }
+        return (int)cudaStreamSynchronize(q);
     }
-    const int ov_chunks = env_override("FE_HOST_CHUNKS");
-    int chunks = ov_chunks > 0 ? ov_chunks : 4;
+    int chunks = 4;
     int64_t per = ((n + chunks - 1) / chunks + 1023) & ~(int64_t)1023;
     if (per < 16384) per = 16384; // below this a chunk's kernel is shorter than the launch + copy set-up it would hide
     chunks = (int)((n + per - 1) / per);
@@ -2813,11 +2690,6 @@ int fe_reset_all(const FeParams *p, const FeSeries *s, const FeState *st, uint64
                                                                                                  redraw);
     return (int)cudaGetLastError();
 }
-
-#ifdef FE_GATHER_CLOCKS
-int fe_debug_gather_clocks(unsigned long long out[16]) { return (int)cudaMemcpyFromSymbol(out, fe_gather_clk, 128); }
-int fe_debug_gather_blocks(unsigned long long out[480]) { return (int)cudaMemcpyFromSymbol(out, fe_gather_block_ns, 480 * 8); }
-#endif
 
 void fe_philox(uint64_t seed, uint64_t env_id, uint64_t step, uint32_t kind, uint32_t out[4]) {
     philox4x32_10(seed, env_id, step, kind, out);

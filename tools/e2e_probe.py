@@ -3,7 +3,7 @@
 One process, one GPU: device-resident step, then int32-dones and bit-packed host steps alternating (so that order effects
 show), each as wall time per step over blocks of 20 steps, with the share spent inside the C call itself.  Also checks
 that the packed bits equal the int32 dones of the same step.
-usage: [FE_PACK_MODE=1|2 FINENVS_B200_LIB=...] python tools/e2e_probe.py [--envs N] [--rounds R]
+usage: python tools/e2e_probe.py [--envs N] [--rounds R]
 """
 import argparse
 import os
@@ -43,7 +43,7 @@ def main():
     obs = torch.empty((N, W, 5), dtype=torch.float32, device="cuda:0")
     rew = torch.empty(N, dtype=torch.float32, device="cuda:0")
     dn = torch.empty(N, dtype=torch.int32, device="cuda:0")
-    print(f"kernel {env.kernel_name()}  lib {os.environ.get('FINENVS_B200_LIB', 'shipped')}  FE_PACK_MODE={os.environ.get('FE_PACK_MODE')}")
+    print(f"kernel {env.kernel_name()}")
 
     def dev_block():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
