@@ -127,6 +127,10 @@ _PROTOTYPES = {
     "fe_backtest_targets": (C.c_int, [C.POINTER(FeParams), C.POINTER(FeSeries), C.POINTER(FeState),
                                       C.POINTER(FeMetricsState), C.c_int64, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p,
                                       C.c_void_p, C.c_uint64, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
+    "fe_backtest_portfolio": (C.c_int, [C.POINTER(FeParams), C.POINTER(FeSeries), C.POINTER(FeState),
+                                        C.POINTER(FeMetricsState), C.c_int64, C.c_void_p, C.c_void_p, C.c_int32,
+                                        C.c_void_p, C.c_int32, C.c_void_p, C.c_uint64, C.c_int32, C.c_void_p, C.c_void_p,
+                                        C.c_int32, C.c_void_p]),
     "fe_es_params_padded": (C.c_int64, [C.POINTER(FeEsNet)]),
     "fe_es_packed_index": (C.c_int64, [C.POINTER(FeEsNet), C.c_int32, C.c_int32, C.c_int32]),
     "fe_es_perturb": (C.c_int, [C.POINTER(FeEsNet), C.c_uint64, C.c_uint64, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p]),

@@ -1349,16 +1349,17 @@ __device__ __forceinline__ float warp_sum32(float v) {
 // chain, so the loads run ahead of it) and the serial part is one DADD + compare per asset.  (A first version walked
 // every phase with __shfl_sync inside the loops: ncu showed ~10 k instructions per env in this warp,
 // WARPSYNC.COLLECTIVE wrappers around every shuffle.)
-template <typename OutT>
-__device__ __forceinline__ void portfolio_step(const FeParams &p, const FeSeries &s, const FeState &st, const Consts &k,
-                                               const int64_t i, const int32_t seg_in, const int32_t ptr_in,
-                                               const int64_t row0, const float *__restrict__ actions,
-                                               OutT *__restrict__ rewards, int32_t *__restrict__ dones, FeStats *stats,
-                                               const uint64_t step, OutT *pf_smem, double *scratch) {
+//
+// The arithmetic is written once, in portfolio_step_core; whatever it reads or writes besides the bar and the shared
+// scratch goes through `io`: PortfolioGlobalIO (the state arrays, outputs and FeStats atomics, for
+// fe_portfolio_book_kernel) or PortfolioBacktestIO (registers across the K steps of fe_backtest_portfolio_kernel).
+template <typename IO>
+__device__ __forceinline__ void portfolio_step_core(const FeParams &p, const FeSeries &s, const Consts &k, const int64_t i,
+                                                    const int32_t seg_in, const int32_t ptr_in, const int64_t row0,
+                                                    const uint64_t step, double *scratch, IO &io) {
     const int A = p.num_assets, W = p.window;
     const int lane = threadIdx.x & 31;
     const bool act = lane < A;
-    const int64_t ia = i * A + lane;
     double *xa = scratch, *xb = scratch + 32; // two 32-double rows; __syncwarp() orders the exchanges
     double O = 1.0, H = 1.0, L = 1.0, C = 1.0, margin = 0.0;
     float lng = 0.0f, sht = 0.0f, d = 0.0f;
@@ -1366,11 +1367,11 @@ __device__ __forceinline__ void portfolio_step(const FeParams &p, const FeSeries
         const double2 *px = reinterpret_cast<const double2 *>(s.prices + ((row0 + W - 1) * A + lane) * 4);
         const double2 oh = __ldg(px), lc = __ldg(px + 1);
         O = oh.x; H = oh.y; L = lc.x; C = lc.y;
-        lng = st.long_sh[ia]; sht = st.short_sh[ia]; margin = st.margin[ia];
-        d = rintf(fmul(__ldg(actions + ia), k.scale));                       // :298-302
+        lng = io.lng(); sht = io.sht(); margin = io.margin();
+        d = rintf(fmul(io.action(), k.scale));                              // :298-302
         d = d < -k.ms ? -k.ms : (d > k.ms ? k.ms : d);
     }
-    float cash = st.cash[i];
+    float cash = io.cash();
     const int32_t len = __ldg(s.seg_len + seg_in);
     float comm = 0.0f;
     float pos = d < 0.0f ? 0.0f : d, neg = d > 0.0f ? 0.0f : d;             // :344-351
@@ -1433,7 +1434,7 @@ __device__ __forceinline__ void portfolio_step(const FeParams &p, const FeSeries
         __syncwarp();
     }
     // :428-431 position feature, built before rewards / dones / reset
-    if (act) pf_smem[lane] = (OutT)__ddiv_rn(dmul((double)fsub(lng, sht), C), k.SB);
+    if (act) io.set_posfeat(lane, __ddiv_rn(dmul((double)fsub(lng, sht), C), k.SB));
     int done = cash < 0.0f;                                                  // :448
     const double mc1 = relu64(dsub(dmul(dmul((double)sht, H), k.mmr1), margin)); // :459-468 at High
     margin = dadd(margin, mc1);
@@ -1461,32 +1462,78 @@ __device__ __forceinline__ void portfolio_step(const FeParams &p, const FeSeries
         if (p.reset_mode == FE_RESET_ALL || (p.reset_mode == FE_RESET_LAST && gid == p.total_envs - 1))
             draw_segment(p, s, gid, step, 0u, seg, ptr);
     }
-    if (act) { st.long_sh[ia] = lng; st.short_sh[ia] = sht; st.margin[ia] = margin; }
-    if (lane == 0) {
+    if (act) io.finish_asset(lng, sht, margin);
+    if (io.env_lane(lane)) {                                                 // the warp-uniform part
         if (p.evaluate) {                                                    // :523-536
-            const int was = st.terminated[i];
+            const int was = io.terminated();
             if (was) rew = 0.0;
-            if (done && !was) { st.terminated[i] = 1; if (stats) atomicAdd(&stats->n_terminated, 1ULL); }
-            st.ep_return[i] = d2f(dadd((double)st.ep_return[i], rew));
-            if (done && stats) atomicAdd(&stats->n_done, 1ULL);
-        } else if (stats) {
-            const float er = d2f(dadd((double)st.ep_return[i], rew));
-            const int32_t el = st.ep_len[i] + 1;
-            if (done) {
-                atomicAdd(&stats->n_done, 1ULL);
-                atomicAdd(&stats->sum_len, (unsigned long long)el);
-                atomicAdd(&stats->sum_return, (double)er);
-                atomicAdd(&stats->sum_return_sq, (double)er * (double)er);
-            }
-            st.ep_return[i] = done ? 0.0f : er;
-            st.ep_len[i] = done ? 0 : el;
+            if (done && !was) io.set_terminated();
+            io.set_ep_return(d2f(dadd((double)io.ep_return(), rew)));
+            if (done) io.count_done();
+        } else if (io.track()) {
+            const float er = d2f(dadd((double)io.ep_return(), rew));
+            const int32_t el = io.ep_len() + 1;
+            if (done) io.count_finished(el, er);
+            io.set_ep_return(done ? 0.0f : er);
+            io.set_ep_len(done ? 0 : el);
         }
+        io.finish_env(seg, ptr, cash, rew, done);
+    }
+}
+
+// the book kernel's accessor: env i's slots of the state arrays (asset slots i * A + lane), its outputs and their mirrors,
+// FeStats atomics from lane 0, and the position feature to the warp's shared-memory row
+template <typename OutT>
+struct PortfolioGlobalIO {
+    const FeState &st;
+    const Consts &k;
+    const int64_t i, ia;
+    const float *__restrict__ actions;
+    OutT *__restrict__ rewards;
+    int32_t *__restrict__ dones;
+    FeStats *stats;
+    OutT *pf_smem;
+    __device__ __forceinline__ float lng() const { return st.long_sh[ia]; }
+    __device__ __forceinline__ float sht() const { return st.short_sh[ia]; }
+    __device__ __forceinline__ double margin() const { return st.margin[ia]; }
+    __device__ __forceinline__ float action() const { return __ldg(actions + ia); }
+    __device__ __forceinline__ float cash() const { return st.cash[i]; }
+    __device__ __forceinline__ void set_posfeat(int lane, double v) { pf_smem[lane] = (OutT)v; }
+    __device__ __forceinline__ void finish_asset(float lng, float sht, double margin) {
+        st.long_sh[ia] = lng; st.short_sh[ia] = sht; st.margin[ia] = margin;
+    }
+    __device__ __forceinline__ bool env_lane(int lane) const { return lane == 0; }
+    __device__ __forceinline__ bool track() const { return stats != nullptr; }
+    __device__ __forceinline__ int terminated() const { return st.terminated[i]; }
+    __device__ __forceinline__ void set_terminated() { st.terminated[i] = 1; if (stats) atomicAdd(&stats->n_terminated, 1ULL); }
+    __device__ __forceinline__ float ep_return() const { return st.ep_return[i]; }
+    __device__ __forceinline__ void set_ep_return(float v) { st.ep_return[i] = v; }
+    __device__ __forceinline__ int32_t ep_len() const { return st.ep_len[i]; }
+    __device__ __forceinline__ void set_ep_len(int32_t v) { st.ep_len[i] = v; }
+    __device__ __forceinline__ void count_done() { if (stats) atomicAdd(&stats->n_done, 1ULL); }
+    __device__ __forceinline__ void count_finished(int32_t el, float er) {
+        atomicAdd(&stats->n_done, 1ULL);
+        atomicAdd(&stats->sum_len, (unsigned long long)el);
+        atomicAdd(&stats->sum_return, (double)er);
+        atomicAdd(&stats->sum_return_sq, (double)er * (double)er);
+    }
+    __device__ __forceinline__ void finish_env(int32_t seg, int32_t ptr, float cash, double rew, int done) {
         st.seg[i] = seg; st.ptr[i] = ptr; st.cash[i] = cash;
         rewards[i] = (OutT)rew;
         dones[i] = done;
         if (k.rewards_mirror) reinterpret_cast<OutT *>(k.rewards_mirror)[i] = (OutT)rew;
-    if (k.dones_mirror) k.dones_mirror[i] = done;
+        if (k.dones_mirror) k.dones_mirror[i] = done;
     }
+};
+
+template <typename OutT>
+__device__ __forceinline__ void portfolio_step(const FeParams &p, const FeSeries &s, const FeState &st, const Consts &k,
+                                               const int64_t i, const int32_t seg_in, const int32_t ptr_in,
+                                               const int64_t row0, const float *__restrict__ actions,
+                                               OutT *__restrict__ rewards, int32_t *__restrict__ dones, FeStats *stats,
+                                               const uint64_t step, OutT *pf_smem, double *scratch) {
+    PortfolioGlobalIO<OutT> io{st, k, i, i * p.num_assets + (threadIdx.x & 31), actions, rewards, dones, stats, pf_smem};
+    portfolio_step_core(p, s, k, i, seg_in, ptr_in, row0, step, scratch, io);
 }
 
 // stream kernel smem: [2 mbarriers 16 B][pf 32 x OutT -> 256 B][unused 768 B][in[2]: CH*4 OutT each][out[2]: CH*5 OutT each]
@@ -2058,10 +2105,12 @@ __device__ __forceinline__ T bt_block_reduce(T v, Op op, T *sh) {
 }
 
 // The action rules of a backtest step: the table value v of env i's column at the step's row -> the action fed to
-// env_compute_core.  load(c) runs once per launch with env i's column c.
+// env_compute_core (or, per asset lane, to portfolio_step_core: E is the accessor holding that lane's long / short).
+// load(c) runs once per launch with env i's column c.
 struct TradeRule {   // fe_backtest: v is the action
     __device__ __forceinline__ void load(int32_t) {}
-    __device__ __forceinline__ float action(float v, const BacktestEnvIO &, const EpisodeRun &) const { return v; }
+    template <typename E>
+    __device__ __forceinline__ float action(float v, const E &, const EpisodeRun &) const { return v; }
 };
 struct TargetRule {  // fe_backtest_targets: v is a target net position (include/finenvs_b200.h)
     const double *__restrict__ exits;   // (num_signals, 2) trailing stop, take-profit; nullptr: no exits
@@ -2070,7 +2119,8 @@ struct TargetRule {  // fe_backtest_targets: v is a target net position (include
     __device__ __forceinline__ void load(int32_t c) {
         if (exits) { stop = __ldg(exits + 2 * (int64_t)c); take = __ldg(exits + 2 * (int64_t)c + 1); }
     }
-    __device__ __forceinline__ float action(float v, const BacktestEnvIO &e, const EpisodeRun &run) const {
+    template <typename E>
+    __device__ __forceinline__ float action(float v, const E &e, const EpisodeRun &run) const {
         float T = rintf(fmul(v, scale));
         T = T < -ms ? -ms : (T > ms ? ms : T);
         if (exits && (dsub(run.peak, run.sum) >= stop || run.sum >= take)) T = 0.0f;
@@ -2278,6 +2328,210 @@ int backtest_entry(const FeParams *p, const FeSeries *s, const FeState *st, cons
                                                                    first_step, num_steps, (OutT *)rewards, dones, history);
         return (int)cudaGetLastError();
     });
+}
+
+// ------------------------------------------------------------------------------------------
+// portfolio signal backtest (fe_backtest_portfolio): K steps in one launch, one WARP per env with lane = asset as in
+// fe_portfolio_book_kernel (lanes >= A neutral).  The table is (num_signals, num_rows, A): each step reads the A values of
+// the env's column at one row (4A contiguous bytes) and the A bars.  The step is portfolio_step_core; the per-asset long /
+// short / margin stay in the lane's registers, and every lane keeps an identical copy of the warp-uniform state (cash,
+// seg, ptr, terminated, episode return / length, the metrics' running state), so the env bookkeeping and the metrics
+// update run once per warp without any exchange.  FeStats and summary contributions accumulate per warp and are reduced
+// once per block after the loop, as in backtest_run; a finished episode takes its record slot with one atomic.
+// ------------------------------------------------------------------------------------------
+constexpr int kPbWarps = kBtWarps;   // envs per block (bt_block_reduce reduces over kBtWarps warps)
+
+// one warp's FeStats and FeMetricsSummary contributions, in shared memory (they change once per finished episode, and in
+// registers they made the kernel spill); lane 0 updates them
+struct PortfolioSums {
+    unsigned long long n_done, n_term, n_len, cnt, len;
+    double s_ret, s_sq, ret, sh, sh2, mdd, hit, max;
+};
+
+// env i's state in registers (portfolio_step_core's accessor for the backtest): the lane's asset and an identical copy
+// of the warp-uniform env state in every lane
+struct PortfolioBacktestIO {
+    float a_lng, a_sht, a_act;
+    double a_margin;
+    int32_t seg, ptr;
+    float e_cash;
+    int term;
+    float eret;
+    int32_t elen;
+    double rew;
+    int done;
+    bool tracking, lead;   // lead: lane 0, the one that counts
+    PortfolioSums *acc;
+    __device__ __forceinline__ float lng() const { return a_lng; }
+    __device__ __forceinline__ float sht() const { return a_sht; }
+    __device__ __forceinline__ double margin() const { return a_margin; }
+    __device__ __forceinline__ float action() const { return a_act; }
+    __device__ __forceinline__ float cash() const { return e_cash; }
+    __device__ __forceinline__ void set_posfeat(int, double) {}   // no observation is built
+    __device__ __forceinline__ void finish_asset(float l, float sh, double m) { a_lng = l; a_sht = sh; a_margin = m; }
+    __device__ __forceinline__ bool env_lane(int) const { return true; }
+    __device__ __forceinline__ bool track() const { return tracking; }
+    __device__ __forceinline__ int terminated() const { return term; }
+    __device__ __forceinline__ void set_terminated() { term = 1; if (lead) acc->n_term += 1; }
+    __device__ __forceinline__ float ep_return() const { return eret; }
+    __device__ __forceinline__ void set_ep_return(float v) { eret = v; }
+    __device__ __forceinline__ int32_t ep_len() const { return elen; }
+    __device__ __forceinline__ void set_ep_len(int32_t v) { elen = v; }
+    __device__ __forceinline__ void count_done() { if (tracking && lead) acc->n_done += 1; }
+    __device__ __forceinline__ void count_finished(int32_t el, float er) {
+        if (!lead) return;
+        acc->n_done += 1;
+        acc->n_len += (unsigned long long)el;
+        acc->s_ret = __dadd_rn(acc->s_ret, (double)er);
+        acc->s_sq = __dadd_rn(acc->s_sq, __dmul_rn((double)er, (double)er));
+    }
+    __device__ __forceinline__ void finish_env(int32_t seg_, int32_t ptr_, float cash_, double rew_, int done_) {
+        seg = seg_; ptr = ptr_; e_cash = cash_; rew = rew_; done = done_;
+    }
+};
+struct AssetPosition { float lng, sht; };   // what TargetRule reads of the lane's asset
+
+template <typename OutT, typename Rule>
+__global__ void __launch_bounds__(kBtThreads)
+fe_backtest_portfolio_kernel(const FeParams p, const FeSeries s, const FeState st, const Consts k, const FeMetricsState m,
+                             const int64_t capacity, FeStats *stats, const float *__restrict__ signal,
+                             const int32_t *__restrict__ column, const uint64_t first_step, const int K,
+                             OutT *__restrict__ rewards, int32_t *__restrict__ dones, const int history, Rule rule) {
+    __shared__ double scratch[kPbWarps][64];
+    __shared__ PortfolioSums sums[kPbWarps];
+    const int64_t N = p.num_envs;
+    const int A = p.num_assets, W = p.window;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int64_t i = (int64_t)blockIdx.x * kPbWarps + warp;
+    const int64_t gid = p.env_id_base + i;
+    const bool active = i < N;   // warp-uniform
+    const bool act = lane < A;
+    PortfolioBacktestIO e{};
+    e.tracking = stats != nullptr;
+    e.lead = lane == 0;
+    e.acc = &sums[warp];
+    if (lane == 0) sums[warp] = PortfolioSums{};
+    __syncwarp();
+    EpisodeRun run{};
+    int emitted = 0;
+    const float *sig = signal;
+    if (active) {
+        if (act) {
+            const int64_t ia = i * A + lane;
+            e.a_lng = st.long_sh[ia]; e.a_sht = st.short_sh[ia]; e.a_margin = st.margin[ia];
+        }
+        e.seg = st.seg[i]; e.ptr = st.ptr[i]; e.e_cash = st.cash[i];
+        if (p.evaluate) e.term = st.terminated[i];
+        if (p.evaluate || e.tracking) e.eret = st.ep_return[i];
+        if (!p.evaluate && e.tracking) e.elen = st.ep_len[i];
+        run.len = m.len[i]; run.pos = m.pos[i];
+        run.sum = m.sum[i]; run.mean = m.mean[i]; run.m2 = m.m2[i]; run.peak = m.peak[i]; run.mdd = m.mdd[i];
+        run.mdd_rel = m.mdd_rel[i];
+        if (m.emitted) emitted = m.emitted[i];
+        const int32_t c = column[i];
+        sig = signal + (int64_t)c * p.num_rows * A + lane;   // int64: S * T * A passes 2^31 on long series
+        rule.load(c);
+    }
+    PortfolioSums &acc = sums[warp];
+    if (active) {
+        for (int t = 0; t < K; ++t) {
+            const uint64_t step = first_step + (uint64_t)t;
+            const int32_t ptr = e.ptr + 1;                               // :281-282 advance time
+            const int64_t row0 = __ldg(s.seg_start + e.seg) + ptr;
+            // row row0 + W - 2 = seg_start + ptr + W - 1 with the pointer before the step: the last row of the window the
+            // env observed.  The trade executes at the next row's Open: no look-ahead.
+            if (act) e.a_act = rule.action(__ldg(sig + (row0 + W - 2) * A), AssetPosition{e.a_lng, e.a_sht}, run);
+            portfolio_step_core(p, s, k, i, e.seg, ptr, row0, step, scratch[warp], e);
+            const OutT ro = (OutT)e.rew;
+            if (lane == 0) {
+                if (history) {
+                    rewards[(int64_t)t * N + i] = ro;
+                    dones[(int64_t)t * N + i] = e.done;
+                } else if (t == K - 1) {
+                    rewards[i] = ro;
+                    dones[i] = e.done;
+                }
+            }
+            const EpisodeRun nx = episode_advance(RunInRegisters{run}, (double)ro, p.starting_balance);
+            if (e.done) {
+                int emit = 1;
+                if (m.emitted) {   // evaluate: only the first episode after the flags were cleared
+                    emit = !emitted;
+                    emitted = 1;
+                }
+                if (emit) {
+                    const double sharpe = episode_sharpe(nx), hit = episode_hit_rate(nx);
+                    if (lane == 0) {
+                        const int64_t slot = (int64_t)atomicAdd(&m.summary->episodes, 1ULL);
+                        if (slot < capacity)
+                            episode_write_record(m, slot, (int64_t)step * p.total_envs + gid, gid, nx.len, nx.sum, sharpe,
+                                                 nx.mdd, nx.mdd_rel, hit);
+                        acc.cnt += 1;
+                        acc.len += (unsigned long long)nx.len;
+                        acc.ret = __dadd_rn(acc.ret, nx.sum);
+                        acc.sh = __dadd_rn(acc.sh, sharpe);
+                        acc.sh2 = __dadd_rn(acc.sh2, __dmul_rn(sharpe, sharpe));
+                        acc.mdd = __dadd_rn(acc.mdd, nx.mdd);
+                        acc.hit = __dadd_rn(acc.hit, hit);
+                        acc.max = fmax(acc.max, nx.mdd);
+                    }
+                }
+                run = EpisodeRun{};
+            } else {
+                run = nx;
+            }
+        }
+        if (act) {
+            const int64_t ia = i * A + lane;
+            st.long_sh[ia] = e.a_lng; st.short_sh[ia] = e.a_sht; st.margin[ia] = e.a_margin;
+        }
+        if (lane == 0) {
+            st.seg[i] = e.seg; st.ptr[i] = e.ptr; st.cash[i] = e.e_cash;
+            if (p.evaluate) st.terminated[i] = (uint8_t)e.term;
+            if (p.evaluate || e.tracking) st.ep_return[i] = e.eret;
+            if (!p.evaluate && e.tracking) st.ep_len[i] = e.elen;
+            episode_store(m, i, run);
+            if (m.emitted) m.emitted[i] = (uint8_t)emitted;
+        }
+    }
+    __syncwarp();
+    const PortfolioSums w = lane == 0 ? acc : PortfolioSums{};   // each warp's sums enter once
+    __shared__ unsigned long long sh_u[kBtWarps];
+    __shared__ double sh_d[kBtWarps];
+    const auto add_u = [](unsigned long long a, unsigned long long b) { return a + b; };
+    const auto add_d = [](double a, double b) { return __dadd_rn(a, b); };
+    const auto max_d = [](double a, double b) { return fmax(a, b); };
+    if (e.tracking) {
+        const unsigned long long nd = bt_block_reduce(w.n_done, add_u, sh_u);
+        const unsigned long long nt = bt_block_reduce(w.n_term, add_u, sh_u);
+        const unsigned long long sl = bt_block_reduce(w.n_len, add_u, sh_u);
+        const double sr = bt_block_reduce(w.s_ret, add_d, sh_d);
+        const double sq = bt_block_reduce(w.s_sq, add_d, sh_d);
+        if (threadIdx.x == 0) {
+            if (nd) atomicAdd(&stats->n_done, nd);
+            if (nt) atomicAdd(&stats->n_terminated, nt);
+            if (sl) atomicAdd(&stats->sum_len, sl);
+            if (nd) { atomicAdd(&stats->sum_return, sr); atomicAdd(&stats->sum_return_sq, sq); }
+        }
+    }
+    const unsigned long long cnt = bt_block_reduce(w.cnt, add_u, sh_u);
+    const unsigned long long blen = bt_block_reduce(w.len, add_u, sh_u);
+    const double bret = bt_block_reduce(w.ret, add_d, sh_d);
+    const double bsh = bt_block_reduce(w.sh, add_d, sh_d);
+    const double bsh2 = bt_block_reduce(w.sh2, add_d, sh_d);
+    const double bmdd = bt_block_reduce(w.mdd, add_d, sh_d);
+    const double bhit = bt_block_reduce(w.hit, add_d, sh_d);
+    const double bmax = bt_block_reduce(w.max, max_d, sh_d);
+    if (threadIdx.x == 0 && cnt) {
+        FeMetricsSummary *sm = m.summary;
+        atomicAdd(&sm->sum_len, blen);
+        atomicAdd(&sm->sum_return, bret);
+        atomicAdd(&sm->sum_sharpe, bsh);
+        atomicAdd(&sm->sum_sharpe_sq, bsh2);
+        atomicAdd(&sm->sum_mdd, bmdd);
+        atomicAdd(&sm->sum_hit_rate, bhit);
+        atomicMax(reinterpret_cast<unsigned long long *>(&sm->max_mdd), (unsigned long long)__double_as_longlong(bmax));
+    }
 }
 
 // side streams of fe_step_host (created once per device, never destroyed: they live as long as the process)
@@ -2493,6 +2747,38 @@ int fe_backtest_targets(const FeParams *p, const FeSeries *s, const FeState *st,
                         void *rewards_dev, int32_t *dones_dev, int32_t history, void *stream) {
     return backtest_entry<true>(p, s, st, m, metrics_capacity, stats_dev, signal_dev, num_signals, column_dev, exits_dev,
                                 first_step, num_steps, rewards_dev, dones_dev, history, stream);
+}
+
+int fe_backtest_portfolio(const FeParams *p, const FeSeries *s, const FeState *st, const FeMetricsState *m,
+                          int64_t metrics_capacity, FeStats *stats_dev, const float *signal_dev, int32_t num_signals,
+                          const int32_t *column_dev, int32_t targets, const double *exits_dev, uint64_t first_step,
+                          int32_t num_steps, void *rewards_dev, int32_t *dones_dev, int32_t history, void *stream) {
+    int rc = check_step(p, s, st, stats_dev);
+    if (rc) return rc;
+    if (!signal_dev || num_signals < 1 || !column_dev || num_steps < 1 || !rewards_dev || !dones_dev) return FE_EINVAL;
+    if (exits_dev && !targets) return FE_EINVAL;
+    if (targets && (p->max_shares < 1 || p->max_shares > FE_TARGET_MAX_SHARES)) return FE_EINVAL;
+    if ((uintptr_t)exits_dev & 7) return FE_EALIGN;
+    if ((rc = check_metrics_state(p, m, metrics_capacity))) return rc;
+    DeviceGuard guard(p->device);
+    if (guard.rc) return guard.rc;
+    const Consts k = make_consts(*p);
+    FeMetricsState ms = *m;
+    if (!p->evaluate) ms.emitted = nullptr;
+    const unsigned blocks = (unsigned)((p->num_envs + kPbWarps - 1) / kPbWarps);
+    cudaStream_t q = (cudaStream_t)stream;
+    return with_out_type(p->out_f64, [&](auto out_type) {
+        using OutT = decltype(out_type);
+        if (targets)
+            fe_backtest_portfolio_kernel<OutT, TargetRule><<<blocks, kBtThreads, 0, q>>>(
+                *p, *s, *st, k, ms, metrics_capacity, stats_dev, signal_dev, column_dev, first_step, num_steps,
+                (OutT *)rewards_dev, dones_dev, history, TargetRule{exits_dev, k.ms, k.scale, 0.0, 0.0});
+        else
+            fe_backtest_portfolio_kernel<OutT, TradeRule><<<blocks, kBtThreads, 0, q>>>(
+                *p, *s, *st, k, ms, metrics_capacity, stats_dev, signal_dev, column_dev, first_step, num_steps,
+                (OutT *)rewards_dev, dones_dev, history, TradeRule{});
+        return (int)cudaGetLastError();
+    });
 }
 
 int fe_materialize(const FeParams *p, const FeSeries *s, const int64_t *obs_row0_dev, const void *obs_posfeat_dev,

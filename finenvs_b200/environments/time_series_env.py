@@ -779,15 +779,73 @@ class TimeSeriesEnv(BaseObject):
         self._require_metrics()
         if self.num_assets != 1:
             raise NotImplementedError("signal backtests are implemented for single-asset envs")
+        K, S, cols = self._backtest_args(signal, num_steps, columns, targets, exits, (self.series.num_rows,),
+                                         "(S, {}) tensor (one row per strategy, one value per series row)")
+        rewards, dones = self._backtest_outputs(K, history)
+        if targets:
+            _lib.check(
+                self._L.fe_backtest_targets(self._pp, self._ps, self._pst, self._pm, self.metrics_capacity,
+                                            self._stats_ptr, signal.data_ptr(), S, cols.data_ptr(),
+                                            exits.data_ptr() if exits is not None else None, self.step_count + 1, K,
+                                            rewards.data_ptr(), dones.data_ptr(), int(bool(history)), self._stream()),
+                "fe_backtest_targets",
+            )
+        else:
+            _lib.check(
+                self._L.fe_backtest(self._pp, self._ps, self._pst, self._pm, self.metrics_capacity, self._stats_ptr,
+                                    signal.data_ptr(), S, cols.data_ptr(), self.step_count + 1, K, rewards.data_ptr(),
+                                    dones.data_ptr(), int(bool(history)), self._stream()),
+                "fe_backtest",
+            )
+        return self._backtest_done(K, history, rewards, dones)
+
+    def backtest_portfolio(self, signal: torch.Tensor, num_steps: int, columns: Optional[torch.Tensor] = None,
+                           history: bool = False, *, targets: bool = False, exits: Optional[torch.Tensor] = None) -> Dict:
+        """backtest() for envs of any number of assets A (1..32), in ONE launch (fe_backtest_portfolio).
+
+        `signal` is a contiguous float32 (S, series.num_rows, A) tensor on the env's device, time-major like the series:
+        one slice per strategy ("column"), one row per row of the staged series, one value per asset.  Env i trades
+        column `columns[i]` (default: default_signal_columns) and at every step reads the A values
+        signal[columns[i], seg_start[seg] + ptr + W - 1, :] with the state before the step (the last row of the window it
+        observes; the trade executes at the next bar's Open).  Each value is that asset's action, or with targets=True
+        its target net position, mapped per asset exactly as backtest() maps the single asset's.  `exits` (S, 2) float64,
+        targets only: a trailing stop and a take-profit per column on the episode's portfolio P&L; when either triggers,
+        every asset's target is 0 for that step (not latched).
+
+        The portfolio env's rules apply: long entries, then short entries, are all-or-nothing per asset and greedy in
+        asset order, so an asset the cash left by the earlier ones cannot pay for stays flat and is retried on the next
+        step; a flip from long to short takes two steps per asset; margin calls and bankruptcy act on the whole account.
+        The result is bit-identical to `num_steps` step_into() calls with those actions (the same state, redraws,
+        stats and episode metrics as backtest() lists), and at A = 1 to backtest() with the (S, num_rows) table.
+
+        Returns {"steps": num_steps}, plus "rewards" / "dones" (num_steps, N) when history=True."""
+        self._require_metrics()
+        A = self.num_assets
+        K, S, cols = self._backtest_args(signal, num_steps, columns, targets, exits, (self.series.num_rows, A),
+                                         "(S, {}, {}) tensor (one slice per strategy, one row per series row, one value "
+                                         "per asset)")
+        rewards, dones = self._backtest_outputs(K, history)
+        _lib.check(
+            self._L.fe_backtest_portfolio(self._pp, self._ps, self._pst, self._pm, self.metrics_capacity,
+                                          self._stats_ptr, signal.data_ptr(), S, cols.data_ptr(), int(bool(targets)),
+                                          exits.data_ptr() if exits is not None else None, self.step_count + 1, K,
+                                          rewards.data_ptr(), dones.data_ptr(), int(bool(history)), self._stream()),
+            "fe_backtest_portfolio",
+        )
+        return self._backtest_done(K, history, rewards, dones)
+
+    def _backtest_args(self, signal, num_steps, columns, targets, exits, tail: Tuple[int, ...], shape_text: str):
+        """The checks every backtest entry makes before it launches (nothing runs on a refusal): -> (K, S, columns as a
+        contiguous int32 tensor on the env's device).  `tail` is the table's shape after S."""
         if self._obs_ring is not None or self._handle_ring is not None:
             raise RuntimeError("a rollout buffer is bound to this env (bind_env): a backtest would leave the observation "
                                "it holds stale")
         K = int(num_steps)
         if K < 1:
             raise ValueError("num_steps must be >= 1")
-        if not torch.is_tensor(signal) or signal.dim() != 2 or signal.shape[1] != self.series.num_rows:
-            raise ValueError(f"signal must be a (S, {self.series.num_rows}) tensor (one row per strategy, one value per "
-                             f"series row); got {tuple(signal.shape) if torch.is_tensor(signal) else type(signal)}")
+        if not torch.is_tensor(signal) or signal.dim() != 1 + len(tail) or tuple(signal.shape[1:]) != tail:
+            raise ValueError(f"signal must be a {shape_text.format(*tail)}; got "
+                             f"{tuple(signal.shape) if torch.is_tensor(signal) else type(signal)}")
         if signal.dtype != torch.float32 or signal.device != self._dev or not signal.is_contiguous():
             raise ValueError(f"signal must be a contiguous float32 tensor on {self._dev}; got {signal.dtype} on "
                              f"{signal.device}{'' if signal.is_contiguous() else ', not contiguous'}")
@@ -817,24 +875,14 @@ class TimeSeriesEnv(BaseObject):
                 raise ValueError("exit thresholds must be > 0 (+inf disables one); got a value <= 0 or NaN")
         if targets and not 1 <= self.max_shares <= _lib.TARGET_MAX_SHARES:
             raise ValueError(f"target backtests need 1 <= max_shares <= {_lib.TARGET_MAX_SHARES}")
+        return K, S, cols
+
+    def _backtest_outputs(self, K: int, history: bool) -> Tuple[torch.Tensor, torch.Tensor]:
         shape = (K, self.num_envs) if history else (self.num_envs,)
-        rewards = torch.empty(shape, dtype=self.obs_dtype, device=self._dev)
-        dones = torch.empty(shape, dtype=torch.int32, device=self._dev)
-        if targets:
-            _lib.check(
-                self._L.fe_backtest_targets(self._pp, self._ps, self._pst, self._pm, self.metrics_capacity,
-                                            self._stats_ptr, signal.data_ptr(), S, cols.data_ptr(),
-                                            exits.data_ptr() if exits is not None else None, self.step_count + 1, K,
-                                            rewards.data_ptr(), dones.data_ptr(), int(bool(history)), self._stream()),
-                "fe_backtest_targets",
-            )
-        else:
-            _lib.check(
-                self._L.fe_backtest(self._pp, self._ps, self._pst, self._pm, self.metrics_capacity, self._stats_ptr,
-                                    signal.data_ptr(), S, cols.data_ptr(), self.step_count + 1, K, rewards.data_ptr(),
-                                    dones.data_ptr(), int(bool(history)), self._stream()),
-                "fe_backtest",
-            )
+        return (torch.empty(shape, dtype=self.obs_dtype, device=self._dev),
+                torch.empty(shape, dtype=torch.int32, device=self._dev))
+
+    def _backtest_done(self, K: int, history: bool, rewards: torch.Tensor, dones: torch.Tensor) -> Dict:
         self.step_count += K
         self._epoch += 1   # a CapturedRollout's observation is stale now
         out = {"steps": K}
@@ -853,9 +901,29 @@ class TimeSeriesEnv(BaseObject):
         if not self.evaluate:
             raise RuntimeError("evaluate_signal needs an env constructed with evaluate=True")
         self._require_metrics()
+        steps = self.backtest(signal, self._evaluate_signal_steps(), columns, targets=targets, exits=exits)["steps"]
+        return self._signal_report(steps)
+
+    def evaluate_portfolio_signal(self, signal: torch.Tensor, columns: Optional[torch.Tensor] = None, *,
+                                  targets: bool = False, exits: Optional[torch.Tensor] = None) -> Dict:
+        """evaluate_signal() for a (S, num_rows, num_assets) portfolio table: one backtest_portfolio() launch of
+        max(seg_len) - W steps, then one host read of the terminated count.  Returns what evaluate_signal() returns and
+        resets the evaluation metrics.  Needs evaluate=True and track_metrics=True."""
+        if not self.evaluate:
+            raise RuntimeError("evaluate_portfolio_signal needs an env constructed with evaluate=True")
+        self._require_metrics()
+        steps = self.backtest_portfolio(signal, self._evaluate_signal_steps(), columns, targets=targets,
+                                        exits=exits)["steps"]
+        return self._signal_report(steps)
+
+    def _evaluate_signal_steps(self) -> int:
+        """Enough steps for every env to finish its current episode from any pointer."""
         if getattr(self, "_signal_steps", None) is None:
             self._signal_steps = int(self.series.seg_len.max().item()) - self.num_intervals
-        steps = self.backtest(signal, self._signal_steps, columns, targets=targets, exits=exits)["steps"]
+        return self._signal_steps
+
+    def _signal_report(self, steps: int) -> Dict:
+        """The evaluate report after a signal backtest, as evaluate_policy() builds it (and the metric reset)."""
         if int(self._stats[1].item()) >= self.num_envs:
             info = {"returns": self._ep_return.clone(), "steps": steps, "metrics": self._first_episode_metrics()}
             self.reset_evaluation_metrics()

@@ -333,6 +333,28 @@ int fe_backtest_targets(const FeParams *p, const FeSeries *s, const FeState *st,
                         const int32_t *column_dev, const double *exits_dev, uint64_t first_step, int32_t num_steps,
                         void *rewards_dev, int32_t *dones_dev, int32_t history, void *stream);
 
+/* Portfolio backtests (any 1 <= num_assets <= 32): the signal table signal_dev (num_signals, p->num_rows, A) float is
+ * time-major like the series, so the A values of one column at one row are 4A contiguous bytes.  At every step env i
+ * reads, with the state before the step,
+ *     v[a] = signal[column[i], seg_start[seg_i] + ptr_i + W - 1, a]          a = 0 .. A-1
+ * and, per asset, applies fe_backtest's rule (targets == 0: v[a] is asset a's action) or fe_backtest_targets' rule
+ * (targets != 0: v[a] is asset a's target net position, T_a = clamp(rintf(v[a] * scale), -ms, ms), action
+ * (T_a - (long_a - short_a)) / scale).  exits_dev (num_signals, 2) double, targets only: a trailing stop and a
+ * take-profit per column on the episode's portfolio P&L (the metrics' running sum / peak of the env, the sum over its
+ * assets); when either triggers, every asset's target is 0 for that step (not latched).  The portfolio env's rules
+ * apply: long entries, then short entries, are all-or-nothing per asset and greedy in asset order (an asset the cash
+ * left by the earlier ones cannot pay for stays flat and is retried on the next step), a flip from long to short takes
+ * two steps per asset, and margin calls and bankruptcy act on the whole account.  The run is bit-identical to
+ * num_steps calls of fe_step + fe_episode_metrics with actions[i, a] computed that way (the same per-env and per-asset
+ * state, redraws, FeStats counts, metrics state, records, summary counts and max_mdd; f64 sums in another order), and
+ * at A = 1 to fe_backtest / fe_backtest_targets.  Checks: fe_backtest's (except num_assets), exits_dev without
+ * targets is FE_EINVAL, a misaligned exits_dev FE_EALIGN, targets with max_shares outside [1, FE_TARGET_MAX_SHARES]
+ * FE_EINVAL; every refusal happens before any CUDA call. */
+int fe_backtest_portfolio(const FeParams *p, const FeSeries *s, const FeState *st, const FeMetricsState *m,
+                          int64_t metrics_capacity, FeStats *stats_dev, const float *signal_dev, int32_t num_signals,
+                          const int32_t *column_dev, int32_t targets, const double *exits_dev, uint64_t first_step,
+                          int32_t num_steps, void *rewards_dev, int32_t *dones_dev, int32_t history, void *stream);
+
 /* ---- ES rollout path (finenvs/agents/networks/parallel_mlp.py, finenvs/agents/ES/evo_agent.py) -------------
  * Population layout of the reference (parallel_mlp.py:121-136): envs [0, T/2) use theta + sigma*eps[p], envs
  * [T/2, T) use theta - sigma*eps[p - T/2] (T = num_envs - num_eval_envs, even), the last num_eval_envs envs use
