@@ -80,6 +80,17 @@ METRICS_SUMMARY_BYTES = 64
 TARGET_MAX_SHARES = 1 << 20
 
 
+# rule backtests (include/finenvs_b200.h, "rule backtests"): FE_RULE_* kinds, the longest lookback, the staging block
+RULE_CONST, RULE_MOMENTUM, RULE_MA_CROSS, RULE_BOLLINGER, RULE_XS_MOMENTUM = 0, 1, 2, 3, 4
+RULE_MAX_LOOKBACK = 65536
+RULE_BLOCK = 1024
+
+
+class FeRule(C.Structure):
+    _fields_ = [("kind", C.c_int32), ("lookback", C.c_int32), ("lookback2", C.c_int32), ("long_only", C.c_int32),
+                ("k", C.c_double), ("size", C.c_float), ("reserved", C.c_int32)]
+
+
 class FeMetricsState(C.Structure):
     _fields_ = [(name, C.c_void_p) for name in (
         "len", "pos", "sum", "mean", "m2", "peak", "mdd", "mdd_rel", "emitted",
@@ -131,6 +142,14 @@ _PROTOTYPES = {
                                         C.POINTER(FeMetricsState), C.c_int64, C.c_void_p, C.c_void_p, C.c_int32,
                                         C.c_void_p, C.c_int32, C.c_void_p, C.c_uint64, C.c_int32, C.c_void_p, C.c_void_p,
                                         C.c_int32, C.c_void_p]),
+    "fe_rule_sums_bytes": (C.c_int64, [C.c_int64, C.c_int32]),
+    "fe_rule_sums_build": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p]),
+    "fe_backtest_rules": (C.c_int, [C.POINTER(FeParams), C.POINTER(FeSeries), C.POINTER(FeState),
+                                    C.POINTER(FeMetricsState), C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
+                                    C.c_void_p, C.c_int32, C.c_void_p, C.c_uint64, C.c_int32, C.c_void_p, C.c_void_p,
+                                    C.c_int32, C.c_void_p]),
+    "fe_rule_table": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p,
+                                C.c_int32, C.c_void_p]),
     "fe_es_params_padded": (C.c_int64, [C.POINTER(FeEsNet)]),
     "fe_es_packed_index": (C.c_int64, [C.POINTER(FeEsNet), C.c_int32, C.c_int32, C.c_int32]),
     "fe_es_perturb": (C.c_int, [C.POINTER(FeEsNet), C.c_uint64, C.c_uint64, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p]),

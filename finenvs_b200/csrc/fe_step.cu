@@ -2059,6 +2059,184 @@ int gather_obs(const FeParams &p, const FeSeries &s, const int64_t *row0, const 
 __global__ void fe_bump_kernel(uint64_t *counter) { *counter += 1; }
 
 // ------------------------------------------------------------------------------------------
+// rules computed on the device (fe_rule_sums_build, fe_rule_table, fe_backtest_rules): the definition is the header's;
+// the numpy restatement the tests compare with repeats every operation below in the same order.
+// ------------------------------------------------------------------------------------------
+static_assert(sizeof(FeRule) == 32, "FeRule: 32 bytes (mirrored by finenvs_b200/rules.py)");
+
+// fe_rule_sums_build's buffer, time-major like the series: element [r * A + a] (base: [block * A + a])
+struct RuleSums {
+    const double *s1, *s2, *base;
+    const int32_t *nf;
+};
+
+__host__ __device__ inline int64_t rule_blocks(int64_t T) { return (T + FE_RULE_BLOCK - 1) / FE_RULE_BLOCK; }
+
+RuleSums rule_sums_view(const void *buf, int64_t T, int A) {
+    const double *s1 = (const double *)buf;
+    const double *s2 = s1 + T * A;
+    const double *base = s2 + T * A;
+    return RuleSums{s1, s2, base, (const int32_t *)(base + rule_blocks(T) * A)};
+}
+
+// one thread per (block, asset): the running sums restart at the block's first row, so they are added in row order
+// (one rounding per row, as numpy's cumsum) and stay the size of one block's deviations whatever the row index
+__global__ void __launch_bounds__(256)
+fe_rule_sums_kernel(const double *__restrict__ prices, const int64_t T, const int A, double *__restrict__ s1,
+                    double *__restrict__ s2, double *__restrict__ base, int32_t *__restrict__ nf) {
+    const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= rule_blocks(T) * A) return;
+    const int a = (int)(idx % A);
+    const int64_t r0 = idx / A * FE_RULE_BLOCK, r1 = r0 + FE_RULE_BLOCK < T ? r0 + FE_RULE_BLOCK : T;
+    double ref = 0.0;
+    for (int64_t r = r0; r < r1; ++r) {
+        const double c = __ldg(prices + (r * A + a) * 4 + 3);
+        if (isfinite(c)) { ref = c; break; }
+    }
+    double t1 = 0.0, t2 = 0.0;
+    int32_t n = 0;
+    for (int64_t r = r0; r < r1; ++r) {
+        const double c = __ldg(prices + (r * A + a) * 4 + 3);
+        double d = 0.0;
+        if (isfinite(c)) d = __dsub_rn(c, ref);
+        else n += 1;
+        t1 = __dadd_rn(t1, d);
+        t2 = __dadd_rn(t2, __dmul_rn(d, d));
+        s1[r * A + a] = t1; s2[r * A + a] = t2; nf[r * A + a] = n;
+    }
+    base[idx] = ref;
+}
+
+__device__ __forceinline__ double rule_close(const double *prices, int A, int64_t r, int a) {
+    return __ldg(prices + (r * A + a) * 4 + 3);
+}
+__device__ __forceinline__ bool rule_lookback_ok(int32_t w) { return w >= 1 && w <= FE_RULE_MAX_LOOKBACK; }
+
+// sums of C - ref over rows lo .. hi (0 <= lo <= hi) of asset a, ref = the base of hi's block, assembled from the block
+// pieces newest first, each shifted from its own base to ref; false when the window holds a non-finite close
+__device__ __forceinline__ bool rule_window(const RuleSums &z, int A, int a, int64_t lo, int64_t hi, double ref,
+                                            double &t1, double &t2) {
+    t1 = 0.0; t2 = 0.0;
+    int32_t bad = 0;
+    const int64_t bh = hi / FE_RULE_BLOCK;
+    for (int64_t b = bh; b >= lo / FE_RULE_BLOCK; --b) {
+        const int64_t b0 = b * FE_RULE_BLOCK;
+        const int64_t e = b == bh ? hi : b0 + FE_RULE_BLOCK - 1;
+        const int64_t s0 = lo > b0 ? lo : b0;
+        double p1 = __ldg(z.s1 + e * A + a), p2 = __ldg(z.s2 + e * A + a);
+        int32_t c = __ldg(z.nf + e * A + a);
+        if (s0 > b0) {
+            p1 = __dsub_rn(p1, __ldg(z.s1 + (s0 - 1) * A + a));
+            p2 = __dsub_rn(p2, __ldg(z.s2 + (s0 - 1) * A + a));
+            c -= __ldg(z.nf + (s0 - 1) * A + a);
+        }
+        if (b != bh) {   // sum (d + dl)^2 = sum d^2 + 2 dl sum d + n dl^2;  sum (d + dl) = sum d + n dl
+            const double dl = __dsub_rn(__ldg(z.base + b * A + a), ref), n = (double)(e - s0 + 1);
+            p2 = __dadd_rn(__dadd_rn(p2, __dmul_rn(__dmul_rn(2.0, dl), p1)), __dmul_rn(n, __dmul_rn(dl, dl)));
+            p1 = __dadd_rn(p1, __dmul_rn(n, dl));
+        }
+        t1 = __dadd_rn(t1, p1);
+        t2 = __dadd_rn(t2, p2);
+        bad |= c;
+    }
+    return bad == 0;
+}
+
+// s of every kind but XS_MOMENTUM at row r for asset a
+__device__ __noinline__ int rule_sign_ts(const FeRule q, const double *prices, const RuleSums z, int A, int64_t r, int a) {
+    switch (q.kind) {
+    case FE_RULE_CONST:
+        return 1;
+    case FE_RULE_MOMENTUM: {
+        if (!rule_lookback_ok(q.lookback) || r < q.lookback) return 0;
+        const double c0 = rule_close(prices, A, r, a), c1 = rule_close(prices, A, r - q.lookback, a);
+        if (!isfinite(c0) || !isfinite(c1)) return 0;
+        return c0 > c1 ? 1 : (c0 < c1 ? -1 : 0);
+    }
+    case FE_RULE_MA_CROSS: {
+        const int32_t f = q.lookback, sl = q.lookback2;
+        if (!rule_lookback_ok(f) || !rule_lookback_ok(sl) || f >= sl || r < sl - 1) return 0;
+        const double ref = __ldg(z.base + r / FE_RULE_BLOCK * A + a);
+        double f1, f2, s1, s2;
+        if (!rule_window(z, A, a, r - f + 1, r, ref, f1, f2) || !rule_window(z, A, a, r - sl + 1, r, ref, s1, s2)) return 0;
+        const double mf = __ddiv_rn(f1, (double)f), ms = __ddiv_rn(s1, (double)sl);
+        return mf > ms ? 1 : (mf < ms ? -1 : 0);
+    }
+    case FE_RULE_BOLLINGER: {
+        const int32_t w = q.lookback;
+        if (!rule_lookback_ok(w) || w < 2 || !(q.k > 0.0) || !isfinite(q.k) || r < w - 1) return 0;
+        const double ref = __ldg(z.base + r / FE_RULE_BLOCK * A + a);
+        double t1, t2;
+        if (!rule_window(z, A, a, r - w + 1, r, ref, t1, t2)) return 0;
+        const double n = (double)w, m = __ddiv_rn(t1, n);
+        double var = __dsub_rn(__ddiv_rn(t2, n), __dmul_rn(m, m));
+        var = var > 0.0 ? var : 0.0;
+        const double band = __dmul_rn(q.k, __dsqrt_rn(var));
+        const double x = __dsub_rn(rule_close(prices, A, r, a), ref);
+        return x > __dadd_rn(m, band) ? -1 : (x < __dsub_rn(m, band) ? 1 : 0);
+    }
+    default:
+        return 0;
+    }
+}
+
+// s of XS_MOMENTUM for lane `lane` of a warp whose lanes 0 .. A-1 are the assets; every lane of the warp calls it with
+// the same rule and row
+__device__ __forceinline__ int rule_sign_xs(const FeRule &q, const double *prices, int A, int64_t r, int lane) {
+    const int32_t w = q.lookback, n = q.lookback2;
+    if (!rule_lookback_ok(w) || n < 1 || n > A / 2 || r < w) return 0;
+    double ratio = 0.0;
+    bool ok = false;
+    if (lane < A) {
+        const double c0 = rule_close(prices, A, r, lane), c1 = rule_close(prices, A, r - w, lane);
+        ratio = __ddiv_rn(c0, c1);
+        ok = isfinite(c0) && isfinite(c1) && c1 != 0.0 && isfinite(ratio);
+    }
+    const unsigned valid = __ballot_sync(0xFFFFFFFFu, ok);
+    int rank = 0;
+    for (int b = 0; b < A; ++b) {
+        const double qb = __shfl_sync(0xFFFFFFFFu, ratio, b);
+        rank += ((valid >> b) & 1u) && (qb > ratio || (qb == ratio && b < lane));
+    }
+    const int m = __popc(valid);
+    if (!ok || m < 2 * n) return 0;
+    return rank < n ? 1 : (rank >= m - n ? -1 : 0);
+}
+
+__device__ __forceinline__ float rule_value(const FeRule &q, int s) {
+    if (q.long_only && s < 0) s = 0;
+    return s > 0 ? q.size : (s < 0 ? -q.size : 0.0f);
+}
+
+// the value of rule q at row r: kWarp = false for one asset (a thread of its own), true for lane `lane` of a warp whose
+// lanes are the A assets (every lane calls it; lanes >= A get 0)
+template <bool kWarp>
+__device__ __forceinline__ float rule_value_at(const FeRule &q, const double *prices, const RuleSums &z, int A, int64_t r,
+                                               int lane) {
+    if (!kWarp) return rule_value(q, rule_sign_ts(q, prices, z, 1, r, 0));
+    if (q.kind == FE_RULE_XS_MOMENTUM) return rule_value(q, rule_sign_xs(q, prices, A, r, lane));
+    return lane < A ? rule_value(q, rule_sign_ts(q, prices, z, A, r, lane)) : 0.0f;
+}
+
+// table[c, r, a] for every (column, row) item: one thread per item (kWarp = false, A = 1) or one warp (lane = asset)
+template <bool kWarp>
+__global__ void __launch_bounds__(256)
+fe_rule_table_kernel(const double *__restrict__ prices, const RuleSums z, const int64_t T, const int A,
+                     const FeRule *__restrict__ rules, const int32_t S, float *__restrict__ table) {
+    const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, all = (int64_t)gridDim.x * blockDim.x;
+    const int64_t first = kWarp ? tid >> 5 : tid, stride = kWarp ? all >> 5 : all;
+    const int lane = threadIdx.x & 31;
+    const int64_t items = (int64_t)S * T;
+    for (int64_t it = first; it < items; it += stride) {   // warp-uniform trip count when kWarp
+        const int64_t c = it / T, r = it - c * T;
+        const FeRule q = rules[c];
+        const float v = rule_value_at<kWarp>(q, prices, z, A, r, lane);
+        if (!kWarp) table[it] = v;
+        else if (lane < A) table[it * A + lane] = v;
+    }
+}
+
+// ------------------------------------------------------------------------------------------
 // signal backtest (fe_backtest, fe_backtest_targets): K steps of every env in one launch, one thread per env.  The
 // action of each step comes from the env's column of a signal table: the value itself (TradeRule) or the delta to a
 // target position (TargetRule); the step is env_compute_core (the trading arithmetic of every step
@@ -2129,14 +2307,47 @@ struct TargetRule {  // fe_backtest_targets: v is a target net position (include
     }
 };
 
-// the backtest loop of both entry points; Rule turns each step's table value into the action.  The structs are taken
-// by value: with references the compiler numbered fe_backtest_kernel's accumulators differently and its SASS changed.
-template <typename OutT, typename Rule>
+// Where a backtest step's value v comes from, once per launch set up with the env's column c.
+//   portfolio loop: load(c, T, A, lane); per step prepare(row, lane) in every lane of the warp (before the loop's
+//                   `if (act)`), then value(row, A), the lane's v at that row;
+//   backtest_run:   load(c); per step value(at, row), where `at` is the table element's address, computed by
+//                   backtest_run as it always was (computed inside the source, or in another order, the pointer
+//                   arithmetic renumbered the registers of fe_backtest_kernel and fe_backtest_targets_kernel).
+struct TableSource {   // fe_backtest*, fe_backtest_portfolio: the (S, T, A) table
+    const float *sig;
+    __device__ __forceinline__ void load(int32_t c, int64_t T, int A, int lane) { sig += (int64_t)c * T * A + lane; }
+    __device__ __forceinline__ void prepare(int64_t, int) {}
+    __device__ __forceinline__ float value(int64_t row, int A) const { return __ldg(sig + row * A); }
+    __device__ __forceinline__ void load(int32_t) {}
+    __device__ __forceinline__ float value(const float *at, int64_t) const { return __ldg(at); }
+};
+template <bool kWarp>
+struct RuleSource {    // fe_backtest_rules: the rule of the column, evaluated on the staged closes
+    const FeRule *__restrict__ rules;
+    const double *__restrict__ prices;
+    RuleSums z;
+    int A;
+    FeRule q;
+    float v;
+    __device__ __forceinline__ void load(int32_t c, int64_t = 0, int = 0, int = 0) { q = rules[c]; }
+    __device__ __forceinline__ void prepare(int64_t row, int lane) {
+        if (kWarp) v = rule_value_at<true>(q, prices, z, A, row, lane);
+    }
+    __device__ __forceinline__ float value(int64_t, int) const { return v; }
+    __device__ __forceinline__ float value(const float *, int64_t row) const {
+        return rule_value_at<false>(q, prices, z, 1, row, 0);
+    }
+};
+
+// the backtest loop of the single-asset entry points; Source gives each step's value (the table's: signal[column[i], row])
+// and Rule turns it into the action.  The structs are taken by value: with references the compiler numbered
+// fe_backtest_kernel's accumulators differently and its SASS changed.
+template <typename OutT, typename Rule, typename Source = TableSource>
 __device__ __forceinline__ void
 backtest_run(const FeParams p, const FeSeries s, const FeState st, const Consts k, const FeMetricsState m,
              const int64_t capacity, FeStats *stats, const float *__restrict__ signal, const int32_t *__restrict__ column,
              const uint64_t first_step, const int K, OutT *__restrict__ rewards, int32_t *__restrict__ dones,
-             const int history, Rule rule) {
+             const int history, Rule rule, Source src = {}) {
     constexpr unsigned kAll = 0xFFFFFFFFu;
     const int64_t N = p.num_envs;
     const int64_t i = (int64_t)blockIdx.x * kBtThreads + threadIdx.x;
@@ -2160,6 +2371,7 @@ backtest_run(const FeParams p, const FeSeries s, const FeState st, const Consts 
         if (m.emitted) emitted = m.emitted[i];
         const int32_t c = column[i];
         sig = signal + (int64_t)c * p.num_rows;
+        src.load(c);
         rule.load(c);
     }
     // FeStats and FeMetricsSummary contributions, flushed once per block after the loop; only the slot counter
@@ -2179,7 +2391,7 @@ backtest_run(const FeParams p, const FeSeries s, const FeState st, const Consts 
             const EnvBar bar = env_load_bar(p, s, ld);
             // row seg_start + ptr + W - 1: the last row of the window the env observed before this step (bar.row0 is the
             // window after the advance).  The trade executes at the next row's Open: no look-ahead.
-            ld.act = rule.action(__ldg(sig + bar.row0 + p.window - 2), e, run);
+            ld.act = rule.action(src.value(sig + bar.row0 + p.window - 2, bar.row0 + p.window - 2), e, run);
             const EnvResult r = env_compute_core(p, s, k, i, ld, bar, track, step, e);
             const OutT ro = (OutT)e.rew;
             if (history) {
@@ -2299,6 +2511,16 @@ fe_backtest_targets_kernel(const FeParams p, const FeSeries s, const FeState st,
     backtest_run<OutT>(p, s, st, k, m, capacity, stats, signal, column, first_step, K, rewards, dones, history, rule);
 }
 
+// fe_backtest_rules at A = 1: backtest_run fed by the rule of the env's column
+template <typename OutT, typename Rule>
+__global__ void __launch_bounds__(kBtThreads)
+fe_backtest_rules_kernel(const FeParams p, const FeSeries s, const FeState st, const Consts k, const FeMetricsState m,
+                         const int64_t capacity, FeStats *stats, const RuleSource<false> src,
+                         const int32_t *__restrict__ column, const uint64_t first_step, const int K,
+                         OutT *__restrict__ rewards, int32_t *__restrict__ dones, const int history, const Rule rule) {
+    backtest_run<OutT>(p, s, st, k, m, capacity, stats, nullptr, column, first_step, K, rewards, dones, history, rule, src);
+}
+
 // fe_backtest (kTargets = false, exits == nullptr) and fe_backtest_targets: validation and launch
 template <bool kTargets>
 int backtest_entry(const FeParams *p, const FeSeries *s, const FeState *st, const FeMetricsState *m, int64_t capacity,
@@ -2391,12 +2613,13 @@ struct PortfolioBacktestIO {
 };
 struct AssetPosition { float lng, sht; };   // what TargetRule reads of the lane's asset
 
-template <typename OutT, typename Rule>
-__global__ void __launch_bounds__(kBtThreads)
-fe_backtest_portfolio_kernel(const FeParams p, const FeSeries s, const FeState st, const Consts k, const FeMetricsState m,
-                             const int64_t capacity, FeStats *stats, const float *__restrict__ signal,
-                             const int32_t *__restrict__ column, const uint64_t first_step, const int K,
-                             OutT *__restrict__ rewards, int32_t *__restrict__ dones, const int history, Rule rule) {
+// the loop of fe_backtest_portfolio_kernel and fe_backtest_rules_portfolio_kernel
+template <typename OutT, typename Source, typename Rule>
+__device__ __forceinline__ void
+backtest_portfolio_run(const FeParams p, const FeSeries s, const FeState st, const Consts k, const FeMetricsState m,
+                       const int64_t capacity, FeStats *stats, Source src, const int32_t *__restrict__ column,
+                       const uint64_t first_step, const int K, OutT *__restrict__ rewards, int32_t *__restrict__ dones,
+                       const int history, Rule rule) {
     __shared__ double scratch[kPbWarps][64];
     __shared__ PortfolioSums sums[kPbWarps];
     const int64_t N = p.num_envs;
@@ -2414,7 +2637,6 @@ fe_backtest_portfolio_kernel(const FeParams p, const FeSeries s, const FeState s
     __syncwarp();
     EpisodeRun run{};
     int emitted = 0;
-    const float *sig = signal;
     if (active) {
         if (act) {
             const int64_t ia = i * A + lane;
@@ -2429,7 +2651,7 @@ fe_backtest_portfolio_kernel(const FeParams p, const FeSeries s, const FeState s
         run.mdd_rel = m.mdd_rel[i];
         if (m.emitted) emitted = m.emitted[i];
         const int32_t c = column[i];
-        sig = signal + (int64_t)c * p.num_rows * A + lane;   // int64: S * T * A passes 2^31 on long series
+        src.load(c, p.num_rows, A, lane);   // int64: S * T * A passes 2^31 on long series
         rule.load(c);
     }
     PortfolioSums &acc = sums[warp];
@@ -2439,8 +2661,10 @@ fe_backtest_portfolio_kernel(const FeParams p, const FeSeries s, const FeState s
             const int32_t ptr = e.ptr + 1;                               // :281-282 advance time
             const int64_t row0 = __ldg(s.seg_start + e.seg) + ptr;
             // row row0 + W - 2 = seg_start + ptr + W - 1 with the pointer before the step: the last row of the window the
-            // env observed.  The trade executes at the next row's Open: no look-ahead.
-            if (act) e.a_act = rule.action(__ldg(sig + (row0 + W - 2) * A), AssetPosition{e.a_lng, e.a_sht}, run);
+            // env observed.  The trade executes at the next row's Open: no look-ahead.  A rule's cross-sectional rank needs
+            // every lane in its shuffles, so prepare runs outside `if (act)`.
+            src.prepare(row0 + W - 2, lane);
+            if (act) e.a_act = rule.action(src.value(row0 + W - 2, A), AssetPosition{e.a_lng, e.a_sht}, run);
             portfolio_step_core(p, s, k, i, e.seg, ptr, row0, step, scratch[warp], e);
             const OutT ro = (OutT)e.rew;
             if (lane == 0) {
@@ -2532,6 +2756,28 @@ fe_backtest_portfolio_kernel(const FeParams p, const FeSeries s, const FeState s
         atomicAdd(&sm->sum_hit_rate, bhit);
         atomicMax(reinterpret_cast<unsigned long long *>(&sm->max_mdd), (unsigned long long)__double_as_longlong(bmax));
     }
+}
+
+template <typename OutT, typename Rule>
+__global__ void __launch_bounds__(kBtThreads)
+fe_backtest_portfolio_kernel(const FeParams p, const FeSeries s, const FeState st, const Consts k, const FeMetricsState m,
+                             const int64_t capacity, FeStats *stats, const float *__restrict__ signal,
+                             const int32_t *__restrict__ column, const uint64_t first_step, const int K,
+                             OutT *__restrict__ rewards, int32_t *__restrict__ dones, const int history, Rule rule) {
+    backtest_portfolio_run<OutT>(p, s, st, k, m, capacity, stats, TableSource{signal}, column, first_step, K, rewards,
+                                 dones, history, rule);
+}
+
+// fe_backtest_rules at A > 1: the portfolio loop fed by the rule of the env's column
+template <typename OutT, typename Rule>
+__global__ void __launch_bounds__(kBtThreads)
+fe_backtest_rules_portfolio_kernel(const FeParams p, const FeSeries s, const FeState st, const Consts k,
+                                   const FeMetricsState m, const int64_t capacity, FeStats *stats,
+                                   const RuleSource<true> src, const int32_t *__restrict__ column,
+                                   const uint64_t first_step, const int K, OutT *__restrict__ rewards,
+                                   int32_t *__restrict__ dones, const int history, const Rule rule) {
+    backtest_portfolio_run<OutT>(p, s, st, k, m, capacity, stats, src, column, first_step, K, rewards, dones, history,
+                                 rule);
 }
 
 // side streams of fe_step_host (created once per device, never destroyed: they live as long as the process)
@@ -2777,6 +3023,94 @@ int fe_backtest_portfolio(const FeParams *p, const FeSeries *s, const FeState *s
             fe_backtest_portfolio_kernel<OutT, TradeRule><<<blocks, kBtThreads, 0, q>>>(
                 *p, *s, *st, k, ms, metrics_capacity, stats_dev, signal_dev, column_dev, first_step, num_steps,
                 (OutT *)rewards_dev, dones_dev, history, TradeRule{});
+        return (int)cudaGetLastError();
+    });
+}
+
+int64_t fe_rule_sums_bytes(int64_t num_rows, int32_t num_assets) {
+    if (num_rows <= 0 || num_assets < 1 || num_assets > 32) return 0;
+    return num_rows * num_assets * (8 + 8 + 4) + rule_blocks(num_rows) * num_assets * 8;
+}
+
+int fe_rule_sums_build(const double *prices_dev, int64_t num_rows, int32_t num_assets, void *sums_dev, int32_t device,
+                       void *stream) {
+    if (!prices_dev || !sums_dev || fe_rule_sums_bytes(num_rows, num_assets) == 0) return FE_EINVAL;
+    if (((uintptr_t)prices_dev | (uintptr_t)sums_dev) & 15) return FE_EALIGN;
+    DeviceGuard guard(device);
+    if (guard.rc) return guard.rc;
+    const RuleSums z = rule_sums_view(sums_dev, num_rows, num_assets);
+    const int64_t threads = rule_blocks(num_rows) * num_assets;
+    fe_rule_sums_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+        prices_dev, num_rows, num_assets, (double *)z.s1, (double *)z.s2, (double *)z.base, (int32_t *)z.nf);
+    return (int)cudaGetLastError();
+}
+
+int fe_backtest_rules(const FeParams *p, const FeSeries *s, const FeState *st, const FeMetricsState *m,
+                      int64_t metrics_capacity, FeStats *stats_dev, const void *rule_sums_dev, const FeRule *rules_dev,
+                      int32_t num_rules, const int32_t *column_dev, int32_t targets, const double *exits_dev,
+                      uint64_t first_step, int32_t num_steps, void *rewards_dev, int32_t *dones_dev, int32_t history,
+                      void *stream) {
+    int rc = check_step(p, s, st, stats_dev);
+    if (rc) return rc;
+    if (!rule_sums_dev || !rules_dev || num_rules < 1 || !column_dev || num_steps < 1 || !rewards_dev || !dones_dev)
+        return FE_EINVAL;
+    if (exits_dev && !targets) return FE_EINVAL;
+    if (targets && (p->max_shares < 1 || p->max_shares > FE_TARGET_MAX_SHARES)) return FE_EINVAL;
+    if (((uintptr_t)exits_dev | (uintptr_t)rules_dev | (uintptr_t)rule_sums_dev) & 7) return FE_EALIGN;
+    if ((rc = check_metrics_state(p, m, metrics_capacity))) return rc;
+    DeviceGuard guard(p->device);
+    if (guard.rc) return guard.rc;
+    const Consts k = make_consts(*p);
+    FeMetricsState ms = *m;
+    if (!p->evaluate) ms.emitted = nullptr;
+    const int A = p->num_assets;
+    const RuleSums z = rule_sums_view(rule_sums_dev, p->num_rows, A);
+    cudaStream_t q = (cudaStream_t)stream;
+    const TargetRule target{exits_dev, k.ms, k.scale, 0.0, 0.0};
+    return with_out_type(p->out_f64, [&](auto out_type) {
+        using OutT = decltype(out_type);
+        OutT *rew = (OutT *)rewards_dev;
+        return with_flag(targets != 0, [&](auto tgt) {
+            using Rule = std::conditional_t<decltype(tgt)::value, TargetRule, TradeRule>;
+            Rule rule{};
+            if constexpr (decltype(tgt)::value) rule = target;
+            if (A == 1) {
+                const unsigned blocks = (unsigned)((p->num_envs + kBtThreads - 1) / kBtThreads);
+                const RuleSource<false> src{rules_dev, s->prices, z, 1, FeRule{}, 0.0f};
+                fe_backtest_rules_kernel<OutT, Rule><<<blocks, kBtThreads, 0, q>>>(
+                    *p, *s, *st, k, ms, metrics_capacity, stats_dev, src, column_dev, first_step, num_steps, rew, dones_dev,
+                    history, rule);
+            } else {
+                const unsigned blocks = (unsigned)((p->num_envs + kPbWarps - 1) / kPbWarps);
+                const RuleSource<true> src{rules_dev, s->prices, z, A, FeRule{}, 0.0f};
+                fe_backtest_rules_portfolio_kernel<OutT, Rule><<<blocks, kBtThreads, 0, q>>>(
+                    *p, *s, *st, k, ms, metrics_capacity, stats_dev, src, column_dev, first_step, num_steps, rew, dones_dev,
+                    history, rule);
+            }
+            return (int)cudaGetLastError();
+        });
+    });
+}
+
+int fe_rule_table(const double *prices_dev, const void *rule_sums_dev, int64_t num_rows, int32_t num_assets,
+                  const FeRule *rules_dev, int32_t num_rules, float *table_dev, int32_t device, void *stream) {
+    if (!prices_dev || !rule_sums_dev || !rules_dev || !table_dev || num_rules < 1) return FE_EINVAL;
+    if (fe_rule_sums_bytes(num_rows, num_assets) == 0) return FE_EINVAL;
+    if ((((uintptr_t)prices_dev | (uintptr_t)rule_sums_dev | (uintptr_t)rules_dev) & 7) || ((uintptr_t)table_dev & 3))
+        return FE_EALIGN;
+    DeviceGuard guard(device);
+    if (guard.rc) return guard.rc;
+    int sms = 0;
+    int rc = device_sm_count(device, &sms);
+    if (rc) return rc;
+    const RuleSums z = rule_sums_view(rule_sums_dev, num_rows, num_assets);
+    const int64_t items = (int64_t)num_rules * num_rows;
+    const bool warp = num_assets > 1;
+    const int64_t need = (items * (warp ? 32 : 1) + 255) / 256, cap = (int64_t)sms * 16;
+    const unsigned blocks = (unsigned)(need < cap ? need : cap);
+    return with_flag(warp, [&](auto w) {
+        fe_rule_table_kernel<decltype(w)::value><<<blocks, 256, 0, (cudaStream_t)stream>>>(
+            prices_dev, z, num_rows, num_assets, rules_dev, num_rules, table_dev);
         return (int)cudaGetLastError();
     });
 }

@@ -192,6 +192,7 @@ class StagedSeries:
     logret64: torch.Tensor | None = None  # kept only when asked (loader parity tests)
     _obs_table: torch.Tensor | None = None  # observation-layout table of the gather kernel (built on first use)
     _obs_table_tried: bool = False
+    _rule_sums: torch.Tensor | None = None  # running sums of the closes for device-side rules (built on first use)
 
     @property
     def num_rows(self) -> int:
@@ -210,7 +211,7 @@ class StagedSeries:
         return self.prices.device
 
     def nbytes(self) -> int:
-        extra = self._obs_table.numel() if self._obs_table is not None else 0
+        extra = sum(t.numel() for t in (self._obs_table, self._rule_sums) if t is not None)
         return extra + sum(t.numel() * t.element_size() for t in (self.prices, self.logret, self.seg_start, self.seg_len))
 
     # the table only pays while it stays L2-resident beside the observation stream (csrc/fe_step.cu: gather_table_resident)
@@ -237,6 +238,21 @@ class StagedSeries:
                                             torch.cuda.current_stream(self.device).cuda_stream), "fe_obs_table_build")
         self._obs_table = table
         return table
+
+    def rule_sums(self) -> torch.Tensor:
+        """Per asset, block-local running sums of the closes and their squares (include/finenvs_b200.h, "rule
+        backtests"), from which the device evaluates moving-average and band rules in O(1 + lookback / 1024) loads
+        per value.  Built once per series on first use (fe_rule_sums_build): fe_rule_sums_bytes(T, A) bytes, about 20
+        per row and asset."""
+        if self._rule_sums is None:
+            L = _lib.lib()
+            T, A = self.num_rows, self.num_assets
+            with torch.cuda.device(self.device):
+                sums = torch.empty(int(L.fe_rule_sums_bytes(T, A)), dtype=torch.uint8, device=self.device)
+                _lib.check(L.fe_rule_sums_build(self.prices.data_ptr(), T, A, sums.data_ptr(), self.device.index,
+                                                torch.cuda.current_stream(self.device).cuda_stream), "fe_rule_sums_build")
+            self._rule_sums = sums
+        return self._rule_sums
 
 
 def stage_series(prices, seg_start, seg_len_raw, window: int, device: str, obs_dtype=torch.float32,

@@ -17,7 +17,7 @@ from typing import Dict, Optional, Tuple
 import numpy as np
 import torch
 
-from .. import _lib
+from .. import _lib, rules as _rules
 from ..base_object import BaseObject
 from ..data import loader
 from ..device_utils import require_cuda_device
@@ -834,22 +834,27 @@ class TimeSeriesEnv(BaseObject):
         )
         return self._backtest_done(K, history, rewards, dones)
 
-    def _backtest_args(self, signal, num_steps, columns, targets, exits, tail: Tuple[int, ...], shape_text: str):
+    def _backtest_args(self, signal, num_steps, columns, targets, exits, tail: Optional[Tuple[int, ...]],
+                       shape_text: str = ""):
         """The checks every backtest entry makes before it launches (nothing runs on a refusal): -> (K, S, columns as a
-        contiguous int32 tensor on the env's device).  `tail` is the table's shape after S."""
+        contiguous int32 tensor on the env's device).  `tail` is the table's shape after S; tail=None: `signal` is the
+        number of columns of a rule set (backtest_rules), there is no table to check."""
         if self._obs_ring is not None or self._handle_ring is not None:
             raise RuntimeError("a rollout buffer is bound to this env (bind_env): a backtest would leave the observation "
                                "it holds stale")
         K = int(num_steps)
         if K < 1:
             raise ValueError("num_steps must be >= 1")
-        if not torch.is_tensor(signal) or signal.dim() != 1 + len(tail) or tuple(signal.shape[1:]) != tail:
-            raise ValueError(f"signal must be a {shape_text.format(*tail)}; got "
-                             f"{tuple(signal.shape) if torch.is_tensor(signal) else type(signal)}")
-        if signal.dtype != torch.float32 or signal.device != self._dev or not signal.is_contiguous():
-            raise ValueError(f"signal must be a contiguous float32 tensor on {self._dev}; got {signal.dtype} on "
-                             f"{signal.device}{'' if signal.is_contiguous() else ', not contiguous'}")
-        S = signal.shape[0]
+        if tail is None:
+            S = int(signal)
+        else:
+            if not torch.is_tensor(signal) or signal.dim() != 1 + len(tail) or tuple(signal.shape[1:]) != tail:
+                raise ValueError(f"signal must be a {shape_text.format(*tail)}; got "
+                                 f"{tuple(signal.shape) if torch.is_tensor(signal) else type(signal)}")
+            if signal.dtype != torch.float32 or signal.device != self._dev or not signal.is_contiguous():
+                raise ValueError(f"signal must be a contiguous float32 tensor on {self._dev}; got {signal.dtype} on "
+                                 f"{signal.device}{'' if signal.is_contiguous() else ', not contiguous'}")
+            S = signal.shape[0]
         if S < 1 or S > 0x7FFFFFFF:
             raise ValueError("signal must have between 1 and 2**31 - 1 rows")
         if columns is None:
@@ -915,6 +920,72 @@ class TimeSeriesEnv(BaseObject):
         steps = self.backtest_portfolio(signal, self._evaluate_signal_steps(), columns, targets=targets,
                                         exits=exits)["steps"]
         return self._signal_report(steps)
+
+    # ------------------------------------------------------------------ rules computed on the device (DESIGN §4.12) ----
+    def _check_rules(self, rules: "_rules.RuleSet") -> int:
+        """Host-side checks of a rule set for this env (nothing touches the device): -> R."""
+        if not isinstance(rules, _rules.RuleSet):
+            raise ValueError(f"rules must be a finenvs_b200.rules.RuleSet; got {type(rules)}")
+        _rules.check_records(rules.records, self.num_assets)
+        return len(rules)
+
+    def _upload_rules(self, rules: "_rules.RuleSet") -> torch.Tensor:
+        """The records, R * 32 bytes on the env's device (after every check has passed)."""
+        return torch.from_numpy(rules.records.view(np.uint8)).to(self._dev)
+
+    def backtest_rules(self, rules: "_rules.RuleSet", num_steps: int, columns: Optional[torch.Tensor] = None,
+                       history: bool = False, *, targets: bool = False, exits: Optional[torch.Tensor] = None) -> Dict:
+        """backtest() / backtest_portfolio() with every value computed on the device by a rule (finenvs_b200.rules)
+        instead of read from a signal table, in ONE launch (fe_backtest_rules).  Column c of the rule set is rule c; env i
+        runs rule columns[i] (default: default_signal_columns) and at every step takes that rule's value at row
+        seg_start[seg] + ptr + W - 1 (state before the step), which reads closes of that row and earlier only.
+        targets / exits are backtest()'s (exits: (R, 2) float64).  The rule's value per row is fixed by the rule and the
+        series alone, so no (R, num_rows[, A]) table is ever built: the series' running sums (StagedSeries.rule_sums(),
+        ~20 bytes per row and asset, staged once) are all the extra memory.
+
+        Contract: at A = 1 the result is bit-identical to backtest(rule_table(rules), num_steps, ...), at A > 1 to
+        backtest_portfolio(rule_table(rules), num_steps, ...) with the same arguments: per-env state, redraws, stats
+        counts, episode metrics state, records, summary counts and max_mdd; f64 sums equal up to their order of
+        addition.  Refuses what backtest() refuses, and rules the env cannot run (xs_momentum needs 2n assets).
+
+        Returns {"steps": num_steps}, plus "rewards" / "dones" (num_steps, N) when history=True."""
+        self._require_metrics()
+        K, S, cols = self._backtest_args(self._check_rules(rules), num_steps, columns, targets, exits, None)
+        recs = self._upload_rules(rules)
+        sums = self.series.rule_sums()
+        rewards, dones = self._backtest_outputs(K, history)
+        _lib.check(
+            self._L.fe_backtest_rules(self._pp, self._ps, self._pst, self._pm, self.metrics_capacity, self._stats_ptr,
+                                      sums.data_ptr(), recs.data_ptr(), S, cols.data_ptr(), int(bool(targets)),
+                                      exits.data_ptr() if exits is not None else None, self.step_count + 1, K,
+                                      rewards.data_ptr(), dones.data_ptr(), int(bool(history)), self._stream()),
+            "fe_backtest_rules",
+        )
+        return self._backtest_done(K, history, rewards, dones)
+
+    def evaluate_rules(self, rules: "_rules.RuleSet", columns: Optional[torch.Tensor] = None, *, targets: bool = False,
+                       exits: Optional[torch.Tensor] = None) -> Dict:
+        """The evaluate-mode report of a rule set: one backtest_rules() launch of max(seg_len) - W steps, then one host
+        read of the terminated count.  Returns what evaluate_signal() / evaluate_portfolio_signal() return for
+        rule_table(rules) and resets the evaluation metrics.  Needs evaluate=True and track_metrics=True."""
+        if not self.evaluate:
+            raise RuntimeError("evaluate_rules needs an env constructed with evaluate=True")
+        self._require_metrics()
+        steps = self.backtest_rules(rules, self._evaluate_signal_steps(), columns, targets=targets, exits=exits)["steps"]
+        return self._signal_report(steps)
+
+    def rule_table(self, rules: "_rules.RuleSet") -> torch.Tensor:
+        """The signal table a rule set defines on this env's series (fe_rule_table, the device function backtest_rules
+        evaluates): float32 (R, num_rows) for a single-asset env, (R, num_rows, A) for a portfolio.  For inspecting or
+        plotting rule values, and the table backtest() / backtest_portfolio() take."""
+        R = self._check_rules(rules)
+        recs = self._upload_rules(rules)
+        A, T = self.num_assets, self.series.num_rows
+        table = torch.empty((R, T) if A == 1 else (R, T, A), dtype=torch.float32, device=self._dev)
+        _lib.check(self._L.fe_rule_table(self.series.prices.data_ptr(), self.series.rule_sums().data_ptr(), T, A,
+                                         recs.data_ptr(), R, table.data_ptr(), self._dev.index, self._stream()),
+                   "fe_rule_table")
+        return table
 
     def _evaluate_signal_steps(self) -> int:
         """Enough steps for every env to finish its current episode from any pointer."""

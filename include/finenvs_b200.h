@@ -355,6 +355,85 @@ int fe_backtest_portfolio(const FeParams *p, const FeSeries *s, const FeState *s
                           const int32_t *column_dev, int32_t targets, const double *exits_dev, uint64_t first_step,
                           int32_t num_steps, void *rewards_dev, int32_t *dones_dev, int32_t history, void *stream);
 
+/* ---- rule backtests (extension; DESIGN.md §4.12, "Rules computed on the device") ---------------------------
+ * A rule is a 32-byte FeRule record; a rule set is an array of them indexed by column, and its value at a row r of the
+ * staged series (the row fe_backtest reads, seg_start + ptr + W - 1 before the step) for asset a is computed from the
+ * closes C[j] = prices[j, a, 3] (f64) of rows j <= r only:
+ *     s in {-1, 0, +1} by kind (0 while r is too small for the lookback, i.e. a row before 0 would be needed):
+ *       FE_RULE_CONST         +1
+ *       FE_RULE_MOMENTUM      (lookback w >= 1) sign(C[r] - C[r-w]); 0 when equal or either close is not finite
+ *       FE_RULE_MA_CROSS      (lookback f, lookback2 sl, 1 <= f < sl) sign(M_f - M_sl), M_k the mean of C over r-k+1 .. r
+ *       FE_RULE_BOLLINGER     (lookback w >= 2, k > 0) -1 if C[r] > M_w + k sd_w, +1 if C[r] < M_w - k sd_w, else 0
+ *                             (sd_w: population standard deviation of the same w closes)
+ *       FE_RULE_XS_MOMENTUM   (lookback w >= 1, lookback2 n, 1 <= n <= A/2; portfolios) rank the assets by
+ *                             q_a = C_a[r] / C_a[r-w], descending, ties to the lower asset index: +1 for the first n,
+ *                             -1 for the last n, 0 otherwise.  An asset whose q is not finite (a non-finite close, or
+ *                             C_a[r-w] == 0) takes no rank and gets 0, and the others are ranked among themselves; when
+ *                             fewer than 2n assets have a finite q, every asset gets 0.
+ *     long_only != 0 maps s to max(s, 0); the value is v = +size, -size or +0.0f for s = +1, -1, 0, and goes into
+ *     fe_backtest_portfolio's rule unchanged (an action, or with targets a target net position).
+ * Time-series kinds apply per asset to the asset's own closes; CONST gives every asset `size`.  Any window containing a
+ * non-finite close gives 0 (MA_CROSS, BOLLINGER).  Every value is a function of (rule, row, asset) alone, computed with
+ * IEEE f64 basic operations and sqrt in a fixed order (no FMA), so a numpy restatement (oracle/oracle_rules.py) matches
+ * bit for bit.  Evaluation is total: an unknown kind, a lookback outside [1, FE_RULE_MAX_LOOKBACK], or a parameter
+ * outside the ranges above gives 0 and reads nothing, so no record can make a kernel read outside the series.
+ *
+ * Window means and deviations come from running sums staged once per series by fe_rule_sums_build: per asset, the
+ * series is cut into blocks of FE_RULE_BLOCK rows; each block has a base (its first finite close, 0 if none) and holds
+ * inclusive running sums, restarted at the block's first row, of d = C - base and d*d (d = 0 for a non-finite close,
+ * which is counted instead).  A window sum is assembled from at most 1 + lookback / FE_RULE_BLOCK block pieces, each
+ * shifted to the base of the window's last block (a single prefix sum over 10 M rows would cancel catastrophically).
+ * Accuracy: the window variance (BOLLINGER's sd_w^2, formed as t2/w - (t1/w)^2 from those sums) has an ABSOLUTE error
+ * of at most a small multiple of u * M (u = 2^-53), where M, the sum of the magnitudes of the staged terms the window
+ * is formed from divided by w, is set by the prices and their drift inside the window's blocks, not by the row index
+ * (measured on every row of a 10 M-row series: below 51 u M; oracle_rules.window_error_scale computes M).  The error is
+ * not relative: a window whose variance is far below u M, such as two nearly equal closes late in a block, can carry a
+ * large relative error in sd_w, and a window of equal closes can get sd_w of order sqrt(u M) instead of 0.  Window
+ * means hold a relative error of a few ulps.  The buffer holds, for
+ * T rows, A assets and B = ceil(T / FE_RULE_BLOCK) blocks: sum d (T, A) f64, sum d*d (T, A) f64, base (B, A) f64,
+ * non-finite count (T, A) int32 — fe_rule_sums_bytes() bytes, 16-byte aligned. */
+#define FE_RULE_CONST 0
+#define FE_RULE_MOMENTUM 1
+#define FE_RULE_MA_CROSS 2
+#define FE_RULE_BOLLINGER 3
+#define FE_RULE_XS_MOMENTUM 4
+#define FE_RULE_MAX_LOOKBACK 65536
+#define FE_RULE_BLOCK 1024
+
+typedef struct FeRule {
+    int32_t kind;       /* FE_RULE_* */
+    int32_t lookback;   /* w (MOMENTUM, BOLLINGER, XS_MOMENTUM) or the fast f (MA_CROSS) */
+    int32_t lookback2;  /* the slow sl (MA_CROSS) or n (XS_MOMENTUM); 0 otherwise */
+    int32_t long_only;  /* != 0: s -> max(s, 0) */
+    double k;           /* BOLLINGER band width in standard deviations; 0 otherwise */
+    float size;         /* v = s * size */
+    int32_t reserved;   /* 0 */
+} FeRule;
+
+int64_t fe_rule_sums_bytes(int64_t num_rows, int32_t num_assets);
+int fe_rule_sums_build(const double *prices_dev, int64_t num_rows, int32_t num_assets, void *sums_dev, int32_t device,
+                       void *stream);
+
+/* fe_backtest_portfolio with every value computed by rule column_dev[i] of rules_dev (num_rules FeRule records,
+ * 8-byte aligned) from the staged closes instead of loaded from a table: at A = 1 the thread-per-env loop of
+ * fe_backtest / fe_backtest_targets, at A > 1 the warp-per-env loop of fe_backtest_portfolio, each fed by the rule.
+ * The run is bit-identical to fe_backtest_portfolio (at A = 1 also fe_backtest / fe_backtest_targets) with the table
+ * fe_rule_table writes for the same rules: everything those calls guarantee, f64 sums up to their order of addition.
+ * rule_sums_dev: fe_rule_sums_build's buffer for s->prices.  Checks: fe_backtest_portfolio's, plus a NULL rules_dev /
+ * rule_sums_dev or num_rules < 1 FE_EINVAL and a misaligned one FE_EALIGN; every refusal happens before any CUDA call.
+ * Records are not checked here: the caller validates them (an out-of-range field evaluates to 0). */
+int fe_backtest_rules(const FeParams *p, const FeSeries *s, const FeState *st, const FeMetricsState *m,
+                      int64_t metrics_capacity, FeStats *stats_dev, const void *rule_sums_dev, const FeRule *rules_dev,
+                      int32_t num_rules, const int32_t *column_dev, int32_t targets, const double *exits_dev,
+                      uint64_t first_step, int32_t num_steps, void *rewards_dev, int32_t *dones_dev, int32_t history,
+                      void *stream);
+
+/* The (num_rules, num_rows, num_assets) float table the rules define: table[c, r, a] = the value of rules_dev[c] at row r
+ * for asset a, computed by the same device function as fe_backtest_rules.  FE_EINVAL for a NULL pointer or a
+ * non-positive size, num_assets outside 1..32; FE_EALIGN for a misaligned pointer. */
+int fe_rule_table(const double *prices_dev, const void *rule_sums_dev, int64_t num_rows, int32_t num_assets,
+                  const FeRule *rules_dev, int32_t num_rules, float *table_dev, int32_t device, void *stream);
+
 /* ---- ES rollout path (finenvs/agents/networks/parallel_mlp.py, finenvs/agents/ES/evo_agent.py) -------------
  * Population layout of the reference (parallel_mlp.py:121-136): envs [0, T/2) use theta + sigma*eps[p], envs
  * [T/2, T) use theta - sigma*eps[p - T/2] (T = num_envs - num_eval_envs, even), the last num_eval_envs envs use
