@@ -738,26 +738,29 @@ constexpr int kGradThreads = 128;
 constexpr int kGradSlab = 512; // pairs per block
 
 __global__ void __launch_bounds__(kGradThreads)
-fe_es_grad_partial_kernel(const int64_t total8, const int64_t num_pairs, const __half *__restrict__ eps,
-                          const float *__restrict__ w, float *__restrict__ partial) {
+fe_es_grad_partial_kernel(const int64_t total8, const int64_t num_pairs, const int64_t slabs,
+                          const __half *__restrict__ eps, const float *__restrict__ w, float *__restrict__ partial) {
     const int64_t q8 = (int64_t)blockIdx.x * kGradThreads + threadIdx.x;
     if (q8 >= total8) return;
-    const int64_t p0 = (int64_t)blockIdx.y * kGradSlab;
-    const int64_t p1 = p0 + kGradSlab < num_pairs ? p0 + kGradSlab : num_pairs;
-    float acc[8];
+    // gridDim.y is at most 65535: a block walks every gridDim.y-th slab when there are more slabs than that
+    for (int64_t slab = blockIdx.y; slab < slabs; slab += gridDim.y) {
+        const int64_t p0 = slab * kGradSlab;
+        const int64_t p1 = p0 + kGradSlab < num_pairs ? p0 + kGradSlab : num_pairs;
+        float acc[8];
 #pragma unroll
-    for (int o = 0; o < 8; ++o) acc[o] = 0.0f;
+        for (int o = 0; o < 8; ++o) acc[o] = 0.0f;
 #pragma unroll 4
-    for (int64_t p = p0; p < p1; ++p) {
-        float e[8];
-        halves8_to_floats(__ldg(reinterpret_cast<const uint4 *>(eps + (p * total8 + q8) * 8)), e);
-        const float wp = __ldg(w + p);
+        for (int64_t p = p0; p < p1; ++p) {
+            float e[8];
+            halves8_to_floats(__ldg(reinterpret_cast<const uint4 *>(eps + (p * total8 + q8) * 8)), e);
+            const float wp = __ldg(w + p);
 #pragma unroll
-        for (int o = 0; o < 8; ++o) acc[o] = fmaf(wp, e[o], acc[o]);
+            for (int o = 0; o < 8; ++o) acc[o] = fmaf(wp, e[o], acc[o]);
+        }
+        float4 *dst = reinterpret_cast<float4 *>(partial + (slab * total8 + q8) * 8);
+        dst[0] = make_float4(acc[0], acc[1], acc[2], acc[3]);
+        dst[1] = make_float4(acc[4], acc[5], acc[6], acc[7]);
     }
-    float4 *dst = reinterpret_cast<float4 *>(partial + ((int64_t)blockIdx.y * total8 + q8) * 8);
-    dst[0] = make_float4(acc[0], acc[1], acc[2], acc[3]);
-    dst[1] = make_float4(acc[4], acc[5], acc[6], acc[7]);
 }
 
 __global__ void __launch_bounds__(256)
@@ -1014,9 +1017,10 @@ int fe_es_gradient(const FeEsNet *net, const void *eps_dev, const float *pair_we
     DeviceGuard guard(pointer_device(eps_dev));
     if (guard.rc) return guard.rc;
     const int64_t total = lay.off[lay.L], total8 = total / 8, slabs = (num_pairs + kGradSlab - 1) / kGradSlab;
-    const dim3 grid((unsigned)((total8 + kGradThreads - 1) / kGradThreads), (unsigned)slabs);
-    fe_es_grad_partial_kernel<<<grid, kGradThreads, 0, (cudaStream_t)stream>>>(total8, num_pairs, (const __half *)eps_dev,
-                                                                               pair_weights_dev, scratch_dev);
+    const dim3 grid((unsigned)((total8 + kGradThreads - 1) / kGradThreads), (unsigned)(slabs < 65535 ? slabs : 65535));
+    fe_es_grad_partial_kernel<<<grid, kGradThreads, 0, (cudaStream_t)stream>>>(total8, num_pairs, slabs,
+                                                                               (const __half *)eps_dev, pair_weights_dev,
+                                                                               scratch_dev);
     fe_es_grad_reduce_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(total, slabs, scratch_dev,
                                                                                                grad_packed_dev);
     return (int)cudaGetLastError();
